@@ -2,7 +2,7 @@
 """bench.py - headline benchmark: Bandersnatch IETF VRF batch verify (BASELINE.json configs[1]) plus, in the same driver-run
 line, every other BASELINE config and the multi-GPU commitment MSM.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--logn 20]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--logn 20] [--dump-outputs DIR]
 
 A step = one pass of `ietf::Verifier::verify` over one batch of 2^logn synthetic proofs per GPU.
 Workload (SURVEY.md 8d): 2^logn DISTINCT items per GPU - sk_i = Secret::from_seed("vrfs-b200-bench-sk" || u64le(i)),
@@ -19,6 +19,8 @@ alpha_i = u64le(i) || 24 x 0x00, proofs produced by the engine's own prover and 
           ring_kzg_msm_ms (3-column commitment MSM for the domains 2^11..2^17; configs[4]) - at N > 1 the point-range-split
           form whose partial sums are exchanged by the MSM's last kernel over NVLink (no NCCL on the data path).
 --impl reference times the CPU oracle as the reference arm.
+--dump-outputs DIR writes the verdicts of the last timed headline step as DIR/ietf_verify_ok.npy (float32, one per item; the
+inputs are the same on every run with the same arguments), so that two builds can be compared output for output.
 Only the cross-checks, the cpu_baseline leg and --impl reference touch oracle/ (tests/oracle_lib.py).
 """
 import argparse
@@ -33,6 +35,7 @@ import time
 import traceback
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark may run from a read-only tree and writes nothing into it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -81,7 +84,28 @@ def parse():
     ap.add_argument("--cpu-sample-logn", type=int, default=18)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the secondary configs (profiling runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the verdicts of the last timed step as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_MAX_ITEMS = 1 << 22        # 16 MiB of float32 verdicts (+ 32 MiB of float64 indices when sampled): under 64 MB in all
+
+
+def dump_outputs(path, arrays):
+    """each array as path/<name>.npy in float32.  An array longer than DUMP_MAX_ITEMS is reduced to a sample of items drawn
+    with a fixed seed (the same for every run of the same size), and the sampled item indices go to path/<name>_index.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, arr in arrays.items():
+        arr = np.asarray(arr)
+        if len(arr) > DUMP_MAX_ITEMS:
+            idx = np.sort(np.random.default_rng(0).choice(len(arr), DUMP_MAX_ITEMS, replace=False))
+            np.save(os.path.join(path, name + "_index.npy"), idx.astype(np.float64))
+            arr = arr[idx]
+        np.save(os.path.join(path, name + ".npy"), arr.astype(np.float32))
 
 
 class ClockSampler:
@@ -513,6 +537,8 @@ def run_reference(a, rank, world):
         got = O.ietf_verify(O.BANDERSNATCH, w["pk"], w["inp"], w["out"], w["c"], w["s"], None, nthreads=cores)
     dt = time.perf_counter() - t0
     assert np.array_equal(got, w["expect"])
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"ietf_verify_ok": got})
     v = n * a.steps / dt
     sample = f"2^{a.ref_logn} distinct proofs per step (oracle-generated, same suite / ad as the GPU workload), {cores} pthreads"
     emit({
@@ -640,7 +666,10 @@ def main():
     ms_total = ev0.elapsed_time(ev1)
     clocks = sampler.stop()
     eng.enable_kernel_timing(False)
-    assert np.array_equal(d_ok.cpu().numpy(), expect)
+    verdicts = d_ok.cpu().numpy()
+    assert np.array_equal(verdicts, expect)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"ietf_verify_ok": verdicts})
 
     # ---- end to end through the host-buffer ABI (pinned host memory; H2D/D2H inside)
     for _ in range(2):

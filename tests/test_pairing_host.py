@@ -5,6 +5,7 @@ import ctypes as C
 import os
 import random
 import subprocess
+import sys
 
 import pytest
 
@@ -109,7 +110,7 @@ def test_lane_programs_match_oracle(emu):
 
 def test_lane_program_generator_self_check():
     """the generator's own model run of the emitted tables (twin and oracle equality) passes, and the committed tables are current"""
-    subprocess.run(["python", os.path.join(ROOT, "tools", "gen_pairing_prog.py"), "--check"], check=True, capture_output=True)
+    subprocess.run([sys.executable, os.path.join(ROOT, "tools", "gen_pairing_prog.py"), "--check"], check=True, capture_output=True)
 
 
 def test_pairing_identity_and_malformed_inputs(emu):
