@@ -91,7 +91,7 @@ static vrfs_status kzg_pairing_launch(vrfs_ctx* ctx, const uint8_t* d_lr, const 
 extern "C" vrfs_status vrfs_pairing_product_batch(vrfs_ctx* ctx, size_t n, int n_pairs, const uint8_t* g1, const uint8_t* g2, const uint32_t* negate_masks,
                                                   uint8_t* out_ok, uint8_t* out_gt) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (n_pairs < 1 || n_pairs > PAIRING_MAX_PAIRS || !g1 || !g2 || !out_ok) return fail(ctx, VRFS_BAD_ARG, "bad argument (1 <= n_pairs <= %d, non-null buffers)", PAIRING_MAX_PAIRS);
   ST(begin_call(ctx, n));
@@ -118,7 +118,7 @@ extern "C" vrfs_status vrfs_kzg_batch_verify(vrfs_ctx* ctx, size_t k, const uint
                                              const uint8_t* proofs, const uint8_t* coeffs_r, const uint8_t* g2, const uint8_t* tau_g2, int check_points,
                                              uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (!out_ok || !g2 || !tau_g2 || (k && (!commitments || !points_z || !values_v || !proofs || !coeffs_r))) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   if (k == 0) { *out_ok = 1; return VRFS_OK; }                   // nothing to check
   if (k > (1u << 24)) return fail(ctx, VRFS_BAD_ARG, "more than 2^24 openings per call are not supported");

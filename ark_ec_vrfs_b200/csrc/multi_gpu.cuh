@@ -42,7 +42,7 @@ static vrfs_status peer_alloc(vrfs_ctx* ctx, int rank, int world) {
 }
 extern "C" vrfs_status vrfs_ctx_peer_export(vrfs_ctx* ctx, int rank, int world, uint8_t* out_handle) {
   if (!ctx || !out_handle) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   static_assert(sizeof(cudaIpcMemHandle_t) == VRFS_PEER_HANDLE_BYTES, "cudaIpcMemHandle_t is 64 bytes");
   ST(peer_alloc(ctx, rank, world));
   cudaIpcMemHandle_t h;
@@ -53,7 +53,7 @@ extern "C" vrfs_status vrfs_ctx_peer_export(vrfs_ctx* ctx, int rank, int world, 
 }
 extern "C" vrfs_status vrfs_ctx_peer_connect(vrfs_ctx* ctx, const uint8_t* handles) {
   if (!ctx || !handles) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   auto& P = ctx->peer;
   if (P.world >= 0) return fail(ctx, VRFS_BAD_ARG, "vrfs_ctx_peer_export must come first");
   const int world = -P.world;
@@ -72,7 +72,7 @@ extern "C" vrfs_status vrfs_ctx_peer_connect(vrfs_ctx* ctx, const uint8_t* handl
 }
 extern "C" vrfs_status vrfs_ctx_peer_set_timeout_ms(vrfs_ctx* ctx, unsigned int ms) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   ctx->peer.timeout_ns = (unsigned long long)(ms ? ms : 1u) * 1000000ull;
   return VRFS_OK;
 }
@@ -102,7 +102,7 @@ static vrfs_status peer_check(vrfs_ctx* ctx) {          // after the stream was 
 // scalars of this rank's point range -> the FULL commitments on every rank
 extern "C" vrfs_status vrfs_msm_g1_prepared_allgather(vrfs_ctx* ctx, const vrfs_msm_bases* h, const uint8_t* scalars, int n_columns, uint8_t* out) {
   if (!ctx || !h || h->ctx != ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   PeerArgs pa;
   ST(peer_begin(ctx, -1, &pa));
   if (n_columns < 1 || n_columns > VRFS_PEER_MAXCOL || !scalars || !out) return fail(ctx, VRFS_BAD_ARG, "bad argument");
@@ -119,7 +119,7 @@ extern "C" vrfs_status vrfs_msm_g1_prepared_allgather(vrfs_ctx* ctx, const vrfs_
 extern "C" vrfs_status vrfs_ring_commit_rows_allgather(vrfs_ctx* ctx, const vrfs_msm_bases* srs_rows, size_t row_lo, size_t keyset_part_size, size_t n_keys,
                                                        const uint8_t* keys_rows, const uint8_t* padding, size_t n_tail, const uint8_t* tail, uint8_t* out_commitment) {
   if (!ctx || !srs_rows || srs_rows->ctx != ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   PeerArgs pa;
   ST(peer_begin(ctx, -1, &pa));
   if (!out_commitment) return fail(ctx, VRFS_BAD_ARG, "null buffer");

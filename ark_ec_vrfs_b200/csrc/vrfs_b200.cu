@@ -250,7 +250,7 @@ struct vrfs_ctx {
   cudaStream_t stream = nullptr;
   cudaStream_t copy_stream = nullptr;                 // H2D of later chunks overlaps the kernels of earlier ones
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  cudaEvent_t ev_chunk[4] = {nullptr, nullptr, nullptr, nullptr};
+  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;   // kernels on copy_stream beside the main stream (side_fork / side_join)
   cudaEvent_t ev_in[VRFS_HOST_PIECES] = {nullptr}, ev_out[VRFS_HOST_PIECES] = {nullptr};   // per-piece host transfers (stage_in_pieces / pieces_copy_out)
   char err[512] = {0};
   std::recursive_mutex mu;            // entry points serialise per context (SURVEY 8b: "internally synchronised")
@@ -280,16 +280,15 @@ static vrfs_status fail(vrfs_ctx* c, vrfs_status st, const char* fmt, ...) {
 //    holding sk are zeroed before release"; the buffers are pooled, so "release" is the end of the call);
 //  * after a failure both streams are drained, so that no copy is still reading the caller's host buffers when the error
 //    code reaches the caller.
-// one NVTX range per ABI call, named after the entry point (`ncu --nvtx --nvtx-include "vrfs_ietf_verify_batch/"` profiles the
-// kernels of one kind of call; header-only NVTX 3: a no-op unless a tool is attached)
-struct NvtxRange {
-  explicit NvtxRange(const char* name) { nvtxRangePushA(name); }
-  ~NvtxRange() { nvtxRangePop(); }
-};
+// An entry point passes its name (__func__): one NVTX range per ABI call, named after the entry point (`ncu --nvtx --nvtx-include
+// "vrfs_ietf_verify_batch/"` profiles the kernels of one kind of call; header-only NVTX 3: a no-op unless a tool is attached).
 struct CallGuard {
   vrfs_ctx* ctx;
-  explicit CallGuard(vrfs_ctx* c) : ctx(c) { ctx->mu.lock(); if (ctx->depth++ == 0) ctx->failed = false; }
+  const char* range;
+  explicit CallGuard(vrfs_ctx* c, const char* name = nullptr) : ctx(c), range(name) {
+    ctx->mu.lock(); if (ctx->depth++ == 0) ctx->failed = false; if (range) nvtxRangePushA(range); }
   ~CallGuard() {
+    if (range) nvtxRangePop();
     if (--ctx->depth == 0) {
       bool wiped = false;
       for (int i = 0; i < BUF_COUNT; i++) {
@@ -338,7 +337,7 @@ static vrfs_status note_kernel(vrfs_ctx* ctx, const char* name) {
 }
 extern "C" vrfs_status vrfs_ctx_enable_kernel_timing(vrfs_ctx* ctx, int on) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   ctx->timing = on != 0;
   ctx->n_timed = 0;
   return VRFS_OK;
@@ -346,7 +345,7 @@ extern "C" vrfs_status vrfs_ctx_enable_kernel_timing(vrfs_ctx* ctx, int on) {
 // device time of every kernel of the most recent *_batch / *_batch_dev call (after a sync); returns the count
 extern "C" int vrfs_ctx_kernel_timings(vrfs_ctx* ctx, const char** names, float* ms, int cap) {
   if (!ctx || !ctx->timing) return 0;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (cudaStreamSynchronize(ctx->stream) != cudaSuccess) return 0;
   int n = ctx->n_timed < cap ? ctx->n_timed : cap;
   for (int i = 0; i < n; i++) {
@@ -412,7 +411,7 @@ extern "C" vrfs_status vrfs_ctx_create(int device, vrfs_ctx** out) {
   ctx->sms = prop.multiProcessorCount;
   CU(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
   CU(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-  for (int i = 0; i < 4; i++) CU(cudaEventCreateWithFlags(&ctx->ev_chunk[i], cudaEventDisableTiming));
+  CU(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming)); CU(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
   for (int i = 0; i < VRFS_HOST_PIECES; i++) { CU(cudaEventCreateWithFlags(&ctx->ev_in[i], cudaEventDisableTiming)); CU(cudaEventCreateWithFlags(&ctx->ev_out[i], cudaEventDisableTiming)); }
   CU(cudaEventCreate(&ctx->ev0));
   CU(cudaEventCreate(&ctx->ev1));
@@ -428,7 +427,8 @@ extern "C" void vrfs_ctx_destroy(vrfs_ctx* ctx) {
   for (int s = 0; s < VRFS_SUITE_COUNT; s++) for (int b = 0; b < 2; b++) if (ctx->fixtab[s][b]) cudaFree(ctx->fixtab[s][b]);
   if (ctx->ev0) cudaEventDestroy(ctx->ev0);
   if (ctx->ev1) cudaEventDestroy(ctx->ev1);
-  for (int i = 0; i < 4; i++) if (ctx->ev_chunk[i]) cudaEventDestroy(ctx->ev_chunk[i]);
+  if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
+  if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
   for (int i = 0; i < VRFS_HOST_PIECES; i++) { if (ctx->ev_in[i]) cudaEventDestroy(ctx->ev_in[i]); if (ctx->ev_out[i]) cudaEventDestroy(ctx->ev_out[i]); }
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -436,7 +436,7 @@ extern "C" void vrfs_ctx_destroy(vrfs_ctx* ctx) {
 }
 extern "C" vrfs_status vrfs_ctx_sync(vrfs_ctx* ctx) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   CU(cudaStreamSynchronize(ctx->stream));
   return VRFS_OK;
 }
@@ -464,7 +464,7 @@ extern "C" vrfs_status vrfs_host_unregister(void* p) {
 // order, e.g. slot 0 holds `sk` during a prove call).  tests/ use it to check that key material is gone after a call returned.
 extern "C" vrfs_status vrfs_ctx_debug_read_staging(vrfs_ctx* ctx, int slot, size_t offset, uint8_t* out, size_t n) {
   if (!ctx || !out) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (slot < 0 || slot >= BUF_COUNT) return fail(ctx, VRFS_BAD_ARG, "no such staging buffer");
   const DevBuf& b = ctx->buf[slot];
   if (!b.p || offset + n > b.cap) return fail(ctx, VRFS_BAD_ARG, "range outside the staging buffer (capacity %zu)", b.cap);
@@ -476,8 +476,8 @@ extern "C" vrfs_status vrfs_ctx_debug_read_staging(vrfs_ctx* ctx, int slot, size
 extern "C" const char* vrfs_last_error(const vrfs_ctx* ctx) { return ctx ? ctx->err : "null context"; }
 extern "C" void* vrfs_ctx_stream(vrfs_ctx* ctx) { return ctx ? (void*)ctx->stream : nullptr; }
 extern "C" uint64_t vrfs_ctx_launch_count(const vrfs_ctx* ctx) { return ctx ? ctx->launches : 0; }
-// the suite behind a vrfs_suite value, handed to a generic lambda as a value of its tag type
-template <class F> static vrfs_status with_suite(vrfs_ctx* ctx, vrfs_suite s, F&& f) {
+// the suite behind a vrfs_suite value, handed to a generic lambda as a value of its tag type; `unknown()` for any other value
+template <class F, class U> static auto suite_switch(vrfs_suite s, F&& f, U&& unknown) -> decltype(unknown()) {
   switch (s) {
     case VRFS_BANDERSNATCH_ELL2: return f(BandSuite{});
     case VRFS_ED25519_TAI: return f(EdSuite{});
@@ -485,19 +485,23 @@ template <class F> static vrfs_status with_suite(vrfs_ctx* ctx, vrfs_suite s, F&
     case VRFS_BANDERSNATCH_SW_TAI: return f(BandSwSuite{});
     case VRFS_JUBJUB_TAI: return f(JubSuite{});
     case VRFS_BABYJUBJUB_TAI: return f(BjjSuite{});
-    default: return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)s);
+    default: return unknown();
   }
 }
-template <class F> static int suite_const(vrfs_suite s, F&& f) {
-  switch (s) {
-    case VRFS_BANDERSNATCH_ELL2: return f(BandSuite{});
-    case VRFS_ED25519_TAI: return f(EdSuite{});
-    case VRFS_P256_TAI: return f(P256Suite{});
-    case VRFS_BANDERSNATCH_SW_TAI: return f(BandSwSuite{});
-    case VRFS_JUBJUB_TAI: return f(JubSuite{});
-    case VRFS_BABYJUBJUB_TAI: return f(BjjSuite{});
-    default: return 0;
-  }
+template <class F> static vrfs_status with_suite(vrfs_ctx* ctx, vrfs_suite s, F&& f) {
+  return suite_switch(s, f, [&] { return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)s); });
+}
+template <class F> static int suite_const(vrfs_suite s, F&& f) { return suite_switch(s, f, [] { return 0; }); }
+// after the argument checks of a batch entry point, before anything is enqueued
+static vrfs_status begin_call(vrfs_ctx* ctx, size_t n) {
+  if (n > 0x7fffffffu) return fail(ctx, VRFS_BAD_ARG, "batch too large (n < 2^31)");
+  CU(cudaSetDevice(ctx->device));
+  return timing_begin(ctx);
+}
+// ... of one that takes a suite: an unknown suite is VRFS_BAD_ARG here, before any size is derived from it
+static vrfs_status begin_call(vrfs_ctx* ctx, vrfs_suite suite, size_t n) {
+  ST(with_suite(ctx, suite, [](auto) { return VRFS_OK; }));
+  return begin_call(ctx, n);
 }
 extern "C" int vrfs_suite_challenge_len(vrfs_suite s) { return suite_const(s, [](auto S_) { return (int)decltype(S_)::CLEN; }); }
 extern "C" int vrfs_suite_hash_len(vrfs_suite s) { return suite_const(s, [](auto S_) { return (int)decltype(S_)::HLEN; }); }
@@ -506,44 +510,49 @@ extern "C" int vrfs_suite_point_enc_len(vrfs_suite s) { return suite_const(s, []
 // =================================================================================================
 // lincomb launcher
 // =================================================================================================
-// `side` = true: enqueue on the context's second stream with its own slab, so that two independent linear combinations of a
-// small batch (U and V of a verify) run concurrently instead of back to back; the caller joins the streams.
-template <class C, int NV, int NF>
-static vrfs_status launch_lincomb(vrfs_ctx* ctx, LincombArgs A, bool side = false) {
-  if (A.n == 0) return VRFS_OK;
-  cudaStream_t stream = side ? ctx->copy_stream : ctx->stream;
+// Kernels on the context's second stream beside the main one: side_fork makes it start after everything enqueued on the main
+// stream so far, side_join makes the main stream wait for everything enqueued on it.
+static vrfs_status side_fork(vrfs_ctx* ctx) { CU(cudaEventRecord(ctx->ev_fork, ctx->stream)); CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_fork, 0)); return VRFS_OK; }
+static vrfs_status side_join(vrfs_ctx* ctx) { CU(cudaEventRecord(ctx->ev_join, ctx->copy_stream)); CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0)); return VRFS_OK; }
+// Persistent grid of a lincomb kernel: as many blocks as fit on the GPU at once, but no more than `threads` threads need; each
+// thread's window-table slab of `slab_per_thread` bytes in buffer `buf`, and the kernel's work counter behind the slabs (zeroed).
+static vrfs_status lincomb_grid(vrfs_ctx* ctx, const void* kernel, size_t threads, size_t slab_per_thread, int buf, cudaStream_t stream,
+                                LincombArgs* A, uint32_t* blocks) {
   int per_sm = 0;
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_lincomb<C, NV, NF>, LINCOMB_THREADS, 0));
+  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, LINCOMB_THREADS, 0));
   if (per_sm < 1) per_sm = 1;
 #ifdef LINCOMB_MAXBLOCKS
   if (per_sm > LINCOMB_MAXBLOCKS) per_sm = LINCOMB_MAXBLOCKS;       // tuning builds: resident threads per SM (the slab scales with them)
 #endif
-  uint32_t blocks = (uint32_t)(ctx->sms * per_sm);
-  uint32_t need = (A.n + LINCOMB_THREADS - 1) / LINCOMB_THREADS;
-  if (blocks > need) blocks = need;
+  *blocks = (uint32_t)std::min((size_t)ctx->sms * per_sm, (threads + LINCOMB_THREADS - 1) / LINCOMB_THREADS);
+  const size_t slabs = (size_t)*blocks * LINCOMB_THREADS * slab_per_thread;
   void* slab = nullptr;
-  ST(ensure(ctx, side ? BUF_SLAB2 : BUF_SLAB, (size_t)blocks * LINCOMB_THREADS * slab_bytes<C>(NV) + 256, &slab));
-  A.slab = (uint8_t*)slab;
-  A.next_item = reinterpret_cast<uint32_t*>((uint8_t*)slab + (size_t)blocks * LINCOMB_THREADS * slab_bytes<C>(NV));   // work counter behind the slabs
-  CU(cudaMemsetAsync(A.next_item, 0, sizeof(uint32_t), stream));
+  ST(ensure(ctx, buf, slabs + 256, &slab));
+  A->slab = (uint8_t*)slab;
+  A->next_item = reinterpret_cast<uint32_t*>(A->slab + slabs);
+  CU(cudaMemsetAsync(A->next_item, 0, sizeof(uint32_t), stream));
+  return VRFS_OK;
+}
+template <int NV, int NF> static const char* lincomb_name() {   // kernel-timing name of k_lincomb<C, NV, NF>
+  static constexpr char name[] = {'l', 'i', 'n', 'c', 'o', 'm', 'b', '<', char('0' + NV), ',', char('0' + NF), '>', '\0'}; return name; }
+// `side` = true: enqueue on the context's second stream with its own slab, so that two independent linear combinations of a
+// small batch (U and V of a verify) run concurrently instead of back to back; the caller forks and joins the streams.
+template <class C, int NV, int NF>
+static vrfs_status launch_lincomb(vrfs_ctx* ctx, LincombArgs A, bool side = false) {
+  if (A.n == 0) return VRFS_OK;
+  cudaStream_t stream = side ? ctx->copy_stream : ctx->stream;
+  uint32_t blocks = 0;
+  ST(lincomb_grid(ctx, (const void*)k_lincomb<C, NV, NF>, A.n, slab_bytes<C>(NV), side ? BUF_SLAB2 : BUF_SLAB, stream, &A, &blocks));
   k_lincomb<C, NV, NF><<<blocks, LINCOMB_THREADS, 0, stream>>>(A);
-  LAUNCHED_AS(ctx, NV == 2 ? "lincomb<2,0>" : NV == 1 && NF == 1 ? "lincomb<1,1>" : NV == 1 ? "lincomb<1,0>" : NF == 2 ? "lincomb<0,2>" : NV == 1 && NF == 2 ? "lincomb<1,2>" : "lincomb<0,1>");
+  LAUNCHED_AS(ctx, (lincomb_name<NV, NF>()));
   return VRFS_OK;
 }
 
 template <class C>
 static vrfs_status launch_lincomb_verify_pair(vrfs_ctx* ctx, LincombArgs U, LincombArgs V) {
-  int per_sm = 0;
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_lincomb_verify_pair<C>, LINCOMB_THREADS, 0));
-  if (per_sm < 1) per_sm = 1;
-  uint32_t blocks = (uint32_t)(ctx->sms * per_sm);
-  const uint32_t need = (2u * V.n + LINCOMB_THREADS - 1) / LINCOMB_THREADS;
-  if (blocks > need) blocks = need;
-  void* slab = nullptr;
-  ST(ensure(ctx, BUF_SLAB, (size_t)blocks * LINCOMB_THREADS * slab_bytes<C>(2) + 256, &slab));
-  U.slab = V.slab = (uint8_t*)slab;
-  U.next_item = V.next_item = reinterpret_cast<uint32_t*>((uint8_t*)slab + (size_t)blocks * LINCOMB_THREADS * slab_bytes<C>(2));
-  CU(cudaMemsetAsync(V.next_item, 0, sizeof(uint32_t), ctx->stream));
+  uint32_t blocks = 0;
+  ST(lincomb_grid(ctx, (const void*)k_lincomb_verify_pair<C>, 2 * (size_t)V.n, slab_bytes<C>(2), BUF_SLAB, ctx->stream, &V, &blocks));
+  U.slab = V.slab; U.next_item = V.next_item;                         // one slab and one task counter for both combinations
   k_lincomb_verify_pair<C><<<blocks, LINCOMB_THREADS, 0, ctx->stream>>>(U, V);
   LAUNCHED_AS(ctx, "lincomb<1,1>+<2,0>");
   return VRFS_OK;
@@ -589,20 +598,14 @@ static vrfs_status ietf_verify_dev(vrfs_ctx* ctx, size_t n, const uint8_t* pk, c
   A.var[0] = {pk, 64, c, 32, 1, cbits};
   A.fix[0] = {s, 32, 0, ctx->fixtab[S::ID][0]};
   A.out_xyz = (uint32_t*)u;
-  if (split) {   // the side stream starts after everything already enqueued on the main stream (inputs, the memset of `valid`)
-    CU(cudaEventRecord(ctx->ev_chunk[2], ctx->stream));
-    CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_chunk[2], 0));
-  }
+  if (split) ST(side_fork(ctx));   // the side stream starts after the inputs and the memset of `valid`
   ST((launch_lincomb<C, 1, 1>(ctx, A, split)));
   // V = s*I - c*O
   A.var[0] = {input, 64, s, 32, 0, 0};
   A.var[1] = {output, 64, c, 32, 1, cbits};
   A.out_xyz = (uint32_t*)v;
   ST((launch_lincomb<C, 2, 0>(ctx, A)));
-  if (split) {
-    CU(cudaEventRecord(ctx->ev_chunk[3], ctx->copy_stream));
-    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk[3], 0));
-  }
+  if (split) ST(side_join(ctx));
   k_ietf_verify_finish<S><<<(unsigned)((n + 128 * FINISH_K - 1) / (128 * FINISH_K)), 128, 0, ctx->stream>>>((uint32_t)n, pk, input, output, c, (const uint32_t*)u,
                                                                                 (const uint32_t*)v, ad, ad_off, (const uint8_t*)valid, out_ok, out_status);
   LAUNCHED_AS(ctx, "ietf_verify_finish");
@@ -613,13 +616,11 @@ extern "C" vrfs_status vrfs_ietf_verify_batch_dev(vrfs_ctx* ctx, vrfs_suite suit
                                                   const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad,
                                                   const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!pk || !input || !output || !c || !s || !out_ok || (ad && !ad_off)) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if (n > 0x7fffffffu) return fail(ctx, VRFS_BAD_ARG, "batch too large (n < 2^31)");
   if (!aligned16(pk) || !aligned16(input) || !aligned16(output) || !aligned16(c) || !aligned16(s)) return fail(ctx, VRFS_BAD_ARG, "device buffers must be 16-byte aligned");
-  CU(cudaSetDevice(ctx->device));
-  ST(timing_begin(ctx));
+  ST(begin_call(ctx, suite, n));
   return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return ietf_verify_dev<S>(ctx, n, pk, input, output, c, s, ad, ad_off, out_ok, out_status); });
 }
 
@@ -658,64 +659,12 @@ static vrfs_status stage_var(vrfs_ctx* ctx, int buf_data, int buf_off, size_t n,
   return VRFS_OK;
 }
 
-// Host buffers, everything enqueued and nothing waited for (the multi-device context enqueues one of these per GPU before it
-// waits for any): the batch is cut into a first piece of one resident wave of the lincomb grid and the remainder, the H2D copies
-// run on their own stream, and the kernels of piece k wait only for piece k's copies - so all but the first ~20 MB of the
-// 256 B/item input transfer hides behind arithmetic (pinned host memory; pageable memory still works, the copies then
-// serialise inside the driver).
-static vrfs_status ietf_verify_host_enqueue(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* pk, const uint8_t* input, const uint8_t* output,
-                                            const uint8_t* c, const uint8_t* s, const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
-  if (!pk || !input || !output || !c || !s || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if (n > 0x7fffffffu) return fail(ctx, VRFS_BAD_ARG, "batch too large (n < 2^31)");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  CU(cudaSetDevice(ctx->device));
-  const uint8_t* d_ad;
-  const uint64_t* d_off;
-  void *d_pk = nullptr, *d_in = nullptr, *d_out = nullptr, *d_c = nullptr, *d_s = nullptr, *d_ok = nullptr, *d_st = nullptr;
-  ST(ensure(ctx, BUF_IN0, n * 64, &d_pk)); ST(ensure(ctx, BUF_IN1, n * 64, &d_in)); ST(ensure(ctx, BUF_IN2, n * 64, &d_out));
-  ST(ensure(ctx, BUF_IN3, n * 32, &d_c)); ST(ensure(ctx, BUF_IN4, n * 32, &d_s)); ST(ensure(ctx, BUF_OUT0, n, &d_ok));
-  if (out_status) ST(ensure(ctx, BUF_OUT1, n, &d_st));
-  ST(stage_ad(ctx, n, ad, ad_off, &d_ad, &d_off));
-  const size_t wave = (size_t)ctx->sms * LINCOMB_MINBLOCKS * LINCOMB_THREADS;
-  size_t cut[3] = {0, n > 3 * wave ? wave : n, n};
-  const int pieces = cut[1] < n ? 2 : 1;
-  for (int k = 0; k < pieces; k++) {
-    const size_t o = cut[k], m = cut[k + 1] - cut[k];
-    CU(cudaMemcpyAsync((uint8_t*)d_pk + o * 64, pk + o * 64, m * 64, cudaMemcpyHostToDevice, ctx->copy_stream));
-    CU(cudaMemcpyAsync((uint8_t*)d_in + o * 64, input + o * 64, m * 64, cudaMemcpyHostToDevice, ctx->copy_stream));
-    CU(cudaMemcpyAsync((uint8_t*)d_out + o * 64, output + o * 64, m * 64, cudaMemcpyHostToDevice, ctx->copy_stream));
-    CU(cudaMemcpyAsync((uint8_t*)d_c + o * 32, c + o * 32, m * 32, cudaMemcpyHostToDevice, ctx->copy_stream));
-    CU(cudaMemcpyAsync((uint8_t*)d_s + o * 32, s + o * 32, m * 32, cudaMemcpyHostToDevice, ctx->copy_stream));
-    CU(cudaEventRecord(ctx->ev_chunk[k], ctx->copy_stream));
-  }
-  for (int k = 0; k < pieces; k++) {
-    const size_t o = cut[k], m = cut[k + 1] - cut[k];
-    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk[k], 0));
-    ST(vrfs_ietf_verify_batch_dev(ctx, suite, m, (const uint8_t*)d_pk + o * 64, (const uint8_t*)d_in + o * 64, (const uint8_t*)d_out + o * 64,
-                                  (const uint8_t*)d_c + o * 32, (const uint8_t*)d_s + o * 32, d_ad, d_off ? d_off + o : nullptr, (uint8_t*)d_ok + o,
-                                  d_st ? (uint8_t*)d_st + o : nullptr));
-  }
-  CU(cudaMemcpyAsync(out_ok, d_ok, n, cudaMemcpyDeviceToHost, ctx->stream));
-  if (out_status) CU(cudaMemcpyAsync(out_status, d_st, n, cudaMemcpyDeviceToHost, ctx->stream));
-  return VRFS_OK;
-}
-extern "C" vrfs_status vrfs_ietf_verify_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* pk, const uint8_t* input,
-                                              const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad,
-                                              const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
-  if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
-  if (n == 0) return VRFS_OK;
-  ST(ietf_verify_host_enqueue(ctx, suite, n, pk, input, output, c, s, ad, ad_off, out_ok, out_status));
-  CU(cudaStreamSynchronize(ctx->stream));
-  return VRFS_OK;
-}
-
 // =================================================================================================
 // measurement helper
 // =================================================================================================
 extern "C" vrfs_status vrfs_measure_mac32_peak(vrfs_ctx* ctx, int variant, double* out_mac_per_s, double* out_sm_mhz_est) {
   if (!ctx || !out_mac_per_s) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   CU(cudaSetDevice(ctx->device));
   const int threads = 256, blocks = ctx->sms * 8;
   void *out = nullptr, *cyc = nullptr;
@@ -896,11 +845,6 @@ static vrfs_status finish_call(vrfs_ctx* ctx) {
   CU(cudaStreamSynchronize(ctx->stream));
   return VRFS_OK;
 }
-static vrfs_status begin_call(vrfs_ctx* ctx, size_t n) {
-  if (n > 0x7fffffffu) return fail(ctx, VRFS_BAD_ARG, "batch too large (n < 2^31)");
-  CU(cudaSetDevice(ctx->device));
-  return timing_begin(ctx);
-}
 static vrfs_status fresh_valid(vrfs_ctx* ctx, size_t n, uint8_t** valid) {
   void* v = nullptr;
   ST(ensure(ctx, BUF_VALID, n, &v));
@@ -917,8 +861,9 @@ static vrfs_status stage_secret(vrfs_ctx* ctx, int which, const void* host, size
 }
 // Host buffers of a large batch call travel in PIECES on the copy stream: one resident wave of the lincomb grid first, then the
 // rest in up to max_pieces - 1 runs of whole waves.  Piece k's kernels wait only for piece k's inputs, so all but the first
-// ~20 MB of the input transfer hides behind arithmetic (as in vrfs_ietf_verify_batch), and piece k's results go back to the
-// host while piece k + 1 computes (pieces_copy_out) - what matters for the prove calls, whose outputs are 64-288 B per item.
+// ~20 MB of the input transfer hides behind arithmetic (pinned host memory; pageable memory still works, the copies then
+// serialise inside the driver), and piece k's results go back to the host while piece k + 1 computes (pieces_copy_out) - what
+// matters for the prove calls, whose outputs are 64-288 B per item.
 struct HostIn { int buf; const void* host; size_t stride; bool secret; uint8_t* dev; };
 struct HostOut { void* host; const uint8_t* dev; size_t stride; };
 struct Pieces { size_t cut[VRFS_HOST_PIECES + 1]; int count; };
@@ -995,6 +940,43 @@ template <class S> static vrfs_status data_to_point_dev(vrfs_ctx* ctx, size_t n,
   return VRFS_OK;
 }
 
+// ---- ietf verify (host buffers) ------------------------------------------------------------
+// Everything enqueued and nothing waited for (the multi-device context enqueues one of these per GPU before it waits for any):
+// the inputs travel in two pieces (stage_in_pieces), the 1 B/item of verdicts return on the main stream after the last piece.
+static vrfs_status ietf_verify_host_enqueue(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* pk, const uint8_t* input, const uint8_t* output,
+                                            const uint8_t* c, const uint8_t* s, const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
+  if (!pk || !input || !output || !c || !s || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  ST(begin_call(ctx, suite, n));
+  const uint8_t* d_ad; const uint64_t* d_off; uint8_t *d_ok, *d_st = nullptr;
+  // ad and the result buffers first: a buffer that grows is reallocated, which waits for the copies already in flight
+  ST(stage_ad(ctx, n, ad, ad_off, &d_ad, &d_off));
+  ST(stage_out(ctx, BUF_OUT0, n, &d_ok));
+  if (out_status) ST(stage_out(ctx, BUF_OUT1, n, &d_st));
+  HostIn in[5] = {{BUF_IN0, pk, 64, false, nullptr}, {BUF_IN1, input, 64, false, nullptr}, {BUF_IN2, output, 64, false, nullptr},
+                  {BUF_IN3, c, 32, false, nullptr}, {BUF_IN4, s, 32, false, nullptr}};
+  Pieces pc;
+  ST(stage_in_pieces(ctx, n, in, 5, &pc, 2));
+  for (int k = 0; k < pc.count; k++) {
+    const size_t o = pc.cut[k], m = pc.cut[k + 1] - pc.cut[k];
+    ST(piece_ready(ctx, k));
+    ST(with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S;
+      return ietf_verify_dev<S>(ctx, m, in[0].dev + o * 64, in[1].dev + o * 64, in[2].dev + o * 64, in[3].dev + o * 32, in[4].dev + o * 32, d_ad,
+                                d_off ? d_off + o : nullptr, d_ok + o, d_st ? d_st + o : nullptr); }));
+  }
+  ST(copy_out(ctx, out_ok, d_ok, n));
+  if (out_status) ST(copy_out(ctx, out_status, d_st, n));
+  return VRFS_OK;
+}
+extern "C" vrfs_status vrfs_ietf_verify_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* pk, const uint8_t* input,
+                                              const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad,
+                                              const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  if (n == 0) return VRFS_OK;
+  ST(ietf_verify_host_enqueue(ctx, suite, n, pk, input, output, c, s, ad, ad_off, out_ok, out_status));
+  return finish_call(ctx);
+}
+
 // ---- ietf prove -----------------------------------------------------------------------------
 template <class S>
 static vrfs_status ietf_prove_dev(vrfs_ctx* ctx, size_t n, const uint8_t* sk, const uint8_t* input, const uint8_t* output, const uint8_t* ad,
@@ -1026,11 +1008,10 @@ static vrfs_status ietf_prove_dev(vrfs_ctx* ctx, size_t n, const uint8_t* sk, co
 extern "C" vrfs_status vrfs_ietf_prove_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* sk, const uint8_t* input, const uint8_t* output,
                                              const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_c, uint8_t* out_s) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!sk || !input || !output || !out_c || !out_s) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_ad; const uint64_t* d_off; uint8_t *d_c, *d_s;
   HostIn in[3] = {{BUF_IN0, sk, 32, true, nullptr}, {BUF_IN1, input, 64, false, nullptr}, {BUF_IN2, output, 64, false, nullptr}};
   Pieces pc;   // two pieces: every further piece costs ~1 % in kernel tails, more than hiding the rest of the 64 B/item of results returns
@@ -1064,11 +1045,10 @@ template <class S> static vrfs_status output_dev(vrfs_ctx* ctx, size_t n, const 
 }
 extern "C" vrfs_status vrfs_output_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* sk, const uint8_t* input, uint8_t* out_output) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!sk || !input || !out_output) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t *d_sk, *d_in; uint8_t* d_o;
   ST(stage_secret(ctx, BUF_IN0, sk, n * 32, &d_sk)); ST(stage_in(ctx, BUF_IN1, input, n * 64, &d_in)); ST(stage_out(ctx, BUF_OUT0, n * 64, &d_o));
   ST(with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return output_dev<S>(ctx, n, d_sk, d_in, d_o); }));
@@ -1095,11 +1075,10 @@ template <class S> static vrfs_status from_seed_dev(vrfs_ctx* ctx, size_t n, con
 extern "C" vrfs_status vrfs_secret_from_seed_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* seeds, const uint64_t* seed_off,
                                                    uint8_t* out_sk, uint8_t* out_pk) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!seed_off || !out_sk) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_seeds; const uint64_t* d_off; uint8_t *d_sk, *d_pk = nullptr;
   ST(stage_ad(ctx, n, seeds, seed_off, &d_seeds, &d_off));
   mark_secret(ctx, BUF_AD, (size_t)(seed_off[n] - seed_off[0]));
@@ -1113,11 +1092,10 @@ extern "C" vrfs_status vrfs_secret_from_seed_batch(vrfs_ctx* ctx, vrfs_suite sui
 }
 extern "C" vrfs_status vrfs_nonce_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* sk, const uint8_t* input, uint8_t* out_k) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!sk || !input || !out_k) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t *d_sk, *d_in; uint8_t* d_k;
   ST(stage_secret(ctx, BUF_IN0, sk, n * 32, &d_sk)); ST(stage_in(ctx, BUF_IN1, input, n * 64, &d_in)); ST(stage_out(ctx, BUF_OUT0, n * 32, &d_k));
   mark_secret(ctx, BUF_OUT0, n * 32);
@@ -1128,11 +1106,10 @@ extern "C" vrfs_status vrfs_nonce_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t 
 }
 extern "C" vrfs_status vrfs_point_to_hash_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* pts, uint8_t* out_hash) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!pts || !out_hash) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_p; uint8_t* d_h;
   const size_t hl = (size_t)vrfs_suite_hash_len(suite);
   ST(stage_in(ctx, BUF_IN0, pts, n * 64, &d_p)); ST(stage_out(ctx, BUF_OUT0, n * hl, &d_h));
@@ -1143,11 +1120,10 @@ extern "C" vrfs_status vrfs_point_to_hash_batch(vrfs_ctx* ctx, vrfs_suite suite,
 }
 extern "C" vrfs_status vrfs_point_encode_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* pts, uint8_t* out_enc) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!pts || !out_enc) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_p; uint8_t* d_e;
   const size_t el = (size_t)vrfs_suite_point_enc_len(suite);
   ST(stage_in(ctx, BUF_IN0, pts, n * 64, &d_p)); ST(stage_out(ctx, BUF_OUT0, n * el, &d_e));
@@ -1158,11 +1134,10 @@ extern "C" vrfs_status vrfs_point_encode_batch(vrfs_ctx* ctx, vrfs_suite suite, 
 }
 extern "C" vrfs_status vrfs_point_decode_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* enc, uint8_t* out_pts, uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!enc || !out_pts || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_e; uint8_t *d_p, *d_ok;
   const size_t el = (size_t)vrfs_suite_point_enc_len(suite);
   ST(stage_in(ctx, BUF_IN0, enc, n * el, &d_e)); ST(stage_out(ctx, BUF_OUT0, n * 64, &d_p)); ST(stage_out(ctx, BUF_OUT1, n, &d_ok));
@@ -1174,11 +1149,10 @@ extern "C" vrfs_status vrfs_point_decode_batch(vrfs_ctx* ctx, vrfs_suite suite, 
 extern "C" vrfs_status vrfs_data_to_point_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* data, const uint64_t* data_off,
                                                 uint8_t* out_pts, uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!data_off || !out_pts || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_d; const uint64_t* d_off; uint8_t *d_p, *d_ok;
   ST(stage_ad(ctx, n, data, data_off, &d_d, &d_off));
   ST(stage_out(ctx, BUF_OUT0, n * 64, &d_p)); ST(stage_out(ctx, BUF_OUT1, n, &d_ok));
@@ -1219,11 +1193,10 @@ static vrfs_status pedersen_prove_dev(vrfs_ctx* ctx, size_t n, const uint8_t* sk
 extern "C" vrfs_status vrfs_pedersen_prove_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* sk, const uint8_t* input, const uint8_t* output,
                                                  const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_proof, uint8_t* out_blinding) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!sk || !input || !output || !out_proof || !out_blinding) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_ad; const uint64_t* d_off; uint8_t *d_pr, *d_bl;
   HostIn in[3] = {{BUF_IN0, sk, 32, true, nullptr}, {BUF_IN1, input, 64, false, nullptr}, {BUF_IN2, output, 64, false, nullptr}};
   Pieces pc;   // 288 B/item of results: worth VRFS_HOST_PIECES pieces (measured 2^20: e2e 19.4 -> 20.8 M/s, kernels 21.8 -> 20.9 M/s)
@@ -1269,11 +1242,10 @@ static vrfs_status pedersen_verify_dev(vrfs_ctx* ctx, size_t n, const uint8_t* i
 extern "C" vrfs_status vrfs_pedersen_verify_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* input, const uint8_t* output, const uint8_t* proof,
                                                   const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!input || !output || !proof || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_ad; const uint64_t* d_off; uint8_t *d_ok, *d_st = nullptr;
   HostIn in[3] = {{BUF_IN0, input, 64, false, nullptr}, {BUF_IN1, output, 64, false, nullptr}, {BUF_IN2, proof, 256, false, nullptr}};
   Pieces pc;
@@ -1352,11 +1324,10 @@ template <class S> static vrfs_status decode_checked_launch(vrfs_ctx* ctx, size_
 }
 extern "C" vrfs_status vrfs_point_decode_checked_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* enc, uint8_t* out_pts, uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!enc || !out_pts || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint32_t el = (uint32_t)vrfs_suite_point_enc_len(suite);
   const uint8_t* d_e; uint8_t *d_p, *d_ok;
   ST(stage_in(ctx, BUF_X0, enc, n * el, &d_e)); ST(stage_out(ctx, BUF_OUT0, n * 64, &d_p)); ST(stage_out(ctx, BUF_OUT1, n, &d_ok));
@@ -1366,11 +1337,10 @@ extern "C" vrfs_status vrfs_point_decode_checked_batch(vrfs_ctx* ctx, vrfs_suite
 }
 extern "C" vrfs_status vrfs_subgroup_check_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* pts, uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!pts || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const uint8_t* d_p; uint8_t* d_ok;
   ST(stage_in(ctx, BUF_IN0, pts, n * 64, &d_p)); ST(stage_out(ctx, BUF_OUT0, n, &d_ok));
   ST(with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; k_subgroup_check<S><<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, d_p, d_ok); return VRFS_OK; }));
@@ -1393,11 +1363,10 @@ template <class S> static vrfs_status ietf_sign_wire_dev(vrfs_ctx* ctx, size_t n
 extern "C" vrfs_status vrfs_ietf_sign_wire_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* sk, const uint8_t* data, const uint64_t* data_off,
                                                  const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_sig, uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!sk || !data_off || !out_sig) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const size_t sl = (size_t)vrfs_suite_ietf_signature_len(suite);
   const uint8_t *d_sk, *d_ad, *d_data; const uint64_t *d_off, *d_doff;
   uint8_t *d_in, *d_out, *d_c, *d_s, *d_ok, *d_sig;
@@ -1433,11 +1402,10 @@ template <class S> static vrfs_status ietf_verify_wire_dev(vrfs_ctx* ctx, size_t
 extern "C" vrfs_status vrfs_ietf_verify_wire_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* pk_enc, const uint8_t* data, const uint64_t* data_off,
                                                    const uint8_t* sig, const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_hash, uint8_t* out_status) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!pk_enc || !data_off || !sig || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const size_t sl = (size_t)vrfs_suite_ietf_signature_len(suite), el = (size_t)vrfs_suite_point_enc_len(suite), hl = (size_t)vrfs_suite_hash_len(suite);
   const uint8_t *d_ad, *d_data; const uint64_t *d_off, *d_doff;
   uint8_t *d_pk, *d_in, *d_out, *d_c, *d_s, *d_flags, *d_ok, *d_hash = nullptr, *d_st = nullptr;
@@ -1529,11 +1497,10 @@ template <class S> static vrfs_status pedersen_sign_wire_dev(vrfs_ctx* ctx, size
 extern "C" vrfs_status vrfs_pedersen_sign_wire_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* sk, const uint8_t* data, const uint64_t* data_off,
                                                      const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_sig, uint8_t* out_blinding, uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!sk || !data_off || !out_sig || !out_blinding) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const size_t sl = (size_t)vrfs_suite_pedersen_signature_len(suite);
   const uint8_t *d_sk, *d_ad, *d_data; const uint64_t *d_off, *d_doff;
   uint8_t *d_in, *d_out, *d_pr, *d_bl, *d_ok, *d_sig;
@@ -1566,11 +1533,10 @@ template <class S, int NP> static vrfs_status pedersen_verify_wire_dev(vrfs_ctx*
 extern "C" vrfs_status vrfs_pedersen_verify_wire_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* data, const uint64_t* data_off, const uint8_t* sig,
                                                        const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!data_off || !sig || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const size_t sl = (size_t)vrfs_suite_pedersen_signature_len(suite);
   const uint8_t *d_sig, *d_ad, *d_data; const uint64_t *d_off, *d_doff;
   uint8_t *d_in, *d_out, *d_pr, *d_flags, *d_ok, *d_st = nullptr;
@@ -1597,11 +1563,10 @@ template <class S> static vrfs_status pedersen_prove_compressed_dev(vrfs_ctx* ct
 extern "C" vrfs_status vrfs_pedersen_prove_compressed_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* sk, const uint8_t* input, const uint8_t* output,
                                                             const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_proof, uint8_t* out_blinding) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!sk || !input || !output || !out_proof || !out_blinding) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const size_t pl = (size_t)vrfs_suite_pedersen_proof_len(suite);
   const uint8_t* d_ad; const uint64_t* d_off; uint8_t *d_pr, *d_bl, *d_enc;
   HostIn in[3] = {{BUF_IN0, sk, 32, true, nullptr}, {BUF_IN1, input, 64, false, nullptr}, {BUF_IN2, output, 64, false, nullptr}};
@@ -1624,11 +1589,10 @@ extern "C" vrfs_status vrfs_pedersen_prove_compressed_batch(vrfs_ctx* ctx, vrfs_
 extern "C" vrfs_status vrfs_pedersen_verify_compressed_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* input, const uint8_t* output, const uint8_t* proof,
                                                              const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n == 0) return VRFS_OK;
   if (!input || !output || !proof || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
-  if ((unsigned)suite >= VRFS_SUITE_COUNT) return fail(ctx, VRFS_BAD_ARG, "unknown suite %d", (int)suite);
-  ST(begin_call(ctx, n));
+  ST(begin_call(ctx, suite, n));
   const size_t pl = (size_t)vrfs_suite_pedersen_proof_len(suite);
   const uint8_t *d_enc, *d_ad, *d_in, *d_out; const uint64_t* d_off;
   uint8_t *d_pr, *d_flags, *d_ok, *d_st = nullptr;
@@ -1713,25 +1677,17 @@ static vrfs_status msm_dev(vrfs_ctx* ctx, MsmPlan p, const void* d_bases, const 
   }
   const unsigned ab = (unsigned)((b_main * p.tpb + 127) / 128);
   const unsigned ab_tail = (unsigned)(((nbuckets - b_main) * pt.tpb + 127) / 128);
+  const auto accumulate = p.prepared ? k_msm_accumulate<true> : k_msm_accumulate<false>;
+  const auto accumulate_big = p.prepared ? k_msm_accumulate_big<true> : k_msm_accumulate_big<false>;
+  if (ab_tail) ST(side_fork(ctx));
+  accumulate<<<ab, 128, 0, ctx->stream>>>(p, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, (G1Pt*)buckets, (size_t)0, b_main);
   if (ab_tail) {
-    CU(cudaEventRecord(ctx->ev_chunk[2], ctx->stream));
-    CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_chunk[2], 0));
-  }
-  if (p.prepared) {
-    k_msm_accumulate<true><<<ab, 128, 0, ctx->stream>>>(p, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, (G1Pt*)buckets, (size_t)0, b_main);
-    if (ab_tail) k_msm_accumulate<true><<<ab_tail, 128, 0, ctx->copy_stream>>>(pt, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, (G1Pt*)buckets, b_main, nbuckets);
-  } else {
-    k_msm_accumulate<false><<<ab, 128, 0, ctx->stream>>>(p, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, (G1Pt*)buckets, (size_t)0, b_main);
-    if (ab_tail) k_msm_accumulate<false><<<ab_tail, 128, 0, ctx->copy_stream>>>(pt, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, (G1Pt*)buckets, b_main, nbuckets);
-  }
-  if (ab_tail) {
-    CU(cudaEventRecord(ctx->ev_chunk[3], ctx->copy_stream));
-    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk[3], 0));
+    accumulate<<<ab_tail, 128, 0, ctx->copy_stream>>>(pt, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, (G1Pt*)buckets, b_main, nbuckets);
+    ST(side_join(ctx));
     ctx->launches++;
   }
   LAUNCHED_AS(ctx, "msm_accumulate");
-  if (p.prepared) k_msm_accumulate_big<true><<<bigb, MSM_BIG_THREADS, 0, ctx->stream>>>(p, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, big_list, big_count, bigpart);
-  else k_msm_accumulate_big<false><<<bigb, MSM_BIG_THREADS, 0, ctx->stream>>>(p, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, big_list, big_count, bigpart);
+  accumulate_big<<<bigb, MSM_BIG_THREADS, 0, ctx->stream>>>(p, d_bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, big_list, big_count, bigpart);
   LAUNCHED_AS(ctx, "msm_accumulate_big");
   k_msm_big_combine<<<bigb, MSM_BIG_THREADS, 0, ctx->stream>>>(big_list, big_count, bigpart, (G1Pt*)buckets);
   LAUNCHED_AS(ctx, "msm_big_combine");
@@ -1791,7 +1747,7 @@ static vrfs_status msm_stateless_dev(vrfs_ctx* ctx, size_t n, int ncol, const vo
 }
 static vrfs_status msm_host(vrfs_ctx* ctx, size_t n, const uint8_t* bases, const uint8_t* scalars, int ncol, uint8_t* out, int out_mode, int window_bits = 0) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (ncol < 1 || ncol > 32) return fail(ctx, VRFS_BAD_ARG, "n_columns must be in 1..32");
   if (!out || (n && (!bases || !scalars))) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   const size_t ob = out_mode ? 144 : 96;
@@ -1825,7 +1781,7 @@ extern "C" vrfs_status vrfs_msm_g1_partial(vrfs_ctx* ctx, size_t n, const uint8_
 }
 static vrfs_status msm_prepare_impl(vrfs_ctx* ctx, size_t n, const uint8_t* bases, int window_bits, int threads_per_bucket, vrfs_msm_bases** out) {
   if (!ctx || !out) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   *out = nullptr;
   if (n == 0 || !bases) return fail(ctx, VRFS_BAD_ARG, "empty base vector");
   if (n > (1u << 24)) return fail(ctx, VRFS_BAD_ARG, "prepared MSM size above 2^24 is not supported");
@@ -1884,7 +1840,7 @@ extern "C" void vrfs_msm_g1_release(vrfs_msm_bases* h) {
   vrfs_ctx* ctx;
   { std::lock_guard<std::mutex> g(g_handles_mu); ctx = h->ctx; }
   if (ctx) {
-    CallGuard guard_(ctx); NvtxRange range_(__func__);
+    CallGuard guard_(ctx, __func__);
     std::lock_guard<std::mutex> g(g_handles_mu);
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
@@ -1902,7 +1858,7 @@ static void orphan_prepared(vrfs_ctx* ctx) {      // called by vrfs_ctx_destroy 
 }
 static vrfs_status msm_prepared_host(vrfs_ctx* ctx, const vrfs_msm_bases* h, const uint8_t* scalars, int n_columns, uint8_t* out, int out_mode) {
   if (!ctx || !h || h->ctx != ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n_columns < 1 || n_columns > 32 || !scalars || !out) return fail(ctx, VRFS_BAD_ARG, "bad argument");
   ST(begin_call(ctx, h->n));
   const size_t ob = out_mode ? 144 : 96;
@@ -1947,7 +1903,7 @@ static vrfs_status ntt_dev(vrfs_ctx* ctx, int logn, uint32_t ncol, int inverse, 
 }
 extern "C" vrfs_status vrfs_fr_fft_batch(vrfs_ctx* ctx, int log_n, int n_columns, int inverse, const uint8_t* in, uint8_t* out) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (log_n < 0 || log_n > 26 || n_columns < 1 || n_columns > 32 || !in || !out) return fail(ctx, VRFS_BAD_ARG, "bad argument (0 <= log_n <= 26, 1 <= n_columns <= 32)");
   const size_t bytes = ((size_t)n_columns << log_n) * 32;
   ST(begin_call(ctx, (size_t)1 << log_n));
@@ -1980,7 +1936,7 @@ static vrfs_status ring_columns_dev(vrfs_ctx* ctx, size_t n, size_t keyset_part,
 extern "C" vrfs_status vrfs_ring_fixed_columns(vrfs_ctx* ctx, size_t domain_size, size_t keyset_part_size, size_t n_keys, const uint8_t* keys,
                                                const uint8_t* padding, size_t n_tail, const uint8_t* tail, uint8_t* out_columns) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (!out_columns) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   ST(begin_call(ctx, domain_size));
   uint8_t* d_cols = nullptr;
@@ -1991,7 +1947,7 @@ extern "C" vrfs_status vrfs_ring_fixed_columns(vrfs_ctx* ctx, size_t domain_size
 extern "C" vrfs_status vrfs_ring_commit(vrfs_ctx* ctx, const vrfs_msm_bases* srs, int srs_is_lagrange, size_t keyset_part_size, size_t n_keys,
                                         const uint8_t* keys, const uint8_t* padding, size_t n_tail, const uint8_t* tail, uint8_t* out_commitment) {
   if (!ctx || !srs || srs->ctx != ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (!out_commitment) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   const size_t n = srs->n;
   ST(begin_call(ctx, n));
@@ -2010,7 +1966,7 @@ extern "C" vrfs_status vrfs_ring_commit(vrfs_ctx* ctx, const vrfs_msm_bases* srs
 extern "C" vrfs_status vrfs_ring_commit_rows_partial(vrfs_ctx* ctx, const vrfs_msm_bases* srs_rows, size_t row_lo, size_t keyset_part_size, size_t n_keys,
                                                      const uint8_t* keys_rows, const uint8_t* padding, size_t n_tail, const uint8_t* tail, uint8_t* out_partial) {
   if (!ctx || !srs_rows || srs_rows->ctx != ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (!out_partial) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   const size_t n = srs_rows->n;
   ST(begin_call(ctx, n));
@@ -2024,7 +1980,7 @@ extern "C" vrfs_status vrfs_ring_commit_rows_partial(vrfs_ctx* ctx, const vrfs_m
 extern "C" vrfs_status vrfs_ring_commit_delta(vrfs_ctx* ctx, const vrfs_msm_bases* srs_lagrange, size_t n_keys, const uint8_t* keys,
                                               const uint8_t* padding, uint8_t* out_delta) {
   if (!ctx || !srs_lagrange || srs_lagrange->ctx != ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   const size_t n = srs_lagrange->n;
   if (!out_delta || !padding || (n_keys && !keys) || n_keys > n) return fail(ctx, VRFS_BAD_ARG, "bad argument (n_keys <= domain size, non-null buffers)");
   ST(begin_call(ctx, n));
@@ -2042,7 +1998,7 @@ extern "C" vrfs_status vrfs_ring_commit_delta(vrfs_ctx* ctx, const vrfs_msm_base
 }
 extern "C" vrfs_status vrfs_g1_compress_batch(vrfs_ctx* ctx, size_t n, const uint8_t* points, uint8_t* out) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n && (!points || !out)) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   if (n == 0) return VRFS_OK;
   ST(begin_call(ctx, n));
@@ -2056,7 +2012,7 @@ extern "C" vrfs_status vrfs_g1_compress_batch(vrfs_ctx* ctx, size_t n, const uin
 }
 extern "C" vrfs_status vrfs_g1_decompress_batch(vrfs_ctx* ctx, size_t n, const uint8_t* enc, int check_subgroup, uint8_t* out_points, uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n && (!enc || !out_points || !out_ok)) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   if (n == 0) return VRFS_OK;
   ST(begin_call(ctx, n));
@@ -2095,7 +2051,7 @@ __global__ void k_fq381_inv_batch(uint32_t n, const uint8_t* in, uint8_t* out, u
 }
 extern "C" vrfs_status vrfs_fq381_inv_batch(vrfs_ctx* ctx, size_t n, const uint8_t* in, uint8_t* out, uint8_t* out_ok) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n && (!in || !out || !out_ok)) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   if (n == 0) return VRFS_OK;
   ST(begin_call(ctx, n));
@@ -2109,7 +2065,7 @@ extern "C" vrfs_status vrfs_fq381_inv_batch(vrfs_ctx* ctx, size_t n, const uint8
 }
 extern "C" vrfs_status vrfs_g1_sum_partials(vrfs_ctx* ctx, int n_parts, int n_columns, const uint8_t* partials, uint8_t* out) {
   if (!ctx) return VRFS_BAD_ARG;
-  CallGuard guard_(ctx); NvtxRange range_(__func__);
+  CallGuard guard_(ctx, __func__);
   if (n_parts < 1 || n_columns < 1 || n_columns > 32 || !partials || !out) return fail(ctx, VRFS_BAD_ARG, "bad argument");
   ST(begin_call(ctx, 1));
   const uint8_t* d_p; uint8_t* d_o;
