@@ -24,7 +24,7 @@ SYMBOLS = [
     "vrfs_ctx_peer_export", "vrfs_ctx_peer_connect", "vrfs_ctx_peer_set_timeout_ms", "vrfs_ctx_peer_world", "vrfs_msm_g1_prepared_allgather", "vrfs_ring_commit_rows_allgather",
     "vrfs_ctx_create_multi", "vrfs_mctx_destroy", "vrfs_mctx_device_count", "vrfs_mctx_device_ctx", "vrfs_mctx_last_error", "vrfs_mctx_launch_count",
     "vrfs_multi_ietf_verify_batch", "vrfs_multi_msm_g1_prepare", "vrfs_multi_msm_g1_prepared", "vrfs_multi_ring_commit", "vrfs_multi_msm_g1_release",
-    "vrfs_pairing_product_batch", "vrfs_kzg_batch_verify",
+    "vrfs_pairing_product_batch", "vrfs_kzg_batch_verify", "vrfs_pedersen_batch_verify", "vrfs_pedersen_batch_verify_wire",
     "vrfs_host_alloc", "vrfs_host_free", "vrfs_host_register", "vrfs_host_unregister",
     "vrfs_ring_fixed_columns", "vrfs_ring_commit", "vrfs_ring_commit_delta", "vrfs_ring_commit_rows_partial", "vrfs_fr_fft_batch", "vrfs_fq381_inv_batch", "vrfs_g1_compress_batch", "vrfs_g1_decompress_batch",
 ]

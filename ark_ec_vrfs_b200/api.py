@@ -219,6 +219,18 @@ def pedersen_verify_signatures(suite, datas, signatures, ad=None, status=False):
     return suite.engine.pedersen_verify_wire(suite.suite_id, datas, signatures, ad, status=status)
 
 
+def pedersen_batch_verify(suite, input, output, ad, proof, seed=None, per_item=False, status=False):
+    """all of a batch of Pedersen proofs (a PedersenProof) verified together by one random linear combination -> bool
+    (Bandersnatch only).  seed: 32 secret bytes, fresh per call (default os.urandom(32)).  per_item / status=True append the
+    per-item verdicts, which the per-item verifier computes only when the batch is rejected."""
+    return suite.engine.pedersen_batch_verify(suite.suite_id, input.points, output.points, proof.raw, ad, seed=seed, per_item=per_item, status=status)
+
+
+def pedersen_batch_verify_signatures(suite, datas, signatures, ad=None, seed=None, per_item=False, status=False):
+    """pedersen_batch_verify from serialised Output || pedersen::Proof signatures and VRF input data"""
+    return suite.engine.pedersen_batch_verify_wire(suite.suite_id, datas, signatures, ad, seed=seed, per_item=per_item, status=status)
+
+
 def ring_commitment_msm(suite_or_engine, bases, scalar_columns):
     """the three KZG commitments behind RingContext::verifier_key: one MSM per column over the SRS bases"""
     eng = suite_or_engine.engine if isinstance(suite_or_engine, Suite) else suite_or_engine

@@ -17,6 +17,7 @@
 #include "h2c.cuh"
 #include "wire.cuh"
 #include "msm.cuh"
+#include "te_msm.cuh"
 #include "ring.cuh"
 #include "pairing_coop.cuh"
 
@@ -235,7 +236,8 @@ struct DevBuf {
   size_t secret_bytes = 0;   // > 0: the running call put key material here (sk, nonces, blinding factors); zeroed before it returns
 };
 enum { BUF_IN0, BUF_IN1, BUF_IN2, BUF_IN3, BUF_IN4, BUF_AD, BUF_OFF, BUF_OUT0, BUF_OUT1, BUF_W0, BUF_W1, BUF_W2, BUF_W3, BUF_VALID, BUF_SLAB,
-       BUF_X0, BUF_X1, BUF_X2, BUF_X3, BUF_X4, BUF_X5, BUF_ZINV, BUF_SLAB2, BUF_COUNT };   // X*: wire-format staging (encoded keys, signatures, h2c data, flags)
+       BUF_X0, BUF_X1, BUF_X2, BUF_X3, BUF_X4, BUF_X5, BUF_ZINV, BUF_SLAB2,
+       BUF_PB0, BUF_PB1, BUF_PB2, BUF_COUNT };   // X*: wire-format staging (encoded keys, signatures, h2c data, flags); PB*: Pedersen batch verification
 
 #define MAX_TIMED 64
 #ifndef VRFS_HOST_PIECES
@@ -1517,18 +1519,27 @@ extern "C" vrfs_status vrfs_pedersen_sign_wire_batch(vrfs_ctx* ctx, vrfs_suite s
 }
 // deserialise NP encoded points + 2 scalars per item, then pedersen::Verifier::verify.  NP = 4: input = Input::new(data) here
 // (h2c flags in flags[(NP+1)n ..]); NP = 3: input and output are the caller's typed values.
-template <class S, int NP> static vrfs_status pedersen_verify_wire_dev(vrfs_ctx* ctx, size_t n, const uint8_t* data, const uint64_t* data_off, const uint8_t* sig, const uint8_t* ad,
-                                                                       const uint64_t* ad_off, uint8_t* input, uint8_t* output, uint8_t* proof256, uint8_t* flags /*(NP+2)n*/,
-                                                                       uint8_t* out_ok, uint8_t* out_status) {
+template <class S, int NP> static vrfs_status pedersen_wire_decode_dev(vrfs_ctx* ctx, size_t n, const uint8_t* data, const uint64_t* data_off, const uint8_t* sig,
+                                                                       uint8_t* input, uint8_t* output, uint8_t* proof256, uint8_t* flags /*(NP+2)n*/) {
   k_ped_wire_points<S, NP><<<item_blocks(NP * n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, sig, output, proof256, flags);
   LAUNCHED_AS(ctx, "decode_checked");
   k_ped_wire_scalars<S, NP><<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, sig, flags, proof256, flags + NP * n);
   LAUNCHED_AS(ctx, "ped_wire_scalars");
   if (NP == 4) ST(data_to_point_dev<S>(ctx, n, data, data_off, input, flags + (NP + 1) * n));
+  return VRFS_OK;
+}
+template <class S, int NP> static vrfs_status pedersen_wire_verdicts_dev(vrfs_ctx* ctx, size_t n, const uint8_t* ad, const uint64_t* ad_off, const uint8_t* input,
+                                                                         const uint8_t* output, const uint8_t* proof256, const uint8_t* flags, uint8_t* out_ok, uint8_t* out_status) {
   ST(pedersen_verify_dev<S>(ctx, n, input, output, proof256, ad, ad_off, out_ok, out_status));
   k_merge_flags<<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, flags + NP * n, NP == 4 ? flags + (NP + 1) * n : nullptr, out_ok, nullptr, 0u, out_status);
   LAUNCHED_AS(ctx, "merge_flags");
   return VRFS_OK;
+}
+template <class S, int NP> static vrfs_status pedersen_verify_wire_dev(vrfs_ctx* ctx, size_t n, const uint8_t* data, const uint64_t* data_off, const uint8_t* sig, const uint8_t* ad,
+                                                                       const uint64_t* ad_off, uint8_t* input, uint8_t* output, uint8_t* proof256, uint8_t* flags /*(NP+2)n*/,
+                                                                       uint8_t* out_ok, uint8_t* out_status) {
+  ST((pedersen_wire_decode_dev<S, NP>(ctx, n, data, data_off, sig, input, output, proof256, flags)));
+  return pedersen_wire_verdicts_dev<S, NP>(ctx, n, ad, ad_off, input, output, proof256, flags, out_ok, out_status);
 }
 extern "C" vrfs_status vrfs_pedersen_verify_wire_batch(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* data, const uint64_t* data_off, const uint8_t* sig,
                                                        const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
@@ -1604,6 +1615,246 @@ extern "C" vrfs_status vrfs_pedersen_verify_compressed_batch(vrfs_ctx* ctx, vrfs
   uint8_t *m_in = const_cast<uint8_t*>(d_in), *m_out = const_cast<uint8_t*>(d_out);
   ST(with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return (pedersen_verify_wire_dev<S, 3>(ctx, n, nullptr, nullptr, d_enc, d_ad, d_off, m_in, m_out, d_pr, d_flags, d_ok, d_st)); }));
   ST(copy_out(ctx, out_ok, d_ok, n));
+  if (out_status) ST(copy_out(ctx, out_status, d_st, n));
+  return finish_call(ctx);
+}
+
+// =================================================================================================
+// Pedersen batch verification by one random linear combination (Bandersnatch only; DESIGN §4 "Pedersen batch verification")
+// =================================================================================================
+//   E_i = Ok_i + c_i O_i - s_i I_i,   F_i = R_i + c_i Yb_i - s_i G - sb_i B      (both 0 for a valid proof)
+// The batch is accepted iff  sum_i rho_i E_i + sigma_i F_i = 0: one MSM (csrc/te_msm.cuh) over the 5n + 2 bases
+// [Ok, O, I, R, Yb of every item | G | B] with the scalars [rho, rho c, -rho s, sigma, sigma c | -sum sigma s | -sum sigma sb].
+// With every point in the prime-order subgroup a non-zero E_j or F_j survives all but one value of its coefficient (false accept
+// <= 2^-127); a 2-torsion component would vanish under every even one.  So the five points of every item are subgroup-checked
+// (typed inputs) or come from the checked wire decoder (`SUBGROUP` = false), and any failure sets the batch's `bad` flag.
+#define PED_BATCH_NP 5
+template <class S, bool SUBGROUP>
+__global__ void __launch_bounds__(ITEM_THREADS) k_pedersen_batch_prep(uint32_t n, uint32_t first, const uint8_t* input, const uint8_t* output, const uint8_t* proof,
+                                                                      const uint8_t* ad, const uint64_t* ad_off, const uint8_t* valid0, const uint8_t* valid1,
+                                                                      const uint8_t* seed, BandAff* bases, uint8_t* scal, uint32_t* prod, uint32_t* bad) {
+  ITEM_INDEX(n);
+  typedef typename S::C C;
+  typedef typename C::Fr R;
+  typedef Fp<R> Fr;
+  VAR_SLICE(ad, ad_off, i, a, alen);
+  const uint8_t* pr = proof + (size_t)256 * i;
+  const size_t g = (size_t)first + i;                              // index of the item in the whole batch
+  uint8_t c32[32];
+  bool ok = pedersen_verify_prep_item<S>(c32, input + (size_t)64 * i, output + (size_t)64 * i, pr, a, alen);
+  if (valid0) ok &= valid0[i] != 0;
+  if (valid1) ok &= valid1[i] != 0;
+  const uint8_t* pts[PED_BATCH_NP] = {pr + 128, output + (size_t)64 * i, input + (size_t)64 * i, pr + 64, pr};   // Ok, O, I, R, Yb
+  for (int j = 0; j < PED_BATCH_NP; j++) {
+    uint32_t rx[8], ry[8];
+    load_le<8>(rx, pts[j]); load_le<8>(ry, pts[j] + 32);
+    bool pok = is_canonical<typename C::Fq>(rx) & is_canonical<typename C::Fq>(ry);
+    const typename C::F x = to_mont<typename C::Fq>(rx), y = to_mont<typename C::Fq>(ry);
+    pok &= Grp<C>::on_curve(x, y);
+    if (SUBGROUP && pok) pok = SubgroupCheck<C>::run(x, y);
+    ok &= pok;
+    BandAff e; band_aff_from_xy(e, x, y);
+    copy_words16(&bases[PED_BATCH_NP * g + j], &e);
+  }
+  // (rho || sigma) = the first 32 bytes of SHA-512("vrfs-b200/pedersen-batch/v1" || seed || LE64(g) || c), two 16-byte
+  // little-endian halves with bit 127 cleared
+  constexpr char dom[] = "vrfs-b200/pedersen-batch/v1";
+  Sha512 h; h.init();
+  for (int k = 0; k + 1 < (int)sizeof(dom); k++) h.put((uint8_t)dom[k]);
+  h.update(seed, 32);
+  for (int k = 0; k < 8; k++) h.put((uint8_t)((uint64_t)g >> (8 * k)));
+  h.update(c32, 32);
+  uint8_t dig[64]; h.final(dig);
+  uint32_t raw[8];
+  Fr coef[2];
+  for (int half = 0; half < 2; half++) {
+    for (int k = 4; k < 8; k++) raw[k] = 0;
+    load_le<4>(raw, dig + 16 * half);
+    raw[3] &= 0x7fffffffu;
+    coef[half] = to_mont<R>(raw);
+  }
+  load_le<8>(raw, c32); const Fr c = to_mont<R>(raw);
+  load_le<8>(raw, pr + 192); const Fr s = to_mont<R>(raw);           // reduced mod r on load, as the per-item verifier does
+  load_le<8>(raw, pr + 224); const Fr sb = to_mont<R>(raw);
+  const Fr k5[PED_BATCH_NP] = {coef[0], coef[0] * c, neg(coef[0] * s), coef[1], coef[1] * c};
+  for (int j = 0; j < PED_BATCH_NP; j++) { from_mont<R>(raw, k5[j]); store_le<8>(scal + (size_t)32 * (PED_BATCH_NP * g + j), raw); }
+  const Fr ss = coef[1] * s, ssb = coef[1] * sb;
+  for (int w = 0; w < 8; w++) { prod[(size_t)16 * g + w] = ss.v[w]; prod[(size_t)16 * g + 8 + w] = ssb.v[w]; }
+  if (!ok) *bad = 1u;
+}
+// sum_i sigma_i s_i and sum_i sigma_i sb_i (Montgomery words, 16 per item): every block adds a strided slice into partial[block];
+// launched again as one block over those partials (`last`), which writes the scalars of G and B, -sum sigma s and -sum sigma sb mod r,
+// and their affine-cached records behind the nitems items
+__global__ void __launch_bounds__(256) k_pedersen_batch_sum(uint32_t n, const uint32_t* prod, uint32_t* partial, int last, uint32_t nitems, BandAff* bases, uint8_t* scal) {
+  typedef Fp<BandFr> Fr;
+  __shared__ uint32_t sh[256][16];
+  Fr a = Fr::zero(), b = Fr::zero();
+  for (uint32_t i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) {
+    Fr p, q;
+    for (int j = 0; j < 8; j++) { p.v[j] = prod[(size_t)16 * i + j]; q.v[j] = prod[(size_t)16 * i + 8 + j]; }
+    a = a + p; b = b + q;
+  }
+  for (int j = 0; j < 8; j++) { sh[threadIdx.x][j] = a.v[j]; sh[threadIdx.x][8 + j] = b.v[j]; }
+  __syncthreads();
+  for (int s = 128; s > 0; s >>= 1) {
+    if ((int)threadIdx.x < s) {
+      Fr p, q;
+      for (int j = 0; j < 8; j++) { p.v[j] = sh[threadIdx.x + s][j]; q.v[j] = sh[threadIdx.x + s][8 + j]; }
+      a = a + p; b = b + q;
+      for (int j = 0; j < 8; j++) { sh[threadIdx.x][j] = a.v[j]; sh[threadIdx.x][8 + j] = b.v[j]; }
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x != 0) return;
+  if (!last) { for (int j = 0; j < 8; j++) { partial[16 * blockIdx.x + j] = a.v[j]; partial[16 * blockIdx.x + 8 + j] = b.v[j]; } return; }
+  uint32_t out[8];
+  from_mont<BandFr>(out, neg(a)); store_le<8>(scal + (size_t)32 * (PED_BATCH_NP * (size_t)nitems), out);
+  from_mont<BandFr>(out, neg(b)); store_le<8>(scal + (size_t)32 * (PED_BATCH_NP * (size_t)nitems + 1), out);
+  BandAff e;
+  band_aff_from_xy(e, BandCurve::gx(), BandCurve::gy()); copy_words16(&bases[PED_BATCH_NP * (size_t)nitems], &e);
+  band_aff_from_xy(e, BandCurve::bx(), BandCurve::by()); copy_words16(&bases[PED_BATCH_NP * (size_t)nitems + 1], &e);
+}
+#define PED_BATCH_SUM_BLOCKS 1024
+
+// Device state of one batch verification, in slots of its own (BUF_PB*): a rejected batch runs the per-item verifier next, which
+// reuses the work buffers W*, VALID and SLAB but must find the staged inputs (IN*, AD, OFF, X*) intact.
+struct PedBatch { BandAff* bases; uint8_t* scal; uint32_t* prod; uint32_t* partial; uint32_t* bad; uint8_t* verdict; uint8_t* seed; };
+static vrfs_status ped_batch_begin(vrfs_ctx* ctx, vrfs_suite suite, size_t n) {
+  ST(begin_call(ctx, suite, n));
+  if (suite != VRFS_BANDERSNATCH_ELL2)
+    return fail(ctx, VRFS_UNSUPPORTED, "batch verification by random linear combination needs points of prime order, and only Bandersnatch has a cheap subgroup test "
+                                       "(the cofactor-8 curves need a full [r]P per point; short-Weierstrass curves have no bucket MSM here): use vrfs_pedersen_verify_batch");
+  if (n > (1u << 24)) return fail(ctx, VRFS_BAD_ARG, "more than 2^24 proofs per batch verification are not supported");
+  return VRFS_OK;
+}
+static vrfs_status ped_batch_alloc(vrfs_ctx* ctx, size_t n, const uint8_t* seed, PedBatch* B) {
+  const size_t nbases = PED_BATCH_NP * n + 2;
+  void *b = nullptr, *s = nullptr, *m = nullptr;
+  ST(ensure(ctx, BUF_PB0, nbases * sizeof(BandAff), &b));
+  ST(ensure(ctx, BUF_PB1, nbases * 32, &s));
+  ST(ensure(ctx, BUF_PB2, 256 + (n + PED_BATCH_SUM_BLOCKS) * 64, &m));   // seed (32 B) | bad flag | verdict | ... | prod (n x 16 words) | partial sums
+  B->bases = (BandAff*)b; B->scal = (uint8_t*)s;
+  B->seed = (uint8_t*)m; B->bad = (uint32_t*)((uint8_t*)m + 32); B->verdict = (uint8_t*)m + 48; B->prod = (uint32_t*)((uint8_t*)m + 256);
+  B->partial = B->prod + 16 * n;
+  mark_secret(ctx, BUF_PB2, 32);                                   // the seed: zeroed when the call returns
+  CU(cudaMemcpyAsync(B->seed, seed, 32, cudaMemcpyHostToDevice, ctx->stream));
+  CU(cudaMemsetAsync(B->bad, 0, 16, ctx->stream));
+  return VRFS_OK;
+}
+// the MSM of the combination and its identity test: *verdict = 1 iff the sum is the identity and *bad = 0
+static vrfs_status te_msm_verdict_dev(vrfs_ctx* ctx, size_t nbases, const BandAff* bases, const uint8_t* scal, const uint32_t* bad, uint8_t* verdict) {
+  const MsmPlan p = te_msm_plan((uint32_t)nbases);
+  const size_t nbuckets = (size_t)p.windows * p.nb, runs = (size_t)p.windows * (p.nb / TE_MSM_CHUNK);
+  void *counts = nullptr, *list = nullptr, *buckets = nullptr, *sums = nullptr;
+  // counts | offsets | cursors | big_count (16 words) | big_list (never written: te_msm_plan lists no oversized bucket)
+  ST(ensure(ctx, BUF_W1, (nbuckets * 3 + 16 + 2) * sizeof(uint32_t), &counts));
+  uint32_t *offsets = (uint32_t*)counts + nbuckets, *cursors = offsets + nbuckets, *big_count = cursors + nbuckets, *big_list = big_count + 16;
+  ST(ensure(ctx, BUF_W2, (size_t)p.windows * nbases * sizeof(uint32_t), &list));
+  ST(ensure(ctx, BUF_W3, nbuckets * sizeof(BandPt), &buckets));
+  ST(ensure(ctx, BUF_SLAB, (runs + (size_t)p.windows) * sizeof(BandPt), &sums));
+  CU(cudaMemsetAsync(counts, 0, (nbuckets * 3 + 16) * sizeof(uint32_t), ctx->stream));
+  const unsigned tsc = (unsigned)((nbases + 127) / 128);
+  k_msm_histogram<<<tsc, 128, 0, ctx->stream>>>(p, scal, (uint32_t*)counts);
+  LAUNCHED_AS(ctx, "te_msm_histogram");
+  k_msm_scan<<<(unsigned)p.windows, MSM_SCAN_THREADS, 0, ctx->stream>>>(p, (const uint32_t*)counts, offsets, big_list, big_count);
+  LAUNCHED_AS(ctx, "te_msm_scan");
+  k_msm_scatter<<<tsc, 128, 0, ctx->stream>>>(p, scal, offsets, cursors, (uint32_t*)list);
+  LAUNCHED_AS(ctx, "te_msm_scatter");
+  k_te_msm_accumulate<<<(unsigned)((nbuckets * p.tpb + 127) / 128), 128, 0, ctx->stream>>>(p, bases, (const uint32_t*)counts, offsets, (const uint32_t*)list, (BandPt*)buckets);
+  LAUNCHED_AS(ctx, "te_msm_accumulate");
+  k_te_msm_chunks<<<(unsigned)((runs + 127) / 128), 128, 0, ctx->stream>>>(p, (const BandPt*)buckets, (BandPt*)sums);
+  LAUNCHED_AS(ctx, "te_msm_chunks");
+  BandPt* wsum = (BandPt*)sums + runs;
+  k_te_msm_window_sum<<<(unsigned)p.windows, TE_MSM_WSUM_THREADS, 0, ctx->stream>>>(p, (const BandPt*)sums, wsum);
+  LAUNCHED_AS(ctx, "te_msm_window_sum");
+  k_te_msm_final<<<1, 32, 0, ctx->stream>>>(p, wsum, bad, verdict);
+  LAUNCHED_AS(ctx, "te_msm_final");
+  return VRFS_OK;
+}
+// after the prep kernels of all items: scalars of G and B, the MSM, and the verdict back to the host (synchronous)
+static vrfs_status ped_batch_verdict(vrfs_ctx* ctx, size_t n, const PedBatch& B, uint8_t* out_all_ok) {
+  const unsigned blocks = (unsigned)std::min((size_t)PED_BATCH_SUM_BLOCKS, (n + 255) / 256);
+  k_pedersen_batch_sum<<<blocks, 256, 0, ctx->stream>>>((uint32_t)n, B.prod, B.partial, 0, 0u, nullptr, nullptr);
+  LAUNCHED_AS(ctx, "pedersen_batch_sum");
+  k_pedersen_batch_sum<<<1, 256, 0, ctx->stream>>>(blocks, B.partial, nullptr, 1, (uint32_t)n, B.bases, B.scal);
+  LAUNCHED_AS(ctx, "pedersen_batch_sum_final");
+  ST(te_msm_verdict_dev(ctx, PED_BATCH_NP * n + 2, B.bases, B.scal, B.bad, B.verdict));
+  ST(copy_out(ctx, out_all_ok, B.verdict, 1));
+  return finish_call(ctx);
+}
+static void ped_batch_all_ok(size_t n, uint8_t* out_ok, uint8_t* out_status) {
+  if (out_ok) memset(out_ok, 1, n);
+  if (out_status) memset(out_status, VRFS_ITEM_OK, n);
+}
+
+extern "C" vrfs_status vrfs_pedersen_batch_verify(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* input, const uint8_t* output, const uint8_t* proof,
+                                                  const uint8_t* ad, const uint64_t* ad_off, const uint8_t* seed, uint8_t* out_all_ok, uint8_t* out_ok, uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  if (!seed || !out_all_ok || (n && (!input || !output || !proof))) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  *out_all_ok = n == 0;
+  if (n == 0) return VRFS_OK;
+  ST(ped_batch_begin(ctx, suite, n));
+  typedef BandSuite S;
+  const uint8_t* d_ad; const uint64_t* d_off;
+  // in pieces: the prep kernel of piece k runs while piece k + 1 (384 B per item) is still on its way
+  HostIn in[3] = {{BUF_IN0, input, 64, false, nullptr}, {BUF_IN1, output, 64, false, nullptr}, {BUF_IN2, proof, 256, false, nullptr}};
+  Pieces pc;
+  ST(stage_in_pieces(ctx, n, in, 3, &pc, VRFS_HOST_PIECES));
+  ST(stage_ad(ctx, n, ad, ad_off, &d_ad, &d_off));
+  PedBatch B;
+  ST(ped_batch_alloc(ctx, n, seed, &B));
+  for (int k = 0; k < pc.count; k++) {
+    const size_t o = pc.cut[k], m = pc.cut[k + 1] - pc.cut[k];
+    ST(piece_ready(ctx, k));
+    k_pedersen_batch_prep<S, true><<<item_blocks(m), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)m, (uint32_t)o, in[0].dev + o * 64, in[1].dev + o * 64, in[2].dev + o * 256,
+                                                                                     d_ad, d_off ? d_off + o : nullptr, nullptr, nullptr, B.seed, B.bases, B.scal, B.prod, B.bad);
+    LAUNCHED_AS(ctx, "pedersen_batch_prep");
+  }
+  ST(ped_batch_verdict(ctx, n, B, out_all_ok));
+  if (*out_all_ok) { ped_batch_all_ok(n, out_ok, out_status); return VRFS_OK; }
+  if (!out_ok && !out_status) return VRFS_OK;
+  // rejected: the per-item verifier over the inputs already on the device (exactly what vrfs_pedersen_verify_batch returns)
+  uint8_t *d_ok, *d_st = nullptr;
+  ST(stage_out(ctx, BUF_OUT0, n, &d_ok));
+  if (out_status) ST(stage_out(ctx, BUF_OUT1, n, &d_st));
+  ST(pedersen_verify_dev<S>(ctx, n, in[0].dev, in[1].dev, in[2].dev, d_ad, d_off, d_ok, d_st));
+  if (out_ok) ST(copy_out(ctx, out_ok, d_ok, n));
+  if (out_status) ST(copy_out(ctx, out_status, d_st, n));
+  return finish_call(ctx);
+}
+extern "C" vrfs_status vrfs_pedersen_batch_verify_wire(vrfs_ctx* ctx, vrfs_suite suite, size_t n, const uint8_t* data, const uint64_t* data_off, const uint8_t* sig,
+                                                       const uint8_t* ad, const uint64_t* ad_off, const uint8_t* seed, uint8_t* out_all_ok, uint8_t* out_ok, uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  if (!seed || !out_all_ok || (n && (!data_off || !sig))) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  *out_all_ok = n == 0;
+  if (n == 0) return VRFS_OK;
+  ST(ped_batch_begin(ctx, suite, n));
+  typedef BandSuite S;
+  const size_t sl = (size_t)vrfs_suite_pedersen_signature_len(suite);
+  const uint8_t *d_sig, *d_ad, *d_data; const uint64_t *d_off, *d_doff;
+  uint8_t *d_in, *d_out, *d_pr, *d_flags;
+  ST(stage_in(ctx, BUF_X1, sig, n * sl, &d_sig));
+  ST(stage_ad(ctx, n, ad, ad_off, &d_ad, &d_off));
+  ST(stage_var(ctx, BUF_X2, BUF_X3, n, data, data_off, &d_data, &d_doff));
+  ST(stage_out(ctx, BUF_IN0, n * 64, &d_in)); ST(stage_out(ctx, BUF_IN1, n * 64, &d_out)); ST(stage_out(ctx, BUF_IN2, n * 256, &d_pr));
+  ST(stage_out(ctx, BUF_X4, 6 * n, &d_flags));
+  ST((pedersen_wire_decode_dev<S, 4>(ctx, n, d_data, d_doff, d_sig, d_in, d_out, d_pr, d_flags)));
+  PedBatch B;
+  ST(ped_batch_alloc(ctx, n, seed, &B));
+  // the decoder has subgroup-checked the output and the proof's points, and hash-to-curve lands in the subgroup
+  k_pedersen_batch_prep<S, false><<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, 0u, d_in, d_out, d_pr, d_ad, d_off, d_flags + 4 * n, d_flags + 5 * n,
+                                                                                    B.seed, B.bases, B.scal, B.prod, B.bad);
+  LAUNCHED_AS(ctx, "pedersen_batch_prep_wire");
+  ST(ped_batch_verdict(ctx, n, B, out_all_ok));
+  if (*out_all_ok) { ped_batch_all_ok(n, out_ok, out_status); return VRFS_OK; }
+  if (!out_ok && !out_status) return VRFS_OK;
+  uint8_t *d_ok, *d_st = nullptr;
+  ST(stage_out(ctx, BUF_OUT0, n, &d_ok));
+  if (out_status) ST(stage_out(ctx, BUF_OUT1, n, &d_st));
+  ST((pedersen_wire_verdicts_dev<S, 4>(ctx, n, d_ad, d_off, d_in, d_out, d_pr, d_flags, d_ok, d_st)));
+  if (out_ok) ST(copy_out(ctx, out_ok, d_ok, n));
   if (out_status) ST(copy_out(ctx, out_status, d_st, n));
   return finish_call(ctx);
 }

@@ -1,6 +1,7 @@
 """Batch engine: a thin, typed wrapper over the C ABI (include/vrfs_b200.h).  Array conventions are the
 ABI's: scalars (n,32) uint8 little-endian, points (n,64) uint8 affine x||y little-endian."""
 import ctypes as C
+import os
 
 import numpy as np
 
@@ -350,6 +351,28 @@ class Engine:
         ok = np.zeros(n, np.uint8); st = np.zeros(n, np.uint8) if status else None
         self._call("vrfs_pedersen_verify_batch", suite, C.c_size_t(n), _p(inp), _p(outp), _p(proof), _p(adb), _p(off), _p(ok), _p(st))
         return (ok, st) if status else ok
+
+    def _batch_verify(self, fn, n, args, seed, per_item, status):
+        seed = _u8(os.urandom(32) if seed is None else seed, (32,))
+        all_ok = np.zeros(1, np.uint8)
+        ok = np.zeros(n, np.uint8) if per_item else None
+        st = np.zeros(n, np.uint8) if status else None
+        self._call(fn, *args, _p(seed), _p(all_ok), _p(ok), _p(st))
+        res = (bool(all_ok[0]),) + ((ok,) if per_item else ()) + ((st,) if status else ())
+        return res if len(res) > 1 else res[0]
+
+    def pedersen_batch_verify(self, suite, inp, outp, proof, ad=None, seed=None, per_item=False, status=False):
+        """Bandersnatch Pedersen proofs checked together by one random linear combination (vrfs_pedersen_batch_verify) -> all_ok.
+        seed: 32 secret bytes (default: os.urandom(32)).  per_item / status=True append the per-item ok flags / vrfs_item_status,
+        which are computed by the per-item verifier only when the batch is rejected."""
+        inp = _u8(inp, (-1, 64)); n = len(inp); outp = _u8(outp, (n, 64)); proof = _u8(proof, (n, 256))
+        adb, off = pack_var(ad, n)
+        return self._batch_verify("vrfs_pedersen_batch_verify", n, (suite, C.c_size_t(n), _p(inp), _p(outp), _p(proof), _p(adb), _p(off)), seed, per_item, status)
+
+    def pedersen_batch_verify_wire(self, suite, datas, sig, ad=None, seed=None, per_item=False, status=False):
+        """pedersen_batch_verify from serialised signatures (the layout of pedersen_verify_wire)"""
+        sig = _u8(sig, (-1, self.pedersen_signature_len(suite))); n = len(sig); data, doff = pack_var(datas, n); adb, off = pack_var(ad, n)
+        return self._batch_verify("vrfs_pedersen_batch_verify_wire", n, (suite, C.c_size_t(n), _p(data), _p(doff), _p(sig), _p(adb), _p(off)), seed, per_item, status)
 
     def pedersen_proof_len(self, suite):
         return int(self._lib.vrfs_suite_pedersen_proof_len(suite))

@@ -164,6 +164,29 @@ vrfs_status vrfs_pedersen_sign_wire_batch(vrfs_ctx*, vrfs_suite, size_t n, const
 vrfs_status vrfs_pedersen_verify_wire_batch(vrfs_ctx*, vrfs_suite, size_t n, const uint8_t* data, const uint64_t* data_off, const uint8_t* sig /*n*sig_len*/,
                                             const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status /* may be NULL */);
 
+/* Batch verification of pedersen::Verifier::verify by one random linear combination (Bandersnatch only).
+ * With E_i = Ok_i + c_i O_i - s_i I_i and F_i = R_i + c_i Yb_i - s_i G - sb_i B (both 0 for a valid proof), the batch is accepted
+ * iff sum_i rho_i E_i + sigma_i F_i = 0, one multi-scalar multiplication over the 5n + 2 points instead of 2n per-item ones.
+ * Coefficients: (rho_i || sigma_i) = the first 32 bytes of SHA-512("vrfs-b200/pedersen-batch/v1" || seed || LE64(i) || c_i), c_i the
+ * proof's challenge as 32 little-endian bytes; each 16-byte half is read little-endian with its top bit cleared (rho_i, sigma_i < 2^127).
+ * seed: 32 secret bytes, fresh per call (whoever made the proofs must not know them).
+ * Every point (I, O, Yb, R, Ok) must lie in the prime-order subgroup, or a torsion component can vanish from the sum; the call tests
+ * that for every item and counts a point outside the subgroup as a failure.  Other suites return VRFS_UNSUPPORTED: their cofactor-8
+ * subgroup test costs more than the batch saves, and short-Weierstrass curves have no bucket path here.
+ * *out_all_ok = 1  => every item verifies (false accept <= 2^-127 per call when the seed is secret);
+ * *out_all_ok = 0  => at least one item fails, is invalid, or has a point outside the prime-order subgroup.
+ * out_ok / out_status (each may be NULL): all 1 / VRFS_ITEM_OK when *out_all_ok = 1; otherwise the call runs the
+ * per-item verifier and returns exactly what vrfs_pedersen_verify_batch returns for the same arguments.
+ * n = 0: VRFS_OK with *out_all_ok = 1.  At most 2^24 proofs per call. */
+vrfs_status vrfs_pedersen_batch_verify(vrfs_ctx*, vrfs_suite, size_t n, const uint8_t* input, const uint8_t* output,
+                                       const uint8_t* proof /*n*256*/, const uint8_t* ad, const uint64_t* ad_off,
+                                       const uint8_t* seed /*32*/, uint8_t* out_all_ok, uint8_t* out_ok, uint8_t* out_status);
+/* the same from serialised signatures (Output || pedersen::Proof, the layout of vrfs_pedersen_verify_wire_batch); their points are
+ * subgroup-checked by the decoder, and out_ok / out_status of a rejected batch are what vrfs_pedersen_verify_wire_batch returns */
+vrfs_status vrfs_pedersen_batch_verify_wire(vrfs_ctx*, vrfs_suite, size_t n, const uint8_t* data, const uint64_t* data_off,
+                                            const uint8_t* sig /*n*sig_len*/, const uint8_t* ad, const uint64_t* ad_off,
+                                            const uint8_t* seed /*32*/, uint8_t* out_all_ok, uint8_t* out_ok, uint8_t* out_status);
+
 /* ring commitment MSM (ark-ec VariableBaseMSM::msm behind ring-proof's KZG commit, SURVEY 3.5):
  * n_columns scalar columns (column-major, n*32 bytes each) over one base vector of n affine G1 points.
  * out: n_columns * 96 bytes affine.

@@ -12,6 +12,7 @@
 #pragma once
 #include <array>
 #include <cstdint>
+#include <random>
 #include <stdexcept>
 #include <string>
 #include <utility>
@@ -222,6 +223,22 @@ inline Bytes verify(const Suite& s, const Input& input, const Output& output, co
   s.engine->check(vrfs_pedersen_verify_compressed_batch(s.engine->ctx(), s.id, n, input.xy.data(), output.xy.data(), proof.bytes.data(), a.ptr(), a.off.data(),
                                                         ok.data(), status_ptr(errors, n)));
   return ok;
+}
+// all proofs verified together by one random linear combination (vrfs_pedersen_batch_verify; Bandersnatch only): true iff every
+// item verifies.  The 32-byte seed comes from std::random_device and is never shown to the caller (whoever made the proofs must not
+// know it).  ok / errors (optional): per-item verdicts, all ok when the batch is accepted, else those of verify() above.
+inline bool batch_verify(const Suite& s, const Input& input, const Output& output, const std::vector<Bytes>& ad, const Proof& proof,
+                         Bytes* ok = nullptr, Errors* errors = nullptr) {
+  Packed a(ad); size_t n = input.size();
+  std::random_device rd;
+  std::array<uint8_t, 32> seed;
+  for (size_t i = 0; i < seed.size(); i += 4) { const uint32_t w = rd(); for (int k = 0; k < 4; k++) seed[i + k] = (uint8_t)(w >> (8 * k)); }
+  if (ok) ok->assign(n, 0);
+  uint8_t all_ok = 0;
+  s.engine->check(vrfs_pedersen_batch_verify(s.engine->ctx(), s.id, n, input.xy.data(), output.xy.data(), proof.raw.data(), a.ptr(),
+                                             ad.empty() ? nullptr : a.off.data(), seed.data(), &all_ok, ok ? ok->data() : nullptr, status_ptr(errors, n)));
+  seed.fill(0);
+  return all_ok != 0;
 }
 }  // namespace pedersen
 
