@@ -69,6 +69,10 @@ class Public:
 
     serialize_compressed = encode
 
+    def prepare(self):
+        """these keys prepared once for many verifies (per-key fixed-base tables on the suite's GPU) -> PreparedPublic"""
+        return PreparedPublic(self.suite, self.suite.engine.public_keys_prepare(self.suite.suite_id, self.points))
+
     @classmethod
     def deserialize_compressed(cls, suite, enc):
         """CanonicalDeserialize with validation (canonical, on curve, prime-order subgroup) -> (Public, ok flags)"""
@@ -80,6 +84,32 @@ class Public:
         """serialised keys + VRF input data + serialised signatures (Output || ietf::Proof) -> (ok flags, Output::hash[, status]);
         one call: deserialise, Input::new, verify, hash"""
         return suite.engine.ietf_verify_wire(suite.suite_id, pk_enc, datas, signatures, ad, status=status)
+
+
+@dataclass
+class PreparedPublic:
+    """a Public that is reused (Public.prepare): verify takes, per proof, the index of its key among the prepared ones"""
+    suite: Suite
+    keys: object                # engine.PreparedPublics
+
+    @property
+    def key_ok(self):
+        """1 where the key is one Public.verify accepts"""
+        return self.keys.key_ok
+
+    def verify(self, key_index, input, output, ad, proof, status=False):
+        """ietf::Verifier::verify with pk[i] = keys[key_index[i]] -> uint8[n] (status=True: (ok, Error variant per item));
+        an index out of range is ITEM_INVALID_DATA for its item"""
+        return self.keys.verify(key_index, input.points, output.points, proof.c, proof.s, ad, status=status)
+
+    def release(self):
+        self.keys.release()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.release()
 
 
 @dataclass

@@ -72,6 +72,7 @@ template <class C> struct Grp<C, true> {
   static constexpr int WINDOWS = C::HAS_GLV ? 32 : 64;      // radix-16 windows per (half-)scalar
   static constexpr int KB_LIMBS = C::HAS_GLV ? 4 : 8;
   static constexpr int FIX_WINDOWS = 256 / VRFS_FIX_BITS;
+  static constexpr int CARRY_WINDOWS = 0;   // r < 2^255: the bias addition never carries out of a 256-bit scalar
   static HD_INLINE void set_identity(Pt& P) { te_set_identity(P); }
   static HD_INLINE void from_affine(Pt& P, const typename C::F& x, const typename C::F& y) { te_from_affine<C>(P, x, y); }
   static HD_INLINE bool on_curve(const typename C::F& x, const typename C::F& y) { return te_on_curve<C>(x, y); }
@@ -91,6 +92,13 @@ template <class C> struct Grp<C, true> {
     else { e.x = x; e.y = y; e.dt = dt; }
   }
   static HD_INLINE void store_xyz(uint32_t* o, const Pt& P) { store_fp_xyz(o, P.X, P.Y, P.Z); }
+  // prepared-key tables: the point (X : Y : Z) (T dropped) back in extended coordinates, and an affine point as a table entry
+  static HD_INLINE void from_xyz(Pt& P, const typename C::F& X, const typename C::F& Y, const typename C::F& Z) { P.X = X * Z; P.Y = Y * Z; P.Z = sqr(Z); P.T = X * Y; }
+  static HD_INLINE void fix_from_affine(FixEntry& e, const typename C::F& x, const typename C::F& y, bool) {
+    typename C::F dt = x * y * C::d();
+    if constexpr (C::A_IS_M1) { e.x = y + x; e.y = y - x; e.dt = dt + dt; }
+    else { e.x = x; e.y = y; e.dt = dt; }
+  }
 };
 template <class C> struct Grp<C, false> {
   typedef SWPoint<C> Pt;
@@ -100,6 +108,7 @@ template <class C> struct Grp<C, false> {
   static constexpr int WINDOWS = 65;       // 64 radix-16 digits + the carry of the bias addition (n ~ 2^256)
   static constexpr int KB_LIMBS = 9;
   static constexpr int FIX_WINDOWS = 256 / VRFS_FIX_BITS + 1;   // + the carry of the bias addition (n ~ 2^256)
+  static constexpr int CARRY_WINDOWS = 1;
   static HD_INLINE void set_identity(Pt& P) { sw_set_identity(P); }
   static HD_INLINE void from_affine(Pt& P, const typename C::F& x, const typename C::F& y) { sw_from_affine<C>(P, x, y); }
   static HD_INLINE bool on_curve(const typename C::F& x, const typename C::F& y) { return sw_on_curve<C>(x, y); }
@@ -119,6 +128,10 @@ template <class C> struct Grp<C, false> {
     e.X = P.X * zi; e.Y = select(inf, C::F::one(), P.Y * zi); e.Z = select(inf, C::F::zero(), C::F::one());
   }
   static HD_INLINE void store_xyz(uint32_t* o, const Pt& P) { store_fp_xyz(o, P.X, P.Y, P.Z); }
+  static HD_INLINE void from_xyz(Pt& P, const typename C::F& X, const typename C::F& Y, const typename C::F& Z) { P.X = X; P.Y = Y; P.Z = Z; }
+  static HD_INLINE void fix_from_affine(FixEntry& e, const typename C::F& x, const typename C::F& y, bool inf) {
+    e.X = select(inf, C::F::zero(), x); e.Y = select(inf, C::F::one(), y); e.Z = select(inf, C::F::zero(), C::F::one());
+  }
 };
 #ifndef VRFS_SKIP_T
 #define VRFS_SKIP_T 1                     // do not compute the T coordinate of sums nobody reads (one product per window)
@@ -194,6 +207,42 @@ template <class C> HD_INLINE void build_table(typename Grp<C>::Entry* tbl, const
   }
 }
 
+// acc += (-1)^neg * k * B, k = the 32-byte scalar at `sc` reduced mod r, over a signed radix-2^BITS table of B
+// (fix_windows<C, BITS>() windows of (1 << (BITS - 1)) + 1 entries d * 2^(BITS w) * B).  Windows above `topw` are skipped: the caller
+// knows that they hold no digit (warp-uniform).  last: nothing follows this term, so its last sum needs no T coordinate.
+// FAR: the table is far larger than L1 - start every window's record on its way to L2 before the first addition.
+// (lincomb_item keeps its own copy of this loop for VRFS_FIX_BITS: calling this one from there changes the code of its kernels.)
+template <class C, int BITS> VRFS_HD constexpr int fix_windows() { return 256 / BITS + Grp<C>::CARRY_WINDOWS; }
+template <class C, int BITS, bool FAR>
+HD_INLINE void add_fixed_term(typename Grp<C>::Pt& acc, const uint8_t* sc, const void* table, bool neg, int topw, bool last) {
+  typedef Grp<C> G;
+  constexpr int ENTRIES = (1 << (BITS - 1)) + 1;
+  uint32_t k[9];
+  load_scalar_mod_r<C>(k, sc);
+  k[8] = 0;
+  add_window_bias<9>(k, BITS == 16 ? 0x80008000u : 0x80808080u, 8);
+  const typename G::FixEntry* tbl = reinterpret_cast<const typename G::FixEntry*>(table);
+  constexpr int TOPW = 256 / BITS;              // index of the carry window (short-Weierstrass suites only)
+  auto digit = [&](int w) { return w == TOPW ? (int)k[8] : (BITS == 16 ? digit16(k, w) : digit8(k, w)); };
+  if (FAR) {
+#pragma unroll 1
+    for (int w = 2; w <= topw; w++) { int dn = digit(w); prefetch_l2(&tbl[(size_t)w * ENTRIES + (dn < 0 ? -dn : dn)], sizeof(typename G::FixEntry)); }
+    { int dn = digit(0); prefetch_l1(&tbl[(dn < 0 ? -dn : dn)], sizeof(typename G::FixEntry)); }
+  }
+#pragma unroll 1
+  for (int w = 0; w <= topw; w++) {
+    if (w + 1 <= topw) {              // next window's entry -> L1 while this addition runs
+      int dn = digit(w + 1);
+      prefetch_l1(&tbl[(size_t)(w + 1) * ENTRIES + (dn < 0 ? -dn : dn)], sizeof(typename G::FixEntry));
+    }
+    int d = digit(w);
+    int idx = d < 0 ? -d : d;
+    typename G::FixEntry e;
+    copy_words16(&e, &tbl[(size_t)w * ENTRIES + idx]);
+    G::add_fix(&acc, &e, (d < 0) != neg, VRFS_SKIP_T ? (!last || w != topw) : true);
+  }
+}
+
 template <class C, int NV, int NF>
 HD_INLINE bool lincomb_item(const LincombArgs& A, uint32_t item, typename Grp<C>::Entry* slab, typename Grp<C>::Pt& acc) {
   typedef Grp<C> G;
@@ -261,6 +310,8 @@ HD_INLINE bool lincomb_item(const LincombArgs& A, uint32_t item, typename Grp<C>
       }
     }
   }
+  // fixed bases.  add_fixed_term below is the same loop with the window width and the top window as parameters (prepared keys);
+  // keep the two in step - this copy stays because routing it through add_fixed_term changes the code of these kernels
 #pragma unroll
   for (int f = 0; f < NF; f++) {
     uint32_t k[9];
@@ -292,6 +343,35 @@ HD_INLINE bool lincomb_item(const LincombArgs& A, uint32_t item, typename Grp<C>
   return ok;
 }
 
+// ---- prepared keys: a per-key fixed-base table of 8-bit windows --------------------------------------------------------------
+// U = s*G - c*Y_k of an IETF verify against a known key: two fixed-base terms and no variable base (no slab, no doublings).
+static constexpr int KEY_FIX_BITS = 8;
+static constexpr int KEY_ENTRIES = (1 << (KEY_FIX_BITS - 1)) + 1;   // 0 .. 128 times 256^w * Y
+template <class C> VRFS_HD constexpr size_t key_table_entries() { return (size_t)fix_windows<C, KEY_FIX_BITS>() * KEY_ENTRIES; }
+struct KeyedArgs {
+  uint32_t n;
+  const uint8_t* s;             // n x 32: s of s*G (G: the context's table of VRFS_FIX_BITS windows)
+  const uint8_t* c;             // n x 32: c of -c*Y_k
+  uint32_t c_bits;              // bound on c's bit length (8 * CHALLENGE_LEN), 0 = full width
+  const uint32_t* key_index;    // n: k of item i (>= n_keys: the table of key 0 is read; the gather kernel rejects the item)
+  uint32_t n_keys;
+  const void* g_table;
+  const void* key_tables;       // n_keys x key_table_entries<C>() FixEntry
+  uint32_t* out_xyz;            // n x 3N limbs
+};
+template <class C> HD_INLINE void lincomb_keyed_item(const KeyedArgs& A, uint32_t item, typename Grp<C>::Pt& acc) {
+  typedef Grp<C> G;
+  uint32_t k = A.key_index[item];
+  if (k >= A.n_keys) k = 0;
+  const int topw_c = A.c_bits != 0 && (int)(A.c_bits / KEY_FIX_BITS) < fix_windows<C, KEY_FIX_BITS>() - 1 ? (int)(A.c_bits / KEY_FIX_BITS)
+                                                                                                        : fix_windows<C, KEY_FIX_BITS>() - 1;
+  G::set_identity(acc);
+  add_fixed_term<C, VRFS_FIX_BITS, VRFS_FIX_BITS == 16>(acc, A.s + (size_t)item * 32, A.g_table, false, fix_windows<C, VRFS_FIX_BITS>() - 1, false);
+  // n_keys x 400 KB is DRAM-resident beyond a few hundred keys: the records of all windows go to L2 up front, as for the G table
+  add_fixed_term<C, KEY_FIX_BITS, true>(acc, A.c + (size_t)item * 32,
+                                        reinterpret_cast<const typename G::FixEntry*>(A.key_tables) + (size_t)k * key_table_entries<C>(), true, topw_c, true);
+}
+
 // one fixed-base table entry: (d * 256^w) * B.  Used once per context by the table kernel.
 template <class C>
 HD_INLINE void fixed_table_entry(typename Grp<C>::FixEntry& out, const typename C::F& bx, const typename C::F& by, int w, int d) {
@@ -304,6 +384,62 @@ HD_INLINE void fixed_table_entry(typename Grp<C>::FixEntry& out, const typename 
     if ((d >> bit) & 1) G::add(&R, &R, &P);
   }
   G::to_fix(out, R);
+}
+
+// Prepared-key tables, layout [key][window][entry]: entry d of window w is d * 256^w * Y.  k_fixed_table's scheme (a doubling
+// chain of its own per entry) is fine for two bases and far too slow for millions of entries; instead
+//  1. key_table_powers: one doubling chain per key gives 256^w * Y for every w, parked as (X : Y : Z) in entry 1 of window w;
+//  2. key_table_window: one thread per window makes d * 256^w * Y, d = 2..128, by successive additions and normalises all of
+//     them with ONE inversion.  Montgomery's trick without a prefix array: the forward pass stores (X_d P_(d-1), Y_d P_(d-1), Z_d)
+//     with P_d = Z_1 ... Z_d, so that x_d = X_d P_(d-1) / P_d; the backward pass walks 1 / P_d down from 1 / P_128 with Z_d.
+// A key that is not valid gets the identity's table.  Returns whether the key is valid (key_ok).
+template <class C> HD_INLINE bool key_table_powers(typename Grp<C>::FixEntry* tbl, const uint8_t* pk) {
+  typedef Grp<C> G;
+  typedef typename C::F F;
+  F x, y;
+  bool inf = false;
+  const bool ok = load_affine<C>(x, y, &inf, pk) && !inf;   // the short-Weierstrass identity is a valid point but no key
+  typename G::Pt P;
+  if (ok) G::from_affine(P, x, y); else G::set_identity(P);
+#pragma unroll 1
+  for (int w = 0; w < fix_windows<C, KEY_FIX_BITS>(); w++) {
+    F* slot = reinterpret_cast<F*>(&tbl[(size_t)w * KEY_ENTRIES + 1]);
+    slot[0] = P.X; slot[1] = P.Y; slot[2] = P.Z;
+    if (w + 1 < fix_windows<C, KEY_FIX_BITS>()) { G::dbl4(&P); G::dbl4(&P); }
+  }
+  return ok;
+}
+template <class C> HD_INLINE void key_table_window(typename Grp<C>::FixEntry* win) {
+  typedef Grp<C> G;
+  typedef typename C::F F;
+  F* s1 = reinterpret_cast<F*>(&win[1]);
+  typename G::Pt B, cur;
+  G::from_xyz(B, s1[0], s1[1], s1[2]);
+  typename G::Entry eb;
+  G::to_entry(eb, B);
+  cur = B;
+  F pre = F::one();
+#pragma unroll 1
+  for (int d = 1; d < KEY_ENTRIES; d++) {
+    if (d > 1) G::add_entry(&cur, &eb, false);
+    F* slot = reinterpret_cast<F*>(&win[d]);
+    slot[0] = cur.X * pre; slot[1] = cur.Y * pre; slot[2] = cur.Z;
+    pre = pre * select(cur.Z.is_zero(), F::one(), cur.Z);     // the short-Weierstrass identity (Z = 0) stays out of the chain
+  }
+  F acc = inv(pre);
+#pragma unroll 1
+  for (int d = KEY_ENTRIES - 1; d >= 1; d--) {
+    F* slot = reinterpret_cast<F*>(&win[d]);
+    const F X = slot[0], Y = slot[1], Z = slot[2];
+    const bool zero = Z.is_zero();
+    typename G::FixEntry e;
+    G::fix_from_affine(e, X * acc, Y * acc, zero);
+    acc = acc * select(zero, F::one(), Z);
+    win[d] = e;
+  }
+  typename G::FixEntry e0;
+  G::fix_from_affine(e0, F::zero(), F::one(), true);
+  win[0] = e0;
 }
 
 }  // namespace vrfs

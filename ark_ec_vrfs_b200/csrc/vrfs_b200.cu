@@ -119,6 +119,44 @@ __global__ void __launch_bounds__(128) k_ietf_verify_finish(uint32_t n, const ui
   ietf_verify_finish_batched<S, FINISH_K>(n, t, stride, pk, input, output, c, u_xyz, v_xyz, ad, ad_off, valid, out_ok, out_status);
 }
 
+// prepared public keys (vrfs_public_keys_prepare): the per-key 8-bit tables (lincomb.cuh "Prepared-key tables"), the keyed U = s*G - c*Y_k,
+// and the gather of each item's key row for k_ietf_verify_finish
+template <class C>
+__global__ void __launch_bounds__(128) k_key_table_powers(uint32_t n_keys, const uint8_t* pks, typename Grp<C>::FixEntry* tables, uint8_t* rows, uint8_t* key_ok) {
+  const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n_keys) return;
+  key_ok[k] = key_table_powers<C>(tables + (size_t)k * key_table_entries<C>(), pks + (size_t)64 * k);
+  copy_words16(reinterpret_cast<uint4(*)[4]>(rows) + k, reinterpret_cast<const uint4(*)[4]>(pks) + k);
+}
+template <class C>
+__global__ void __launch_bounds__(128) k_key_table_windows(uint32_t n_keys, typename Grp<C>::FixEntry* tables) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_keys * (uint32_t)fix_windows<C, KEY_FIX_BITS>()) return;
+  key_table_window<C>(tables + (size_t)t * KEY_ENTRIES);      // windows of consecutive keys are contiguous
+}
+// 128-thread blocks: the short-Weierstrass suites need ~134 registers to run without spills (3 blocks, 12 warps per SM); the
+// twisted-Edwards ones fit 128 registers and keep the 16 warps per SM of k_lincomb
+#define KEYED_THREADS 128
+template <class C>
+__global__ void __launch_bounds__(KEYED_THREADS, C::IS_TE ? 4 : 3) k_lincomb_keyed(KeyedArgs A) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;   // every item costs the same: a plain grid, no work counter
+  if (i >= A.n) return;
+  typename Grp<C>::Pt acc;
+  lincomb_keyed_item<C>(A, i, acc);
+  Grp<C>::store_xyz(A.out_xyz + (size_t)i * 24, acc);
+}
+// item i's key row (zeros for an index out of range); valid[i] = 0 for such an index or a key that is not valid
+__global__ void __launch_bounds__(128) k_gather_keys(uint32_t n, const uint32_t* key_index, uint32_t n_keys, const uint8_t* rows, const uint8_t* key_ok,
+                                                     uint8_t* out_rows, uint8_t* valid) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t k = key_index[i];
+  uint4 r[4] = {};
+  if (k < n_keys) copy_words16(&r, reinterpret_cast<const uint4(*)[4]>(rows) + k);
+  copy_words16(reinterpret_cast<uint4(*)[4]>(out_rows) + i, &r);
+  if (k >= n_keys || !key_ok[k]) valid[i] = 0;
+}
+
 // integer-pipe roofline microbenchmarks (SURVEY 8d): independent multiply-accumulate chains per thread
 template <int VARIANT>
 __global__ void __launch_bounds__(256) k_mac_bench(uint32_t* out, int iters, unsigned long long* cycles) {
@@ -237,7 +275,8 @@ struct DevBuf {
 };
 enum { BUF_IN0, BUF_IN1, BUF_IN2, BUF_IN3, BUF_IN4, BUF_AD, BUF_OFF, BUF_OUT0, BUF_OUT1, BUF_W0, BUF_W1, BUF_W2, BUF_W3, BUF_VALID, BUF_SLAB,
        BUF_X0, BUF_X1, BUF_X2, BUF_X3, BUF_X4, BUF_X5, BUF_ZINV, BUF_SLAB2,
-       BUF_PB0, BUF_PB1, BUF_PB2, BUF_COUNT };   // X*: wire-format staging (encoded keys, signatures, h2c data, flags); PB*: Pedersen batch verification
+       BUF_PB0, BUF_PB1, BUF_PB2, BUF_KEYROWS, BUF_COUNT };   // X*: wire-format staging (encoded keys, signatures, h2c data, flags); PB*: Pedersen batch verification;
+                                                             // KEYROWS: the key rows a prepared-key verify gathers for its finish kernel
 
 #define MAX_TIMED 64
 #ifndef VRFS_HOST_PIECES
@@ -262,6 +301,7 @@ struct vrfs_ctx {
   DevBuf buf[BUF_COUNT];
   void* fixtab[VRFS_SUITE_COUNT][2] = {};   // [suite][G | blinding base], built on first use
   std::vector<struct vrfs_msm_bases*> prepared;   // live prepared-base handles (freed / orphaned by vrfs_ctx_destroy)
+  std::vector<struct vrfs_public_keys*> prepared_keys;   // live prepared-key handles (likewise)
   // peer group of the multi-GPU MSM exchange (csrc/msm.cuh "multi-GPU exchange"): world = 0 until connected
   struct {
     int rank = 0, world = 0;
@@ -321,6 +361,7 @@ struct CallGuard {
 static vrfs_status note_kernel(vrfs_ctx* ctx, const char* name);
 static vrfs_status timing_begin(vrfs_ctx* ctx);
 static void orphan_prepared(vrfs_ctx* ctx);
+static void orphan_public_keys(vrfs_ctx* ctx);
 static void peer_teardown(vrfs_ctx* ctx);
 
 static vrfs_status timing_begin(vrfs_ctx* ctx) {
@@ -424,6 +465,7 @@ extern "C" void vrfs_ctx_destroy(vrfs_ctx* ctx) {
   cudaSetDevice(ctx->device);
   if (ctx->stream) cudaStreamSynchronize(ctx->stream);
   orphan_prepared(ctx);
+  orphan_public_keys(ctx);
   peer_teardown(ctx);
   for (int i = 0; i < BUF_COUNT; i++) if (ctx->buf[i].p) cudaFree(ctx->buf[i].p);
   for (int s = 0; s < VRFS_SUITE_COUNT; s++) for (int b = 0; b < 2; b++) if (ctx->fixtab[s][b]) cudaFree(ctx->fixtab[s][b]);
@@ -2125,6 +2167,167 @@ extern "C" vrfs_status vrfs_msm_g1_prepared(vrfs_ctx* ctx, const vrfs_msm_bases*
 }
 extern "C" vrfs_status vrfs_msm_g1_prepared_partial(vrfs_ctx* ctx, const vrfs_msm_bases* h, const uint8_t* scalars, int n_columns, uint8_t* out_partial) {
   return msm_prepared_host(ctx, h, scalars, n_columns, out_partial, 1);
+}
+
+// =================================================================================================
+// ietf verify against prepared public keys
+// =================================================================================================
+// A verifier that sees millions of proofs from a few thousand known keys makes Y a fixed base like G: with one table of 8-bit
+// windows per key, c*Y is 32 mixed additions (16-17 for a 16-byte challenge), with no doublings, window slab or GLV split.
+#define VRFS_MAX_PREPARED_KEYS 65536
+struct vrfs_public_keys {
+  vrfs_ctx* ctx;          // nullptr once the context was destroyed first (the tables are gone; release only frees this record)
+  vrfs_suite suite;
+  size_t n_keys;
+  void* mem;              // one allocation: tables | rows | key_ok
+  const void* tables;     // n_keys x key_table_entries<C>() FixEntry, layout [key][window][entry]
+  const uint8_t* rows;    // n_keys x 64: the keys as given (the finish kernel encodes pk from them)
+  const uint8_t* key_ok;  // n_keys
+};
+template <class S>
+static vrfs_status public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n_keys, const uint8_t* pks, uint8_t* out_key_ok, vrfs_public_keys** out) {
+  typedef typename S::C C;
+  typedef typename Grp<C>::FixEntry E;
+  const size_t tbytes = n_keys * key_table_entries<C>() * sizeof(E);
+  vrfs_public_keys* h = new (std::nothrow) vrfs_public_keys();
+  if (!h) return fail(ctx, VRFS_CUDA_ERROR, "out of host memory");
+  h->ctx = ctx; h->suite = suite; h->n_keys = n_keys;
+  cudaError_t e = cudaMalloc(&h->mem, tbytes + n_keys * 65);
+  if (e != cudaSuccess) {
+    cudaGetLastError(); delete h;
+    return fail(ctx, VRFS_CUDA_ERROR, "cudaMalloc of %zu bytes of key tables failed: %s", tbytes + n_keys * 65, cudaGetErrorString(e));
+  }
+  h->tables = h->mem; h->rows = (const uint8_t*)h->mem + tbytes; h->key_ok = h->rows + n_keys * 64;
+  // a failure below must not leak the tables nor hand out a half-built handle
+  auto build = [&]() -> vrfs_status {
+    const uint8_t* d_pk;
+    ST(stage_in(ctx, BUF_IN0, pks, n_keys * 64, &d_pk));
+    k_key_table_powers<C><<<(unsigned)((n_keys + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n_keys, d_pk, (E*)h->mem, (uint8_t*)h->rows, (uint8_t*)h->key_ok);
+    LAUNCHED_AS(ctx, "key_table_powers");
+    const size_t windows = n_keys * fix_windows<C, KEY_FIX_BITS>();
+    k_key_table_windows<C><<<(unsigned)((windows + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n_keys, (E*)h->mem);
+    LAUNCHED_AS(ctx, "key_table_windows");
+    if (out_key_ok) ST(copy_out(ctx, out_key_ok, h->key_ok, n_keys));
+    return finish_call(ctx);
+  };
+  const vrfs_status st = build();
+  if (st != VRFS_OK) { cudaStreamSynchronize(ctx->stream); cudaFree(h->mem); delete h; return st; }
+  ctx->prepared_keys.push_back(h);
+  *out = h;
+  return VRFS_OK;
+}
+extern "C" vrfs_status vrfs_public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n_keys, const uint8_t* pks, uint8_t* out_key_ok, vrfs_public_keys** out) {
+  if (!ctx || !out) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  *out = nullptr;
+  if (!pks) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  if (n_keys < 1 || n_keys > VRFS_MAX_PREPARED_KEYS) return fail(ctx, VRFS_BAD_ARG, "n_keys must be in 1..%d", VRFS_MAX_PREPARED_KEYS);
+  ST(begin_call(ctx, suite, n_keys));
+  return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return public_keys_prepare<S>(ctx, suite, n_keys, pks, out_key_ok, out); });
+}
+// Same lifetime rules as vrfs_msm_bases (vrfs_msm_g1_release): released before or after the context, orphaned by vrfs_ctx_destroy.
+extern "C" void vrfs_public_keys_release(vrfs_public_keys* h) {
+  if (!h) return;
+  vrfs_ctx* ctx;
+  { std::lock_guard<std::mutex> g(g_handles_mu); ctx = h->ctx; }
+  if (ctx) {
+    CallGuard guard_(ctx, __func__);
+    std::lock_guard<std::mutex> g(g_handles_mu);
+    cudaSetDevice(ctx->device);
+    cudaStreamSynchronize(ctx->stream);
+    cudaFree(h->mem);
+    auto& v = ctx->prepared_keys;
+    v.erase(std::remove(v.begin(), v.end(), h), v.end());
+  }
+  delete h;
+}
+static void orphan_public_keys(vrfs_ctx* ctx) {   // called by vrfs_ctx_destroy (device set, stream synchronised)
+  std::lock_guard<std::mutex> g(g_handles_mu);
+  for (vrfs_public_keys* h : ctx->prepared_keys) { cudaFree(h->mem); h->mem = nullptr; h->ctx = nullptr; }
+  ctx->prepared_keys.clear();
+}
+
+// U = s*G - c*Y_k (k_lincomb_keyed: both terms fixed-base), V = s*I - c*O as in ietf_verify_dev, the finish kernel of ietf_verify_dev
+// on the gathered key rows.  Small batches run U on the side stream beside V, like ietf_verify_dev.
+template <class S>
+static vrfs_status ietf_verify_prepared_dev(vrfs_ctx* ctx, const vrfs_public_keys* h, size_t n, const uint32_t* key_index, const uint8_t* input,
+                                            const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad, const uint64_t* ad_off,
+                                            uint8_t* out_ok, uint8_t* out_status) {
+  typedef typename S::C C;
+  void *u = nullptr, *v = nullptr, *valid = nullptr, *pk = nullptr;
+  ST(need_tables<S>(ctx));
+  ST(ensure(ctx, BUF_W0, n * 96, &u));
+  ST(ensure(ctx, BUF_W1, n * 96, &v));
+  ST(ensure(ctx, BUF_VALID, n, &valid));
+  ST(ensure(ctx, BUF_KEYROWS, n * 64, &pk));
+  CU(cudaMemsetAsync(valid, 1, n, ctx->stream));
+  k_gather_keys<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n, key_index, (uint32_t)h->n_keys, h->rows, h->key_ok, (uint8_t*)pk, (uint8_t*)valid);
+  LAUNCHED_AS(ctx, "gather_keys");
+  const bool split = n <= (size_t)ctx->sms * VRFS_SPLIT_ITEMS_PER_SM;
+  const uint32_t cbits = S::CLEN < 32 ? 8u * S::CLEN : 0u;
+  const KeyedArgs K = {(uint32_t)n, s, c, cbits, key_index, (uint32_t)h->n_keys, ctx->fixtab[S::ID][0], h->tables, (uint32_t*)u};
+  if (split) ST(side_fork(ctx));
+  k_lincomb_keyed<C><<<(unsigned)((n + KEYED_THREADS - 1) / KEYED_THREADS), KEYED_THREADS, 0, split ? ctx->copy_stream : ctx->stream>>>(K);
+  LAUNCHED_AS(ctx, "lincomb_keyed");
+  LincombArgs A = {};
+  A.n = (uint32_t)n;
+  A.valid = (uint8_t*)valid;
+  A.var[0] = {input, 64, s, 32, 0, 0};
+  A.var[1] = {output, 64, c, 32, 1, cbits};
+  A.out_xyz = (uint32_t*)v;
+  ST((launch_lincomb<C, 2, 0>(ctx, A)));
+  if (split) ST(side_join(ctx));
+  k_ietf_verify_finish<S><<<(unsigned)((n + 128 * FINISH_K - 1) / (128 * FINISH_K)), 128, 0, ctx->stream>>>((uint32_t)n, (const uint8_t*)pk, input, output, c, (const uint32_t*)u,
+                                                                                (const uint32_t*)v, ad, ad_off, (const uint8_t*)valid, out_ok, out_status);
+  LAUNCHED_AS(ctx, "ietf_verify_finish");
+  return VRFS_OK;
+}
+static vrfs_status check_keys(vrfs_ctx* ctx, const vrfs_public_keys* h) {
+  if (!h || h->ctx != ctx) return fail(ctx, VRFS_BAD_ARG, "prepared keys of another (or a destroyed) context");
+  return VRFS_OK;
+}
+extern "C" vrfs_status vrfs_ietf_verify_prepared_batch_dev(vrfs_ctx* ctx, const vrfs_public_keys* keys, size_t n, const uint32_t* key_index,
+                                                           const uint8_t* input, const uint8_t* output, const uint8_t* c, const uint8_t* s,
+                                                           const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  ST(check_keys(ctx, keys));
+  if (n == 0) return VRFS_OK;
+  if (!key_index || !input || !output || !c || !s || !out_ok || (ad && !ad_off)) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  if (!aligned16(key_index) || !aligned16(input) || !aligned16(output) || !aligned16(c) || !aligned16(s))
+    return fail(ctx, VRFS_BAD_ARG, "device buffers must be 16-byte aligned");
+  ST(begin_call(ctx, keys->suite, n));
+  return with_suite(ctx, keys->suite, [&](auto S_) { typedef decltype(S_) S;
+    return ietf_verify_prepared_dev<S>(ctx, keys, n, key_index, input, output, c, s, ad, ad_off, out_ok, out_status); });
+}
+// host buffers: staged in pieces like vrfs_ietf_verify_batch (ietf_verify_host_enqueue), 4 bytes of key index per item instead of 64 of key
+extern "C" vrfs_status vrfs_ietf_verify_prepared_batch(vrfs_ctx* ctx, const vrfs_public_keys* keys, size_t n, const uint32_t* key_index,
+                                                       const uint8_t* input, const uint8_t* output, const uint8_t* c, const uint8_t* s,
+                                                       const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  ST(check_keys(ctx, keys));
+  if (n == 0) return VRFS_OK;
+  if (!key_index || !input || !output || !c || !s || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  ST(begin_call(ctx, keys->suite, n));
+  const uint8_t* d_ad; const uint64_t* d_off; uint8_t *d_ok, *d_st = nullptr;
+  ST(stage_ad(ctx, n, ad, ad_off, &d_ad, &d_off));
+  ST(stage_out(ctx, BUF_OUT0, n, &d_ok));
+  if (out_status) ST(stage_out(ctx, BUF_OUT1, n, &d_st));
+  HostIn in[5] = {{BUF_IN0, key_index, 4, false, nullptr}, {BUF_IN1, input, 64, false, nullptr}, {BUF_IN2, output, 64, false, nullptr},
+                  {BUF_IN3, c, 32, false, nullptr}, {BUF_IN4, s, 32, false, nullptr}};
+  Pieces pc;
+  ST(stage_in_pieces(ctx, n, in, 5, &pc, 2));
+  for (int k = 0; k < pc.count; k++) {
+    const size_t o = pc.cut[k], m = pc.cut[k + 1] - pc.cut[k];
+    ST(piece_ready(ctx, k));
+    ST(with_suite(ctx, keys->suite, [&](auto S_) { typedef decltype(S_) S;
+      return ietf_verify_prepared_dev<S>(ctx, keys, m, (const uint32_t*)in[0].dev + o, in[1].dev + o * 64, in[2].dev + o * 64, in[3].dev + o * 32,
+                                         in[4].dev + o * 32, d_ad, d_off ? d_off + o : nullptr, d_ok + o, d_st ? d_st + o : nullptr); }));
+  }
+  ST(copy_out(ctx, out_ok, d_ok, n));
+  if (out_status) ST(copy_out(ctx, out_status, d_st, n));
+  return finish_call(ctx);
 }
 // =================================================================================================
 // ring fixed columns + commitment (SURVEY 8f-2; csrc/ring.cuh)

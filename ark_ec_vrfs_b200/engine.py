@@ -101,6 +101,54 @@ class PreparedBases:
                 self.engine._prepared.remove(self)
 
 
+def _dev_ptr(x):
+    """a device pointer: an int, or a torch CUDA tensor (its data_ptr())"""
+    if x is None:
+        return None
+    return C.c_void_p(x.data_ptr() if hasattr(x, "data_ptr") else int(x) or None)
+
+
+class PreparedPublics:
+    """Public keys prepared once for many verifies (vrfs_public_keys_prepare): one fixed-base table per key on the engine's GPU.
+    key_ok[k] = 1 where keys[k] is a key ietf_verify accepts.  Usable as a context manager; release() frees the tables."""
+
+    def __init__(self, engine, handle, suite, key_ok):
+        self.engine, self.handle, self.suite, self.key_ok = engine, handle, suite, key_ok
+
+    @property
+    def n_keys(self):
+        return len(self.key_ok)
+
+    def verify(self, key_index, inp, outp, c, s, ad=None, status=False):
+        """ietf_verify with pk[i] = keys[key_index[i]] (an index >= n_keys: ITEM_INVALID_DATA) -> ok flags [, status]"""
+        key_index = np.ascontiguousarray(key_index, dtype=np.uint32).reshape(-1); n = len(key_index)
+        inp = _u8(inp, (n, 64)); outp = _u8(outp, (n, 64)); c = _u8(c, (n, 32)); s = _u8(s, (n, 32))
+        adb, off = pack_var(ad, n)
+        ok = np.zeros(n, np.uint8); st = np.zeros(n, np.uint8) if status else None
+        self.engine._call("vrfs_ietf_verify_prepared_batch", self.handle, C.c_size_t(n), _p(key_index), _p(inp), _p(outp), _p(c), _p(s),
+                          _p(adb), _p(off), _p(ok), _p(st))
+        return (ok, st) if status else ok
+
+    def verify_dev(self, n, d_key_index, d_inp, d_outp, d_c, d_s, d_ok, d_ad=None, d_off=None, d_status=None):
+        """device buffers (ints or torch CUDA tensors; key_index uint32, 16-byte aligned); enqueued on the context stream
+        (Engine.stream) - the caller orders its producers before and its readers after it (e.g. Engine.sync())"""
+        self.engine._call("vrfs_ietf_verify_prepared_batch_dev", self.handle, C.c_size_t(n), _dev_ptr(d_key_index), _dev_ptr(d_inp), _dev_ptr(d_outp),
+                          _dev_ptr(d_c), _dev_ptr(d_s), _dev_ptr(d_ad), _dev_ptr(d_off), _dev_ptr(d_ok), _dev_ptr(d_status))
+
+    def release(self):
+        if self.handle:
+            self.engine._lib.vrfs_public_keys_release(self.handle)
+            self.handle = None
+            if self in self.engine._prepared:
+                self.engine._prepared.remove(self)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.release()
+
+
 def host_buffer(shape):
     """A zeroed uint8 array in page-locked host memory (vrfs_host_alloc): batch calls on such buffers copy beside their kernels.
     The allocation is freed when the array (and every view of it) is gone."""
@@ -209,6 +257,16 @@ class Engine:
         """device pointers (ints); enqueues on the context stream, returns immediately"""
         v = lambda x: C.c_void_p(x) if x else None
         self._check(self._lib.vrfs_ietf_verify_batch_dev(self._ctx, suite, C.c_size_t(n), v(d_pk), v(d_inp), v(d_outp), v(d_c), v(d_s), v(d_ad), v(d_off), v(d_ok), v(d_status)))
+
+    def public_keys_prepare(self, suite, pks):
+        """(n_keys, 64) affine keys of one suite -> PreparedPublics: per-key fixed-base tables (~400 KB per key) on this GPU, so that
+        proofs of known signers are verified by key index (vrfs_public_keys_prepare)"""
+        pks = _u8(pks, (-1, 64)); key_ok = np.zeros(len(pks), np.uint8)
+        h = C.c_void_p()
+        self._call("vrfs_public_keys_prepare", suite, C.c_size_t(len(pks)), _p(pks), _p(key_ok), C.byref(h))
+        p = PreparedPublics(self, h, suite, key_ok)
+        self._prepared.append(p)
+        return p
 
     def ietf_verify_host_ptrs(self, suite, n, pk, inp, outp, c, s, ok, ad=None, off=None, status=None):
         """raw host pointers (ints), e.g. of pinned torch tensors; synchronous"""

@@ -118,6 +118,33 @@ vrfs_status vrfs_ietf_verify_batch_dev(vrfs_ctx*, vrfs_suite, size_t n, const ui
                                        const uint8_t* d_output, const uint8_t* d_c, const uint8_t* d_s, const uint8_t* d_ad,
                                        const uint64_t* d_ad_off, uint8_t* d_out_ok, uint8_t* d_out_status /* may be NULL */);
 
+/* ietf::Verifier::verify against PREPARED public keys: "prepare once, verify many" for a known signer set (a validator set, a
+ * committee).  vrfs_public_keys_prepare builds, on this context's GPU, one fixed-base table per key (8-bit signed windows, about
+ * 400 KB per key), so that c*Y costs 32 mixed additions (16-17 for a 16-byte challenge) instead of a variable-base multiplication.
+ *   prepare: n_keys affine keys (x || y, the layout of every typed call) of one suite.  out_key_ok (may be NULL): 1 per key that
+ *            vrfs_ietf_verify_batch would accept as a key (canonical, on the curve, not the short-Weierstrass identity), else 0.
+ *            1 <= n_keys <= 65536, else VRFS_BAD_ARG.  An allocation that fails returns VRFS_CUDA_ERROR and leaks nothing.
+ *   verify:  item i is ietf::Verifier::verify with pk[i] = pks[key_index[i]]: out_ok / out_status are exactly those of
+ *            vrfs_ietf_verify_batch on the gathered keys.  key_index[i] >= n_keys makes item i VRFS_ITEM_INVALID_DATA (never an
+ *            out-of-range read).  4 bytes of key index travel per item instead of 64 bytes of key.  The _dev form takes 16-byte
+ *            aligned device buffers and is asynchronous on the context's stream, like vrfs_ietf_verify_batch_dev.
+ * A handle belongs to the context that prepared it; with any other context the calls return VRFS_BAD_ARG.  vrfs_ctx_destroy frees
+ * the tables of the handles still alive and orphans them; releasing an orphan (or NULL) only frees its record.
+ * Keys are meant to be typed `Public` values, i.e. in the prime-order subgroup (decode them with vrfs_point_decode_checked_batch).
+ * For an on-curve key with a small-order component the two calls need not agree on a crafted proof: vrfs_ietf_verify_batch
+ * computes c*Y for Bandersnatch through the GLV split k1*Y + k2*psi(Y), which equals c*Y only on the subgroup, while the table
+ * computes c*Y itself.  Both reject honest proofs under such a key (its encoding enters the challenge). */
+typedef struct vrfs_public_keys vrfs_public_keys;
+vrfs_status vrfs_public_keys_prepare(vrfs_ctx*, vrfs_suite, size_t n_keys, const uint8_t* pks /*n_keys*64*/,
+                                     uint8_t* out_key_ok /*n_keys, may be NULL*/, vrfs_public_keys** out);
+void vrfs_public_keys_release(vrfs_public_keys*);
+vrfs_status vrfs_ietf_verify_prepared_batch(vrfs_ctx*, const vrfs_public_keys*, size_t n, const uint32_t* key_index,
+                                            const uint8_t* input, const uint8_t* output, const uint8_t* c, const uint8_t* s,
+                                            const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status /* may be NULL */);
+vrfs_status vrfs_ietf_verify_prepared_batch_dev(vrfs_ctx*, const vrfs_public_keys*, size_t n, const uint32_t* d_key_index,
+                                                const uint8_t* d_input, const uint8_t* d_output, const uint8_t* d_c, const uint8_t* d_s,
+                                                const uint8_t* d_ad, const uint64_t* d_ad_off, uint8_t* d_out_ok, uint8_t* d_out_status /* may be NULL */);
+
 /* pedersen::Prover::prove / Verifier::verify (A.10).  proof = pk_com || r || ok (3 x 64-byte affine) || s || sb (2 x 32 bytes) = 256 bytes. */
 vrfs_status vrfs_pedersen_prove_batch(vrfs_ctx*, vrfs_suite, size_t n, const uint8_t* sk, const uint8_t* input, const uint8_t* output,
                                       const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_proof /*n*256*/, uint8_t* out_blinding /*n*32*/);

@@ -163,6 +163,33 @@ struct Public : Points {
   }
 };
 
+// A Public that is reused ("prepare once, verify many"): one fixed-base table per key on the engine's GPU (vrfs_public_keys_prepare),
+// proofs verified by key index.  The engine must outlive the calls; destroying it first leaves release safe (RAII).
+class PreparedPublics {
+ public:
+  explicit PreparedPublics(const Public& keys) : suite_(keys.suite), key_ok_(keys.size()) {
+    suite_.engine->check(vrfs_public_keys_prepare(suite_.engine->ctx(), suite_.id, keys.size(), keys.xy.data(), key_ok_.data(), &h_));
+  }
+  ~PreparedPublics() { vrfs_public_keys_release(h_); }
+  PreparedPublics(const PreparedPublics&) = delete;
+  PreparedPublics& operator=(const PreparedPublics&) = delete;
+  size_t size() const { return key_ok_.size(); }
+  const Bytes& key_ok() const { return key_ok_; }            // 1 = a key Public::verify accepts
+  // ietf::Verifier::verify with pk[i] = keys[key_index[i]]; an index out of range is Error::InvalidData for that item
+  Bytes verify(const std::vector<uint32_t>& key_index, const Input& input, const Output& output, const std::vector<Bytes>& ad, const ietf::Proof& proof,
+               Errors* errors = nullptr) const {
+    Packed a(ad); size_t n = key_index.size(); Bytes ok(n);
+    suite_.engine->check(vrfs_ietf_verify_prepared_batch(suite_.engine->ctx(), h_, n, key_index.data(), input.xy.data(), output.xy.data(), proof.c.data(),
+                                                         proof.s.data(), a.ptr(), a.off.data(), ok.data(), status_ptr(errors, n)));
+    return ok;
+  }
+
+ private:
+  Suite suite_;
+  Bytes key_ok_;
+  vrfs_public_keys* h_ = nullptr;
+};
+
 struct Secret {
   Suite suite;
   Bytes scalars;                                         // n x 32
