@@ -17,6 +17,7 @@ SYMBOLS = [
     "vrfs_point_encode_batch", "vrfs_point_decode_batch", "vrfs_nonce_batch",
     "vrfs_ietf_prove_batch", "vrfs_ietf_verify_batch", "vrfs_ietf_verify_batch_dev",
     "vrfs_public_keys_prepare", "vrfs_public_keys_release", "vrfs_ietf_verify_prepared_batch", "vrfs_ietf_verify_prepared_batch_dev",
+    "vrfs_public_keys_prepare_encoded", "vrfs_ietf_verify_prepared_wire_batch",
     "vrfs_pedersen_prove_batch", "vrfs_pedersen_verify_batch",
     "vrfs_suite_ietf_signature_len", "vrfs_point_decode_checked_batch", "vrfs_subgroup_check_batch", "vrfs_ietf_sign_wire_batch", "vrfs_ietf_verify_wire_batch",
     "vrfs_suite_pedersen_signature_len", "vrfs_pedersen_sign_wire_batch", "vrfs_pedersen_verify_wire_batch",

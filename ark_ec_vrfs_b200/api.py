@@ -73,6 +73,12 @@ class Public:
         """these keys prepared once for many verifies (per-key fixed-base tables on the suite's GPU) -> PreparedPublic"""
         return PreparedPublic(self.suite, self.suite.engine.public_keys_prepare(self.suite.suite_id, self.points))
 
+    @staticmethod
+    def prepare_compressed(suite, enc):
+        """serialised keys (e.g. a published validator set) deserialised with validation and prepared once -> PreparedPublic whose
+        verify_signatures takes serialised signatures by key index; key_ok = 0 where deserialize_compressed rejects the key"""
+        return PreparedPublic(suite, suite.engine.public_keys_prepare_encoded(suite.suite_id, enc))
+
     @classmethod
     def deserialize_compressed(cls, suite, enc):
         """CanonicalDeserialize with validation (canonical, on curve, prime-order subgroup) -> (Public, ok flags)"""
@@ -101,6 +107,11 @@ class PreparedPublic:
         """ietf::Verifier::verify with pk[i] = keys[key_index[i]] -> uint8[n] (status=True: (ok, Error variant per item));
         an index out of range is ITEM_INVALID_DATA for its item"""
         return self.keys.verify(key_index, input.points, output.points, proof.c, proof.s, ad, status=status)
+
+    def verify_signatures(self, key_index, datas, signatures, ad=None, status=False):
+        """Public.verify_signatures with pk_enc[i] = the encoding of key key_index[i] -> (ok flags, Output::hash[, status]);
+        only for keys from Public.prepare_compressed"""
+        return self.keys.verify_wire(key_index, datas, signatures, ad, status=status)
 
     def release(self):
         self.keys.release()

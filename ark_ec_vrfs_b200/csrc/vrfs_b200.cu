@@ -1357,6 +1357,28 @@ __global__ void k_merge_flags(uint32_t n, const uint8_t* a, const uint8_t* b, ui
   if (status) status[i] = (uint8_t)(ok ? ITEM_OK : !wellformed ? ITEM_INVALID_DATA : status[i] == ITEM_OK ? ITEM_VERIFICATION_FAILURE : status[i]);
   if (hash && !ok) for (uint32_t j = 0; j < hlen; j++) hash[(size_t)hlen * i + j] = 0;
 }
+// signature against a prepared key named by index (vrfs_ietf_verify_prepared_wire_batch), in place of k_decode_checked (key and
+// Output), k_wire_parse_proof and k_gather_keys: item i's key row (zeros for an index out of range), its Output decoded with the
+// subgroup check, c and s parsed.  valid[i] = the index names a valid key (what k_gather_keys leaves); wellformed[i] = that and
+// both deserialisations succeeded (k_merge_flags' `a`, which the wire call takes from k_wire_parse_proof)
+template <class S> __global__ void __launch_bounds__(ITEM_THREADS) k_wire_prepared_unpack(uint32_t n, const uint32_t* key_index, uint32_t n_keys, const uint8_t* rows,
+                                                                                           const uint8_t* key_ok, const uint8_t* sig, uint8_t* out_rows, uint8_t* output,
+                                                                                           uint8_t* c, uint8_t* s, uint8_t* valid, uint8_t* wellformed) {
+  ITEM_INDEX(n);
+  constexpr uint32_t SL = S::ENC_LEN + S::CLEN + 32;
+  const uint8_t* e = sig + (size_t)SL * i;
+  uint8_t tmp[S::ENC_LEN];
+  for (int j = 0; j < S::ENC_LEN; j++) tmp[j] = e[j];
+  const bool out_ok = wire_decode_point_checked<S>(output + (size_t)64 * i, tmp);
+  const bool parsed = wire_parse_proof<S>(c + (size_t)32 * i, s + (size_t)32 * i, e + S::ENC_LEN);
+  const uint32_t k = key_index[i];                               // after the decode: nothing of the key is live across it
+  const bool key = k < n_keys && key_ok[k];
+  uint4 r[4] = {};
+  if (k < n_keys) copy_words16(&r, reinterpret_cast<const uint4(*)[4]>(rows) + k);
+  copy_words16(reinterpret_cast<uint4(*)[4]>(out_rows) + i, &r);
+  valid[i] = (uint8_t)key;
+  wellformed[i] = (uint8_t)(key && out_ok && parsed);
+}
 
 extern "C" int vrfs_suite_ietf_signature_len(vrfs_suite s) { return vrfs_suite_point_enc_len(s) + vrfs_suite_challenge_len(s) + 32; }
 
@@ -2181,17 +2203,21 @@ struct vrfs_public_keys {
   size_t n_keys;
   void* mem;              // one allocation: tables | rows | key_ok
   const void* tables;     // n_keys x key_table_entries<C>() FixEntry, layout [key][window][entry]
-  const uint8_t* rows;    // n_keys x 64: the keys as given (the finish kernel encodes pk from them)
+  const uint8_t* rows;    // n_keys x 64: the keys as given, or as decoded (the finish kernel encodes pk from them)
   const uint8_t* key_ok;  // n_keys
+  bool from_encodings;    // vrfs_public_keys_prepare_encoded: every key with key_ok = 1 passed the decoder's subgroup check
 };
+// `encoded`: pks holds n_keys encodings (Codec::point_encode), decoded and subgroup-checked by k_decode_checked into the rows
+// the tables are built from; key_ok = that decode's flag AND the affine key test of k_key_table_powers
 template <class S>
-static vrfs_status public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n_keys, const uint8_t* pks, uint8_t* out_key_ok, vrfs_public_keys** out) {
+static vrfs_status public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n_keys, const uint8_t* pks, bool encoded, uint8_t* out_key_ok,
+                                       vrfs_public_keys** out) {
   typedef typename S::C C;
   typedef typename Grp<C>::FixEntry E;
   const size_t tbytes = n_keys * key_table_entries<C>() * sizeof(E);
   vrfs_public_keys* h = new (std::nothrow) vrfs_public_keys();
   if (!h) return fail(ctx, VRFS_CUDA_ERROR, "out of host memory");
-  h->ctx = ctx; h->suite = suite; h->n_keys = n_keys;
+  h->ctx = ctx; h->suite = suite; h->n_keys = n_keys; h->from_encodings = encoded;
   cudaError_t e = cudaMalloc(&h->mem, tbytes + n_keys * 65);
   if (e != cudaSuccess) {
     cudaGetLastError(); delete h;
@@ -2201,12 +2227,25 @@ static vrfs_status public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n
   // a failure below must not leak the tables nor hand out a half-built handle
   auto build = [&]() -> vrfs_status {
     const uint8_t* d_pk;
-    ST(stage_in(ctx, BUF_IN0, pks, n_keys * 64, &d_pk));
+    uint8_t* d_dec_ok = nullptr;
+    if (encoded) {
+      const uint8_t* d_enc; uint8_t* d_dec;
+      ST(stage_in(ctx, BUF_X0, pks, n_keys * S::ENC_LEN, &d_enc));
+      ST(stage_out(ctx, BUF_IN0, n_keys * 64, &d_dec)); ST(stage_out(ctx, BUF_X4, n_keys, &d_dec_ok));
+      ST(decode_checked_launch<S>(ctx, n_keys, d_enc, S::ENC_LEN, d_dec, nullptr, 0, nullptr, d_dec_ok));
+      d_pk = d_dec;
+    } else {
+      ST(stage_in(ctx, BUF_IN0, pks, n_keys * 64, &d_pk));
+    }
     k_key_table_powers<C><<<(unsigned)((n_keys + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n_keys, d_pk, (E*)h->mem, (uint8_t*)h->rows, (uint8_t*)h->key_ok);
     LAUNCHED_AS(ctx, "key_table_powers");
     const size_t windows = n_keys * fix_windows<C, KEY_FIX_BITS>();
     k_key_table_windows<C><<<(unsigned)((windows + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n_keys, (E*)h->mem);
     LAUNCHED_AS(ctx, "key_table_windows");
+    if (encoded) {   // key_ok &= decode flag.  A failed decode leaves a zero row, which k_key_table_powers rejects on its own; this does not rely on it
+      k_merge_flags<<<item_blocks(n_keys), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n_keys, d_dec_ok, nullptr, (uint8_t*)h->key_ok, nullptr, 0u, nullptr);
+      LAUNCHED_AS(ctx, "merge_flags");
+    }
     if (out_key_ok) ST(copy_out(ctx, out_key_ok, h->key_ok, n_keys));
     return finish_call(ctx);
   };
@@ -2223,7 +2262,17 @@ extern "C" vrfs_status vrfs_public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite,
   if (!pks) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   if (n_keys < 1 || n_keys > VRFS_MAX_PREPARED_KEYS) return fail(ctx, VRFS_BAD_ARG, "n_keys must be in 1..%d", VRFS_MAX_PREPARED_KEYS);
   ST(begin_call(ctx, suite, n_keys));
-  return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return public_keys_prepare<S>(ctx, suite, n_keys, pks, out_key_ok, out); });
+  return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return public_keys_prepare<S>(ctx, suite, n_keys, pks, false, out_key_ok, out); });
+}
+extern "C" vrfs_status vrfs_public_keys_prepare_encoded(vrfs_ctx* ctx, vrfs_suite suite, size_t n_keys, const uint8_t* pk_enc, uint8_t* out_key_ok,
+                                                        vrfs_public_keys** out) {
+  if (!ctx || !out) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  *out = nullptr;
+  if (!pk_enc) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  if (n_keys < 1 || n_keys > VRFS_MAX_PREPARED_KEYS) return fail(ctx, VRFS_BAD_ARG, "n_keys must be in 1..%d", VRFS_MAX_PREPARED_KEYS);
+  ST(begin_call(ctx, suite, n_keys));
+  return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return public_keys_prepare<S>(ctx, suite, n_keys, pk_enc, true, out_key_ok, out); });
 }
 // Same lifetime rules as vrfs_msm_bases (vrfs_msm_g1_release): released before or after the context, orphaned by vrfs_ctx_destroy.
 extern "C" void vrfs_public_keys_release(vrfs_public_keys* h) {
@@ -2248,21 +2297,17 @@ static void orphan_public_keys(vrfs_ctx* ctx) {   // called by vrfs_ctx_destroy 
 }
 
 // U = s*G - c*Y_k (k_lincomb_keyed: both terms fixed-base), V = s*I - c*O as in ietf_verify_dev, the finish kernel of ietf_verify_dev
-// on the gathered key rows.  Small batches run U on the side stream beside V, like ietf_verify_dev.
+// on the key rows `pk` with the flags `valid` that the caller's gather left.  Small batches run U on the side stream beside V, like
+// ietf_verify_dev.
 template <class S>
-static vrfs_status ietf_verify_prepared_dev(vrfs_ctx* ctx, const vrfs_public_keys* h, size_t n, const uint32_t* key_index, const uint8_t* input,
-                                            const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad, const uint64_t* ad_off,
-                                            uint8_t* out_ok, uint8_t* out_status) {
+static vrfs_status ietf_verify_keyed_dev(vrfs_ctx* ctx, const vrfs_public_keys* h, size_t n, const uint32_t* key_index, const uint8_t* pk,
+                                         const uint8_t* input, const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad,
+                                         const uint64_t* ad_off, uint8_t* valid, uint8_t* out_ok, uint8_t* out_status) {
   typedef typename S::C C;
-  void *u = nullptr, *v = nullptr, *valid = nullptr, *pk = nullptr;
+  void *u = nullptr, *v = nullptr;
   ST(need_tables<S>(ctx));
   ST(ensure(ctx, BUF_W0, n * 96, &u));
   ST(ensure(ctx, BUF_W1, n * 96, &v));
-  ST(ensure(ctx, BUF_VALID, n, &valid));
-  ST(ensure(ctx, BUF_KEYROWS, n * 64, &pk));
-  CU(cudaMemsetAsync(valid, 1, n, ctx->stream));
-  k_gather_keys<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n, key_index, (uint32_t)h->n_keys, h->rows, h->key_ok, (uint8_t*)pk, (uint8_t*)valid);
-  LAUNCHED_AS(ctx, "gather_keys");
   const bool split = n <= (size_t)ctx->sms * VRFS_SPLIT_ITEMS_PER_SM;
   const uint32_t cbits = S::CLEN < 32 ? 8u * S::CLEN : 0u;
   const KeyedArgs K = {(uint32_t)n, s, c, cbits, key_index, (uint32_t)h->n_keys, ctx->fixtab[S::ID][0], h->tables, (uint32_t*)u};
@@ -2271,15 +2316,49 @@ static vrfs_status ietf_verify_prepared_dev(vrfs_ctx* ctx, const vrfs_public_key
   LAUNCHED_AS(ctx, "lincomb_keyed");
   LincombArgs A = {};
   A.n = (uint32_t)n;
-  A.valid = (uint8_t*)valid;
+  A.valid = valid;
   A.var[0] = {input, 64, s, 32, 0, 0};
   A.var[1] = {output, 64, c, 32, 1, cbits};
   A.out_xyz = (uint32_t*)v;
   ST((launch_lincomb<C, 2, 0>(ctx, A)));
   if (split) ST(side_join(ctx));
-  k_ietf_verify_finish<S><<<(unsigned)((n + 128 * FINISH_K - 1) / (128 * FINISH_K)), 128, 0, ctx->stream>>>((uint32_t)n, (const uint8_t*)pk, input, output, c, (const uint32_t*)u,
-                                                                                (const uint32_t*)v, ad, ad_off, (const uint8_t*)valid, out_ok, out_status);
+  k_ietf_verify_finish<S><<<(unsigned)((n + 128 * FINISH_K - 1) / (128 * FINISH_K)), 128, 0, ctx->stream>>>((uint32_t)n, pk, input, output, c, (const uint32_t*)u,
+                                                                                (const uint32_t*)v, ad, ad_off, valid, out_ok, out_status);
   LAUNCHED_AS(ctx, "ietf_verify_finish");
+  return VRFS_OK;
+}
+template <class S>
+static vrfs_status ietf_verify_prepared_dev(vrfs_ctx* ctx, const vrfs_public_keys* h, size_t n, const uint32_t* key_index, const uint8_t* input,
+                                            const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad, const uint64_t* ad_off,
+                                            uint8_t* out_ok, uint8_t* out_status) {
+  void *valid = nullptr, *pk = nullptr;
+  ST(ensure(ctx, BUF_VALID, n, &valid));
+  ST(ensure(ctx, BUF_KEYROWS, n * 64, &pk));
+  CU(cudaMemsetAsync(valid, 1, n, ctx->stream));
+  k_gather_keys<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n, key_index, (uint32_t)h->n_keys, h->rows, h->key_ok, (uint8_t*)pk, (uint8_t*)valid);
+  LAUNCHED_AS(ctx, "gather_keys");
+  return ietf_verify_keyed_dev<S>(ctx, h, n, key_index, (const uint8_t*)pk, input, output, c, s, ad, ad_off, (uint8_t*)valid, out_ok, out_status);
+}
+// serialised signature + data + key index -> verdict (+ Output::hash of accepted items): ietf_verify_wire_dev with the key taken
+// from the prepared set.  k_wire_prepared_unpack stands for the decode, parse and gather kernels; flags = wellformed | h2c ok (2n).
+template <class S>
+static vrfs_status ietf_verify_prepared_wire_dev(vrfs_ctx* ctx, const vrfs_public_keys* h, size_t n, const uint32_t* key_index, const uint8_t* data,
+                                                 const uint64_t* data_off, const uint8_t* sig, const uint8_t* ad, const uint64_t* ad_off, uint8_t* input,
+                                                 uint8_t* output, uint8_t* c, uint8_t* s, uint8_t* flags, uint8_t* out_ok, uint8_t* out_hash, uint8_t* out_status) {
+  void *valid = nullptr, *pk = nullptr;
+  ST(ensure(ctx, BUF_VALID, n, &valid));
+  ST(ensure(ctx, BUF_KEYROWS, n * 64, &pk));
+  k_wire_prepared_unpack<S><<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, key_index, (uint32_t)h->n_keys, h->rows, h->key_ok, sig,
+                                                                              (uint8_t*)pk, output, c, s, (uint8_t*)valid, flags);
+  LAUNCHED_AS(ctx, "wire_prepared_unpack");
+  ST(data_to_point_dev<S>(ctx, n, data, data_off, input, flags + n));
+  ST(ietf_verify_keyed_dev<S>(ctx, h, n, key_index, (const uint8_t*)pk, input, output, c, s, ad, ad_off, (uint8_t*)valid, out_ok, out_status));
+  if (out_hash) {
+    k_point_to_hash<S><<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, output, out_hash);
+    LAUNCHED_AS(ctx, "point_to_hash");
+  }
+  k_merge_flags<<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, flags, flags + n, out_ok, out_hash, (uint32_t)S::HLEN, out_status);
+  LAUNCHED_AS(ctx, "merge_flags");
   return VRFS_OK;
 }
 static vrfs_status check_keys(vrfs_ctx* ctx, const vrfs_public_keys* h) {
@@ -2327,6 +2406,48 @@ extern "C" vrfs_status vrfs_ietf_verify_prepared_batch(vrfs_ctx* ctx, const vrfs
   }
   ST(copy_out(ctx, out_ok, d_ok, n));
   if (out_status) ST(copy_out(ctx, out_status, d_st, n));
+  return finish_call(ctx);
+}
+// serialised signatures verified against keys prepared from their encodings (vrfs_public_keys_prepare_encoded), the key named by
+// index: the results of vrfs_ietf_verify_wire_batch on the gathered encodings.  Staged like that call.
+extern "C" vrfs_status vrfs_ietf_verify_prepared_wire_batch(vrfs_ctx* ctx, const vrfs_public_keys* keys, size_t n, const uint32_t* key_index,
+                                                            const uint8_t* data, const uint64_t* data_off, const uint8_t* sig, const uint8_t* ad,
+                                                            const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_hash, uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  ST(check_keys(ctx, keys));
+  // keys that never passed the decoder's subgroup check: c*Y from the table need not be the wire call's c*Y (header)
+  if (!keys->from_encodings) return fail(ctx, VRFS_BAD_ARG, "prepared keys not made from encodings (vrfs_public_keys_prepare_encoded)");
+  if (n == 0) return VRFS_OK;
+  if (!key_index || !data_off || !sig || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  ST(begin_call(ctx, keys->suite, n));
+  const size_t sl = (size_t)vrfs_suite_ietf_signature_len(keys->suite), hl = (size_t)vrfs_suite_hash_len(keys->suite);
+  const uint8_t *d_ad, *d_data; const uint64_t *d_off, *d_doff;
+  uint8_t *d_in, *d_out, *d_c, *d_s, *d_flags, *d_ok, *d_hash = nullptr, *d_st = nullptr;
+  // key indices and signatures on the copy stream in one piece, data and ad on the main stream (see vrfs_ietf_verify_wire_batch)
+  HostIn in[2] = {{BUF_X0, key_index, 4, false, nullptr}, {BUF_X1, sig, sl, false, nullptr}};
+  Pieces pc;
+  ST(stage_in_pieces(ctx, n, in, 2, &pc, 1));
+  ST(stage_ad(ctx, n, ad, ad_off, &d_ad, &d_off));
+  ST(stage_var(ctx, BUF_X2, BUF_X3, n, data, data_off, &d_data, &d_doff));
+  ST(stage_out(ctx, BUF_IN1, n * 64, &d_in)); ST(stage_out(ctx, BUF_IN2, n * 64, &d_out));
+  ST(stage_out(ctx, BUF_IN3, n * 32, &d_c)); ST(stage_out(ctx, BUF_IN4, n * 32, &d_s)); ST(stage_out(ctx, BUF_X4, 2 * n, &d_flags));
+  ST(stage_out(ctx, BUF_OUT0, n, &d_ok));
+  if (out_hash) ST(stage_out(ctx, BUF_OUT1, n * hl, &d_hash));
+  if (out_status) ST(stage_out(ctx, BUF_X5, n, &d_st));
+  HostOut out[3] = {{out_ok, d_ok, 1}, {nullptr, nullptr, 0}, {nullptr, nullptr, 0}};
+  int nout = 1;
+  if (out_hash) out[nout++] = {out_hash, d_hash, hl};
+  if (out_status) out[nout++] = {out_status, d_st, 1};
+  for (int k = 0; k < pc.count; k++) {
+    const size_t o = pc.cut[k], m = pc.cut[k + 1] - pc.cut[k];
+    ST(piece_ready(ctx, k));
+    ST(with_suite(ctx, keys->suite, [&](auto S_) { typedef decltype(S_) S;
+      return ietf_verify_prepared_wire_dev<S>(ctx, keys, m, (const uint32_t*)in[0].dev + o, d_data, d_doff + o, in[1].dev + o * sl, d_ad,
+                                              d_off ? d_off + o : nullptr, d_in + o * 64, d_out + o * 64, d_c + o * 32, d_s + o * 32, d_flags + o * 2,
+                                              d_ok + o, d_hash ? d_hash + o * hl : nullptr, d_st ? d_st + o : nullptr); }));
+    ST(pieces_copy_out(ctx, pc, k, out, nout));
+  }
   return finish_call(ctx);
 }
 // =================================================================================================

@@ -110,10 +110,11 @@ def _dev_ptr(x):
 
 class PreparedPublics:
     """Public keys prepared once for many verifies (vrfs_public_keys_prepare): one fixed-base table per key on the engine's GPU.
-    key_ok[k] = 1 where keys[k] is a key ietf_verify accepts.  Usable as a context manager; release() frees the tables."""
+    key_ok[k] = 1 where keys[k] is a key ietf_verify accepts.  Usable as a context manager; release() frees the tables.
+    from_encodings: made by Engine.public_keys_prepare_encoded, which verify_wire requires."""
 
-    def __init__(self, engine, handle, suite, key_ok):
-        self.engine, self.handle, self.suite, self.key_ok = engine, handle, suite, key_ok
+    def __init__(self, engine, handle, suite, key_ok, from_encodings=False):
+        self.engine, self.handle, self.suite, self.key_ok, self.from_encodings = engine, handle, suite, key_ok, from_encodings
 
     @property
     def n_keys(self):
@@ -134,6 +135,23 @@ class PreparedPublics:
         (Engine.stream) - the caller orders its producers before and its readers after it (e.g. Engine.sync())"""
         self.engine._call("vrfs_ietf_verify_prepared_batch_dev", self.handle, C.c_size_t(n), _dev_ptr(d_key_index), _dev_ptr(d_inp), _dev_ptr(d_outp),
                           _dev_ptr(d_c), _dev_ptr(d_s), _dev_ptr(d_ad), _dev_ptr(d_off), _dev_ptr(d_ok), _dev_ptr(d_status))
+
+    def verify_wire(self, key_index, datas, sig, ad=None, want_hash=True, status=False, out_ok=None, out_hash=None):
+        """Engine.ietf_verify_wire with pk_enc[i] = the encoding of key key_index[i] (vrfs_ietf_verify_prepared_wire_batch; keys from
+        Engine.public_keys_prepare_encoded) -> (ok, beta[, status]) like that call; a key with key_ok = 0 or an index >= n_keys:
+        ITEM_INVALID_DATA"""
+        e = self.engine
+        key_index = np.ascontiguousarray(key_index, dtype=np.uint32).reshape(-1); n = len(key_index)
+        sig = _u8(sig, (n, e.ietf_signature_len(self.suite))); data, doff = pack_var(datas, n); adb, off = pack_var(ad, n)
+        hl = e.hash_len(self.suite)
+        ok = _u8(out_ok, (n,)) if out_ok is not None else np.zeros(n, np.uint8)
+        h = (_u8(out_hash, (n, hl)) if out_hash is not None else np.zeros((n, hl), np.uint8)) if want_hash else None
+        st = np.zeros(n, np.uint8) if status else None
+        e._call("vrfs_ietf_verify_prepared_wire_batch", self.handle, C.c_size_t(n), _p(key_index), _p(data), _p(doff), _p(sig), _p(adb), _p(off),
+                _p(ok), _p(h), _p(st))
+        res = (ok, h) if want_hash else (ok,)
+        res = res + (st,) if status else res
+        return res if len(res) > 1 else res[0]
 
     def release(self):
         if self.handle:
@@ -265,6 +283,17 @@ class Engine:
         h = C.c_void_p()
         self._call("vrfs_public_keys_prepare", suite, C.c_size_t(len(pks)), _p(pks), _p(key_ok), C.byref(h))
         p = PreparedPublics(self, h, suite, key_ok)
+        self._prepared.append(p)
+        return p
+
+    def public_keys_prepare_encoded(self, suite, pk_enc):
+        """(n_keys, point_enc_len) encoded keys -> PreparedPublics (from_encodings=True): each key decoded with the subgroup check
+        once, then prepared like public_keys_prepare; key_ok = 0 where the encoding or the decoded key is rejected
+        (vrfs_public_keys_prepare_encoded).  Its verify_wire verifies serialised signatures by key index."""
+        pk_enc = _u8(pk_enc, (-1, self.point_enc_len(suite))); key_ok = np.zeros(len(pk_enc), np.uint8)
+        h = C.c_void_p()
+        self._call("vrfs_public_keys_prepare_encoded", suite, C.c_size_t(len(pk_enc)), _p(pk_enc), _p(key_ok), C.byref(h))
+        p = PreparedPublics(self, h, suite, key_ok, from_encodings=True)
         self._prepared.append(p)
         return p
 

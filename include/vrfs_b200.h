@@ -144,6 +144,23 @@ vrfs_status vrfs_ietf_verify_prepared_batch(vrfs_ctx*, const vrfs_public_keys*, 
 vrfs_status vrfs_ietf_verify_prepared_batch_dev(vrfs_ctx*, const vrfs_public_keys*, size_t n, const uint32_t* d_key_index,
                                                 const uint8_t* d_input, const uint8_t* d_output, const uint8_t* d_c, const uint8_t* d_s,
                                                 const uint8_t* d_ad, const uint64_t* d_ad_off, uint8_t* d_out_ok, uint8_t* d_out_status /* may be NULL */);
+/* The same from bytes: a signer set published as encoded keys, signatures verified by key index (a block header's author index and
+ * seal).  vrfs_public_keys_prepare_encoded decodes each key once like vrfs_point_decode_checked_batch (canonical, on the curve,
+ * prime-order subgroup) and prepares the decoded points: out_key_ok[k] = 1 iff the encoding decodes AND vrfs_public_keys_prepare
+ * would accept the decoded point.  Such a handle also serves vrfs_ietf_verify_prepared_batch[_dev], exactly like an affine handle
+ * of the decoded points, and no key of it has a small-order component, so the caveat above cannot arise.
+ * vrfs_ietf_verify_prepared_wire_batch: item i is vrfs_ietf_verify_wire_batch with pk_enc[i] = the encoding of key key_index[i] as
+ * given to prepare: out_ok, out_hash and out_status equal that call's byte for byte, for every key encoding.  An item that names a
+ * key with key_ok = 0, or an index >= n_keys, is VRFS_ITEM_INVALID_DATA with ok 0 and a zero hash.  Each key is decoded and
+ * subgroup-checked once at prepare instead of once per item, 4 bytes of key index travel instead of an encoded key, and
+ * U = s*G - c*Y comes from the key's table.  A handle made by vrfs_public_keys_prepare (keys never subgroup-checked) is refused with
+ * VRFS_BAD_ARG.  Handle rules, n_keys range and NULL buffers as above; out_hash may be NULL.  There is no _dev form. */
+vrfs_status vrfs_public_keys_prepare_encoded(vrfs_ctx*, vrfs_suite, size_t n_keys, const uint8_t* pk_enc /*n_keys*enc_len*/,
+                                             uint8_t* out_key_ok /*n_keys, may be NULL*/, vrfs_public_keys** out);
+vrfs_status vrfs_ietf_verify_prepared_wire_batch(vrfs_ctx*, const vrfs_public_keys*, size_t n, const uint32_t* key_index,
+                                                 const uint8_t* data, const uint64_t* data_off, const uint8_t* sig /*n*sig_len*/,
+                                                 const uint8_t* ad, const uint64_t* ad_off,
+                                                 uint8_t* out_ok, uint8_t* out_hash /*n*hash_len, may be NULL*/, uint8_t* out_status /* may be NULL */);
 
 /* pedersen::Prover::prove / Verifier::verify (A.10).  proof = pk_com || r || ok (3 x 64-byte affine) || s || sb (2 x 32 bytes) = 256 bytes. */
 vrfs_status vrfs_pedersen_prove_batch(vrfs_ctx*, vrfs_suite, size_t n, const uint8_t* sk, const uint8_t* input, const uint8_t* output,

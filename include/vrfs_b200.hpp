@@ -183,8 +183,22 @@ class PreparedPublics {
                                                          proof.s.data(), a.ptr(), a.off.data(), ok.data(), status_ptr(errors, n)));
     return ok;
   }
+  // keys as serialised (n x point_enc_len bytes), each deserialised and subgroup-checked once (vrfs_public_keys_prepare_encoded):
+  // key_ok = 0 where Public::deserialize_compressed rejects the encoding or Public::verify rejects the key
+  static PreparedPublics from_compressed(const Suite& s, const Bytes& enc) { return PreparedPublics(s, enc); }
+  // Public::verify_signatures with pk_enc[i] = the encoding of key key_index[i] -> (ok, Output::hash); only for from_compressed sets
+  std::pair<Bytes, Bytes> verify_signatures(const std::vector<uint32_t>& key_index, const std::vector<Bytes>& datas, const Bytes& sigs,
+                                            const std::vector<Bytes>& ad, Errors* errors = nullptr) const {
+    Packed d(datas), a(ad); size_t n = key_index.size(); Bytes ok(n), beta(n * suite_.hash_len());
+    suite_.engine->check(vrfs_ietf_verify_prepared_wire_batch(suite_.engine->ctx(), h_, n, key_index.data(), d.ptr(), d.off.data(), sigs.data(), a.ptr(),
+                                                              a.off.data(), ok.data(), beta.data(), status_ptr(errors, n)));
+    return {std::move(ok), std::move(beta)};
+  }
 
  private:
+  PreparedPublics(const Suite& s, const Bytes& enc) : suite_(s), key_ok_(enc.size() / s.point_enc_len()) {
+    suite_.engine->check(vrfs_public_keys_prepare_encoded(suite_.engine->ctx(), suite_.id, key_ok_.size(), enc.data(), key_ok_.data(), &h_));
+  }
   Suite suite_;
   Bytes key_ok_;
   vrfs_public_keys* h_ = nullptr;
