@@ -18,6 +18,8 @@ SYMBOLS = [
     "vrfs_ietf_prove_batch", "vrfs_ietf_verify_batch", "vrfs_ietf_verify_batch_dev",
     "vrfs_public_keys_prepare", "vrfs_public_keys_release", "vrfs_ietf_verify_prepared_batch", "vrfs_ietf_verify_prepared_batch_dev",
     "vrfs_public_keys_prepare_encoded", "vrfs_ietf_verify_prepared_wire_batch",
+    "vrfs_inputs_prepare", "vrfs_inputs_release", "vrfs_ietf_verify_prepared_io_batch", "vrfs_ietf_verify_prepared_io_batch_dev",
+    "vrfs_ietf_verify_prepared_io_wire_batch",
     "vrfs_pedersen_prove_batch", "vrfs_pedersen_verify_batch",
     "vrfs_suite_ietf_signature_len", "vrfs_point_decode_checked_batch", "vrfs_subgroup_check_batch", "vrfs_ietf_sign_wire_batch", "vrfs_ietf_verify_wire_batch",
     "vrfs_suite_pedersen_signature_len", "vrfs_pedersen_sign_wire_batch", "vrfs_pedersen_verify_wire_batch",

@@ -113,6 +113,16 @@ class PreparedPublic:
         only for keys from Public.prepare_compressed"""
         return self.keys.verify_wire(key_index, datas, signatures, ad, status=status)
 
+    def verify_prepared_input(self, key_index, inputs, input_index, output, ad, proof, status=False):
+        """verify with input[i] = the point of prepared input input_index[i] (`inputs` from Input.prepare) -> uint8[n]
+        (status=True: (ok, Error variant per item)); an input index out of range is ITEM_INVALID_DATA for its item"""
+        return self.keys.verify_io(inputs.inputs, key_index, input_index, output.points, proof.c, proof.s, ad, status=status)
+
+    def verify_signatures_prepared_input(self, key_index, inputs, input_index, signatures, ad=None, status=False):
+        """verify_signatures with datas[i] = the data of prepared input input_index[i] -> (ok flags, Output::hash[, status]);
+        only for keys from Public.prepare_compressed; no hash-to-curve per signature"""
+        return self.keys.verify_io_wire(inputs.inputs, key_index, input_index, signatures, ad, status=status)
+
     def release(self):
         self.keys.release()
 
@@ -133,6 +143,37 @@ class Input:
         """Input::new(data) = Suite::data_to_point; returns (Input, ok flags) for Option<Input>"""
         pts, ok = suite.engine.data_to_point(suite.suite_id, datas)
         return cls(suite, pts), ok
+
+    @staticmethod
+    def prepare(suite, datas):
+        """Input::new of a few inputs that many proofs share (a lottery or beacon round), done once, with a fixed-base table per input
+        point on the suite's GPU -> PreparedInput, whose proofs PreparedPublic verifies by input index"""
+        return PreparedInput(suite, suite.engine.inputs_prepare(suite.suite_id, datas))
+
+
+@dataclass
+class PreparedInput:
+    """Inputs that are reused (Input.prepare)"""
+    suite: Suite
+    inputs: object              # engine.PreparedInputs
+
+    @property
+    def input_ok(self):
+        """Input::new's Option as flags: 0 where no point was found"""
+        return self.inputs.input_ok
+
+    @property
+    def points(self):
+        return self.inputs.points
+
+    def release(self):
+        self.inputs.release()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.release()
 
 
 @dataclass

@@ -243,7 +243,8 @@ HD_INLINE void add_fixed_term(typename Grp<C>::Pt& acc, const uint8_t* sc, const
   }
 }
 
-template <class C, int NV, int NF>
+// MORE: the caller adds further terms to acc after this returns, so the last sum needs its T coordinate even when NF = 0
+template <class C, int NV, int NF, bool MORE = false>
 HD_INLINE bool lincomb_item(const LincombArgs& A, uint32_t item, typename Grp<C>::Entry* slab, typename Grp<C>::Pt& acc) {
   typedef Grp<C> G;
   typedef typename C::F F;
@@ -306,7 +307,7 @@ HD_INLINE bool lincomb_item(const LincombArgs& A, uint32_t item, typename Grp<C>
         copy_words16(&e, &slab[t * TBL_ENTRIES + idx]);
         // the last addition of a window is followed by the next window's doublings (which do not read T) or, after the last
         // window, by nothing but the fixed-base additions: its T is only computed when somebody reads it
-        G::add_entry(&acc, &e, (d < 0) != kneg[t], VRFS_SKIP_T ? (t != NT - 1 || (w == 0 && NF > 0)) : true);
+        G::add_entry(&acc, &e, (d < 0) != kneg[t], VRFS_SKIP_T ? (t != NT - 1 || (w == 0 && (NF > 0 || MORE))) : true);
       }
     }
   }
@@ -370,6 +371,29 @@ template <class C> HD_INLINE void lincomb_keyed_item(const KeyedArgs& A, uint32_
   // n_keys x 400 KB is DRAM-resident beyond a few hundred keys: the records of all windows go to L2 up front, as for the G table
   add_fixed_term<C, KEY_FIX_BITS, true>(acc, A.c + (size_t)item * 32,
                                         reinterpret_cast<const typename G::FixEntry*>(A.key_tables) + (size_t)k * key_table_entries<C>(), true, topw_c, true);
+}
+
+// ---- prepared inputs: V = s*I_j - c*O of an IETF verify against a known VRF input ---------------------------------------------
+// I_j has a table of the prepared-key layout (vrfs_inputs_prepare), so s*I_j is 32-33 mixed additions; c*O stays the variable-base
+// Straus loop of lincomb_item<C, 1, 0> (GLV halves on Bandersnatch, sc_bits-trimmed windows for a 16-byte challenge) on a slab of
+// one base.  L.var[0] = the c*O term, L.fix[0] = the s*I term with `table` = the n_inputs tables back to back.
+struct IoArgs {
+  LincombArgs L;
+  const uint32_t* input_index;  // n: j of item i (>= n_inputs: the table of input 0 is read; the gather kernel rejects the item)
+  uint32_t n_inputs;
+};
+template <class C>
+HD_INLINE bool lincomb_io_item(const IoArgs& A, uint32_t item, typename Grp<C>::Entry* slab, typename Grp<C>::Pt& acc) {
+  typedef Grp<C> G;
+  const bool ok = lincomb_item<C, 1, 0, true>(A.L, item, slab, acc);
+  uint32_t j = A.input_index[item];
+  if (j >= A.n_inputs) j = 0;
+  const FixTerm& f = A.L.fix[0];
+  // FAR: up to 65536 tables of ~400 KB, far larger than L2 - as for the key tables of lincomb_keyed_item
+  add_fixed_term<C, KEY_FIX_BITS, true>(acc, f.sc + (size_t)item * f.sc_stride,
+                                        reinterpret_cast<const typename G::FixEntry*>(f.table) + (size_t)j * key_table_entries<C>(), f.negate != 0,
+                                        fix_windows<C, KEY_FIX_BITS>() - 1, true);
+  return ok;
 }
 
 // one fixed-base table entry: (d * 256^w) * B.  Used once per context by the table kernel.

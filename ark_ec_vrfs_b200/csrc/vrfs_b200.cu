@@ -156,6 +156,31 @@ __global__ void __launch_bounds__(128) k_gather_keys(uint32_t n, const uint32_t*
   copy_words16(reinterpret_cast<uint4(*)[4]>(out_rows) + i, &r);
   if (k >= n_keys || !key_ok[k]) valid[i] = 0;
 }
+// prepared inputs (vrfs_inputs_prepare): V = s*I_j - c*O (lincomb.cuh lincomb_io_item) on the persistent grid of k_lincomb - the
+// variable base c*O needs a window-table slab, which the grid keeps per resident thread instead of per item.  128-thread blocks:
+// at 128 registers the variable-base loop spills on Bandersnatch (GLV) and the short-Weierstrass suites, as k_lincomb<C, 1, 0>
+// does; 3 blocks per SM (12 warps) give them ~170 registers and no spills, the other twisted-Edwards suites keep 16 warps.
+#define IO_THREADS 128
+template <class C> constexpr int io_min_blocks() { return C::IS_TE && Grp<C>::SPLIT == 1 ? 4 : 3; }
+template <class C>
+__global__ void __launch_bounds__(IO_THREADS, io_min_blocks<C>()) k_lincomb_io(IoArgs A) {
+  const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31u;
+  typename Grp<C>::Entry* slab = reinterpret_cast<typename Grp<C>::Entry*>(A.L.slab + (size_t)tid * slab_bytes<C>(1));
+  for (;;) {
+    uint32_t base = 0;
+    if (lane == 0) base = atomicAdd(A.L.next_item, 32u);
+    base = __shfl_sync(0xffffffffu, base, 0);
+    if (base >= A.L.n) break;
+    const uint32_t item = base + lane;
+    if (item < A.L.n) {
+      typename Grp<C>::Pt acc;
+      const bool ok = lincomb_io_item<C>(A, item, slab, acc);
+      Grp<C>::store_xyz(A.L.out_xyz + (size_t)item * 24, acc);
+      if (A.L.valid != nullptr && !ok) A.L.valid[item] = 0;
+    }
+    __syncwarp();
+  }
+}
 
 // integer-pipe roofline microbenchmarks (SURVEY 8d): independent multiply-accumulate chains per thread
 template <int VARIANT>
@@ -275,8 +300,8 @@ struct DevBuf {
 };
 enum { BUF_IN0, BUF_IN1, BUF_IN2, BUF_IN3, BUF_IN4, BUF_AD, BUF_OFF, BUF_OUT0, BUF_OUT1, BUF_W0, BUF_W1, BUF_W2, BUF_W3, BUF_VALID, BUF_SLAB,
        BUF_X0, BUF_X1, BUF_X2, BUF_X3, BUF_X4, BUF_X5, BUF_ZINV, BUF_SLAB2,
-       BUF_PB0, BUF_PB1, BUF_PB2, BUF_KEYROWS, BUF_COUNT };   // X*: wire-format staging (encoded keys, signatures, h2c data, flags); PB*: Pedersen batch verification;
-                                                             // KEYROWS: the key rows a prepared-key verify gathers for its finish kernel
+       BUF_PB0, BUF_PB1, BUF_PB2, BUF_KEYROWS, BUF_INROWS, BUF_COUNT };   // X*: wire-format staging (encoded keys, signatures, h2c data, flags); PB*: Pedersen batch verification;
+                                                             // KEYROWS / INROWS: the key / input rows a prepared verify gathers for its finish kernel
 
 #define MAX_TIMED 64
 #ifndef VRFS_HOST_PIECES
@@ -561,15 +586,15 @@ static vrfs_status side_join(vrfs_ctx* ctx) { CU(cudaEventRecord(ctx->ev_join, c
 // Persistent grid of a lincomb kernel: as many blocks as fit on the GPU at once, but no more than `threads` threads need; each
 // thread's window-table slab of `slab_per_thread` bytes in buffer `buf`, and the kernel's work counter behind the slabs (zeroed).
 static vrfs_status lincomb_grid(vrfs_ctx* ctx, const void* kernel, size_t threads, size_t slab_per_thread, int buf, cudaStream_t stream,
-                                LincombArgs* A, uint32_t* blocks) {
+                                LincombArgs* A, uint32_t* blocks, unsigned block_threads = LINCOMB_THREADS) {
   int per_sm = 0;
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, LINCOMB_THREADS, 0));
+  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, (int)block_threads, 0));
   if (per_sm < 1) per_sm = 1;
 #ifdef LINCOMB_MAXBLOCKS
   if (per_sm > LINCOMB_MAXBLOCKS) per_sm = LINCOMB_MAXBLOCKS;       // tuning builds: resident threads per SM (the slab scales with them)
 #endif
-  *blocks = (uint32_t)std::min((size_t)ctx->sms * per_sm, (threads + LINCOMB_THREADS - 1) / LINCOMB_THREADS);
-  const size_t slabs = (size_t)*blocks * LINCOMB_THREADS * slab_per_thread;
+  *blocks = (uint32_t)std::min((size_t)ctx->sms * per_sm, (threads + block_threads - 1) / block_threads);
+  const size_t slabs = (size_t)*blocks * block_threads * slab_per_thread;
   void* slab = nullptr;
   ST(ensure(ctx, buf, slabs + 256, &slab));
   A->slab = (uint8_t*)slab;
@@ -599,6 +624,14 @@ static vrfs_status launch_lincomb_verify_pair(vrfs_ctx* ctx, LincombArgs U, Linc
   U.slab = V.slab; U.next_item = V.next_item;                         // one slab and one task counter for both combinations
   k_lincomb_verify_pair<C><<<blocks, LINCOMB_THREADS, 0, ctx->stream>>>(U, V);
   LAUNCHED_AS(ctx, "lincomb<1,1>+<2,0>");
+  return VRFS_OK;
+}
+template <class C>
+static vrfs_status launch_lincomb_io(vrfs_ctx* ctx, IoArgs A) {
+  uint32_t blocks = 0;
+  ST(lincomb_grid(ctx, (const void*)k_lincomb_io<C>, A.L.n, slab_bytes<C>(1), BUF_SLAB, ctx->stream, &A.L, &blocks, IO_THREADS));
+  k_lincomb_io<C><<<blocks, IO_THREADS, 0, ctx->stream>>>(A);
+  LAUNCHED_AS(ctx, "lincomb_io");
   return VRFS_OK;
 }
 
@@ -2206,21 +2239,30 @@ struct vrfs_public_keys {
   const uint8_t* rows;    // n_keys x 64: the keys as given, or as decoded (the finish kernel encodes pk from them)
   const uint8_t* key_ok;  // n_keys
   bool from_encodings;    // vrfs_public_keys_prepare_encoded: every key with key_ok = 1 passed the decoder's subgroup check
+  bool is_inputs;         // the record of a vrfs_inputs handle
 };
-// `encoded`: pks holds n_keys encodings (Codec::point_encode), decoded and subgroup-checked by k_decode_checked into the rows
-// the tables are built from; key_ok = that decode's flag AND the affine key test of k_key_table_powers
+// Prepared VRF inputs (vrfs_inputs_prepare) share the record, the build and the lifetime rules of prepared keys: the rows are the
+// input points Input::new(data) gave, key_ok is input_ok, and the tables serve s*I as the key tables serve c*Y.
+struct vrfs_inputs : vrfs_public_keys {};
+static void delete_record(vrfs_public_keys* h) {
+  if (h->is_inputs) delete static_cast<vrfs_inputs*>(h); else delete h;
+}
+// What the rows are made from: affine points; encodings (Codec::point_encode), decoded and subgroup-checked by k_decode_checked;
+// or VRF input data, hashed to the curve by data_to_point_dev.  key_ok = the decode or hash-to-curve flag AND the affine key test
+// of k_key_table_powers.
+enum PrepareFrom { FROM_POINTS, FROM_ENCODINGS, FROM_DATA };
 template <class S>
-static vrfs_status public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n_keys, const uint8_t* pks, bool encoded, uint8_t* out_key_ok,
-                                       vrfs_public_keys** out) {
+static vrfs_status public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n_keys, const uint8_t* pks, const uint64_t* data_off, PrepareFrom from,
+                                       uint8_t* out_key_ok, uint8_t* out_rows, vrfs_public_keys** out) {
   typedef typename S::C C;
   typedef typename Grp<C>::FixEntry E;
   const size_t tbytes = n_keys * key_table_entries<C>() * sizeof(E);
-  vrfs_public_keys* h = new (std::nothrow) vrfs_public_keys();
+  vrfs_public_keys* h = from == FROM_DATA ? new (std::nothrow) vrfs_inputs() : new (std::nothrow) vrfs_public_keys();
   if (!h) return fail(ctx, VRFS_CUDA_ERROR, "out of host memory");
-  h->ctx = ctx; h->suite = suite; h->n_keys = n_keys; h->from_encodings = encoded;
+  h->ctx = ctx; h->suite = suite; h->n_keys = n_keys; h->from_encodings = from == FROM_ENCODINGS; h->is_inputs = from == FROM_DATA;
   cudaError_t e = cudaMalloc(&h->mem, tbytes + n_keys * 65);
   if (e != cudaSuccess) {
-    cudaGetLastError(); delete h;
+    cudaGetLastError(); delete_record(h);
     return fail(ctx, VRFS_CUDA_ERROR, "cudaMalloc of %zu bytes of key tables failed: %s", tbytes + n_keys * 65, cudaGetErrorString(e));
   }
   h->tables = h->mem; h->rows = (const uint8_t*)h->mem + tbytes; h->key_ok = h->rows + n_keys * 64;
@@ -2228,12 +2270,18 @@ static vrfs_status public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n
   auto build = [&]() -> vrfs_status {
     const uint8_t* d_pk;
     uint8_t* d_dec_ok = nullptr;
-    if (encoded) {
+    if (from == FROM_ENCODINGS) {
       const uint8_t* d_enc; uint8_t* d_dec;
       ST(stage_in(ctx, BUF_X0, pks, n_keys * S::ENC_LEN, &d_enc));
       ST(stage_out(ctx, BUF_IN0, n_keys * 64, &d_dec)); ST(stage_out(ctx, BUF_X4, n_keys, &d_dec_ok));
       ST(decode_checked_launch<S>(ctx, n_keys, d_enc, S::ENC_LEN, d_dec, nullptr, 0, nullptr, d_dec_ok));
       d_pk = d_dec;
+    } else if (from == FROM_DATA) {   // staged like the data of vrfs_ietf_verify_wire_batch
+      const uint8_t* d_data; const uint64_t* d_doff; uint8_t* d_pts;
+      ST(stage_var(ctx, BUF_X2, BUF_X3, n_keys, pks, data_off, &d_data, &d_doff));
+      ST(stage_out(ctx, BUF_IN0, n_keys * 64, &d_pts)); ST(stage_out(ctx, BUF_X4, n_keys, &d_dec_ok));
+      ST(data_to_point_dev<S>(ctx, n_keys, d_data, d_doff, d_pts, d_dec_ok));
+      d_pk = d_pts;
     } else {
       ST(stage_in(ctx, BUF_IN0, pks, n_keys * 64, &d_pk));
     }
@@ -2242,15 +2290,16 @@ static vrfs_status public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n
     const size_t windows = n_keys * fix_windows<C, KEY_FIX_BITS>();
     k_key_table_windows<C><<<(unsigned)((windows + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n_keys, (E*)h->mem);
     LAUNCHED_AS(ctx, "key_table_windows");
-    if (encoded) {   // key_ok &= decode flag.  A failed decode leaves a zero row, which k_key_table_powers rejects on its own; this does not rely on it
+    if (d_dec_ok) {   // key_ok &= decode / hash-to-curve flag.  A failure leaves a zero row, which k_key_table_powers rejects on its own; this does not rely on it
       k_merge_flags<<<item_blocks(n_keys), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n_keys, d_dec_ok, nullptr, (uint8_t*)h->key_ok, nullptr, 0u, nullptr);
       LAUNCHED_AS(ctx, "merge_flags");
     }
     if (out_key_ok) ST(copy_out(ctx, out_key_ok, h->key_ok, n_keys));
+    if (out_rows) ST(copy_out(ctx, out_rows, h->rows, n_keys * 64));
     return finish_call(ctx);
   };
   const vrfs_status st = build();
-  if (st != VRFS_OK) { cudaStreamSynchronize(ctx->stream); cudaFree(h->mem); delete h; return st; }
+  if (st != VRFS_OK) { cudaStreamSynchronize(ctx->stream); cudaFree(h->mem); delete_record(h); return st; }
   ctx->prepared_keys.push_back(h);
   *out = h;
   return VRFS_OK;
@@ -2262,7 +2311,7 @@ extern "C" vrfs_status vrfs_public_keys_prepare(vrfs_ctx* ctx, vrfs_suite suite,
   if (!pks) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   if (n_keys < 1 || n_keys > VRFS_MAX_PREPARED_KEYS) return fail(ctx, VRFS_BAD_ARG, "n_keys must be in 1..%d", VRFS_MAX_PREPARED_KEYS);
   ST(begin_call(ctx, suite, n_keys));
-  return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return public_keys_prepare<S>(ctx, suite, n_keys, pks, false, out_key_ok, out); });
+  return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return public_keys_prepare<S>(ctx, suite, n_keys, pks, nullptr, FROM_POINTS, out_key_ok, nullptr, out); });
 }
 extern "C" vrfs_status vrfs_public_keys_prepare_encoded(vrfs_ctx* ctx, vrfs_suite suite, size_t n_keys, const uint8_t* pk_enc, uint8_t* out_key_ok,
                                                         vrfs_public_keys** out) {
@@ -2272,7 +2321,21 @@ extern "C" vrfs_status vrfs_public_keys_prepare_encoded(vrfs_ctx* ctx, vrfs_suit
   if (!pk_enc) return fail(ctx, VRFS_BAD_ARG, "null buffer");
   if (n_keys < 1 || n_keys > VRFS_MAX_PREPARED_KEYS) return fail(ctx, VRFS_BAD_ARG, "n_keys must be in 1..%d", VRFS_MAX_PREPARED_KEYS);
   ST(begin_call(ctx, suite, n_keys));
-  return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return public_keys_prepare<S>(ctx, suite, n_keys, pk_enc, true, out_key_ok, out); });
+  return with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S; return public_keys_prepare<S>(ctx, suite, n_keys, pk_enc, nullptr, FROM_ENCODINGS, out_key_ok, nullptr, out); });
+}
+extern "C" vrfs_status vrfs_inputs_prepare(vrfs_ctx* ctx, vrfs_suite suite, size_t n_inputs, const uint8_t* data, const uint64_t* data_off,
+                                           uint8_t* out_input_ok, uint8_t* out_points, vrfs_inputs** out) {
+  if (!ctx || !out) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  *out = nullptr;
+  if (!data_off) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  if (n_inputs < 1 || n_inputs > VRFS_MAX_PREPARED_KEYS) return fail(ctx, VRFS_BAD_ARG, "n_inputs must be in 1..%d", VRFS_MAX_PREPARED_KEYS);
+  ST(begin_call(ctx, suite, n_inputs));
+  vrfs_public_keys* h = nullptr;
+  ST(with_suite(ctx, suite, [&](auto S_) { typedef decltype(S_) S;
+    return public_keys_prepare<S>(ctx, suite, n_inputs, data, data_off, FROM_DATA, out_input_ok, out_points, &h); }));
+  *out = static_cast<vrfs_inputs*>(h);
+  return VRFS_OK;
 }
 // Same lifetime rules as vrfs_msm_bases (vrfs_msm_g1_release): released before or after the context, orphaned by vrfs_ctx_destroy.
 extern "C" void vrfs_public_keys_release(vrfs_public_keys* h) {
@@ -2288,8 +2351,9 @@ extern "C" void vrfs_public_keys_release(vrfs_public_keys* h) {
     auto& v = ctx->prepared_keys;
     v.erase(std::remove(v.begin(), v.end(), h), v.end());
   }
-  delete h;
+  delete_record(h);
 }
+extern "C" void vrfs_inputs_release(vrfs_inputs* h) { vrfs_public_keys_release(h); }
 static void orphan_public_keys(vrfs_ctx* ctx) {   // called by vrfs_ctx_destroy (device set, stream synchronised)
   std::lock_guard<std::mutex> g(g_handles_mu);
   for (vrfs_public_keys* h : ctx->prepared_keys) { cudaFree(h->mem); h->mem = nullptr; h->ctx = nullptr; }
@@ -2298,11 +2362,13 @@ static void orphan_public_keys(vrfs_ctx* ctx) {   // called by vrfs_ctx_destroy 
 
 // U = s*G - c*Y_k (k_lincomb_keyed: both terms fixed-base), V = s*I - c*O as in ietf_verify_dev, the finish kernel of ietf_verify_dev
 // on the key rows `pk` with the flags `valid` that the caller's gather left.  Small batches run U on the side stream beside V, like
-// ietf_verify_dev.
+// ietf_verify_dev.  With prepared inputs `pin`, V = s*I_j - c*O over input input_index[i]'s table (k_lincomb_io); `input` then holds
+// the gathered input rows, which the finish kernel encodes.
 template <class S>
 static vrfs_status ietf_verify_keyed_dev(vrfs_ctx* ctx, const vrfs_public_keys* h, size_t n, const uint32_t* key_index, const uint8_t* pk,
                                          const uint8_t* input, const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad,
-                                         const uint64_t* ad_off, uint8_t* valid, uint8_t* out_ok, uint8_t* out_status) {
+                                         const uint64_t* ad_off, uint8_t* valid, uint8_t* out_ok, uint8_t* out_status,
+                                         const vrfs_public_keys* pin = nullptr, const uint32_t* input_index = nullptr) {
   typedef typename S::C C;
   void *u = nullptr, *v = nullptr;
   ST(need_tables<S>(ctx));
@@ -2317,42 +2383,74 @@ static vrfs_status ietf_verify_keyed_dev(vrfs_ctx* ctx, const vrfs_public_keys* 
   LincombArgs A = {};
   A.n = (uint32_t)n;
   A.valid = valid;
-  A.var[0] = {input, 64, s, 32, 0, 0};
-  A.var[1] = {output, 64, c, 32, 1, cbits};
   A.out_xyz = (uint32_t*)v;
-  ST((launch_lincomb<C, 2, 0>(ctx, A)));
+  if (pin) {
+    IoArgs B = {A, input_index, (uint32_t)pin->n_keys};
+    B.L.var[0] = {output, 64, c, 32, 1, cbits};
+    B.L.fix[0] = {s, 32, 0, pin->tables};
+    ST(launch_lincomb_io<C>(ctx, B));
+  } else {
+    A.var[0] = {input, 64, s, 32, 0, 0};
+    A.var[1] = {output, 64, c, 32, 1, cbits};
+    ST((launch_lincomb<C, 2, 0>(ctx, A)));
+  }
   if (split) ST(side_join(ctx));
   k_ietf_verify_finish<S><<<(unsigned)((n + 128 * FINISH_K - 1) / (128 * FINISH_K)), 128, 0, ctx->stream>>>((uint32_t)n, pk, input, output, c, (const uint32_t*)u,
                                                                                 (const uint32_t*)v, ad, ad_off, valid, out_ok, out_status);
   LAUNCHED_AS(ctx, "ietf_verify_finish");
   return VRFS_OK;
 }
+// item i's row of the prepared inputs into `rows` (k_gather_keys does this for any row table); flag[i] = 0 for an index out of range
+// or an input with input_ok = 0
+static vrfs_status gather_inputs(vrfs_ctx* ctx, const vrfs_public_keys* pin, size_t n, const uint32_t* input_index, uint8_t* rows, uint8_t* flag) {
+  k_gather_keys<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n, input_index, (uint32_t)pin->n_keys, pin->rows, pin->key_ok, rows, flag);
+  LAUNCHED_AS(ctx, "gather_inputs");
+  return VRFS_OK;
+}
+// With prepared inputs `pin` the input points are gathered by input_index (`input` is not read) and V comes from their tables.
 template <class S>
 static vrfs_status ietf_verify_prepared_dev(vrfs_ctx* ctx, const vrfs_public_keys* h, size_t n, const uint32_t* key_index, const uint8_t* input,
                                             const uint8_t* output, const uint8_t* c, const uint8_t* s, const uint8_t* ad, const uint64_t* ad_off,
-                                            uint8_t* out_ok, uint8_t* out_status) {
+                                            uint8_t* out_ok, uint8_t* out_status, const vrfs_public_keys* pin = nullptr,
+                                            const uint32_t* input_index = nullptr) {
   void *valid = nullptr, *pk = nullptr;
   ST(ensure(ctx, BUF_VALID, n, &valid));
   ST(ensure(ctx, BUF_KEYROWS, n * 64, &pk));
   CU(cudaMemsetAsync(valid, 1, n, ctx->stream));
   k_gather_keys<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n, key_index, (uint32_t)h->n_keys, h->rows, h->key_ok, (uint8_t*)pk, (uint8_t*)valid);
   LAUNCHED_AS(ctx, "gather_keys");
-  return ietf_verify_keyed_dev<S>(ctx, h, n, key_index, (const uint8_t*)pk, input, output, c, s, ad, ad_off, (uint8_t*)valid, out_ok, out_status);
+  if (pin) {
+    void* rows = nullptr;
+    ST(ensure(ctx, BUF_INROWS, n * 64, &rows));
+    ST(gather_inputs(ctx, pin, n, input_index, (uint8_t*)rows, (uint8_t*)valid));
+    input = (const uint8_t*)rows;
+  }
+  return ietf_verify_keyed_dev<S>(ctx, h, n, key_index, (const uint8_t*)pk, input, output, c, s, ad, ad_off, (uint8_t*)valid, out_ok, out_status, pin,
+                                  input_index);
 }
 // serialised signature + data + key index -> verdict (+ Output::hash of accepted items): ietf_verify_wire_dev with the key taken
 // from the prepared set.  k_wire_prepared_unpack stands for the decode, parse and gather kernels; flags = wellformed | h2c ok (2n).
+// With prepared inputs `pin` the gather of item i's input row stands for hash-to-curve (`data` is not read): its flag is the h2c
+// flag, so a bad input index or an input with input_ok = 0 ends like data without a point.
 template <class S>
 static vrfs_status ietf_verify_prepared_wire_dev(vrfs_ctx* ctx, const vrfs_public_keys* h, size_t n, const uint32_t* key_index, const uint8_t* data,
                                                  const uint64_t* data_off, const uint8_t* sig, const uint8_t* ad, const uint64_t* ad_off, uint8_t* input,
-                                                 uint8_t* output, uint8_t* c, uint8_t* s, uint8_t* flags, uint8_t* out_ok, uint8_t* out_hash, uint8_t* out_status) {
+                                                 uint8_t* output, uint8_t* c, uint8_t* s, uint8_t* flags, uint8_t* out_ok, uint8_t* out_hash, uint8_t* out_status,
+                                                 const vrfs_public_keys* pin = nullptr, const uint32_t* input_index = nullptr) {
   void *valid = nullptr, *pk = nullptr;
   ST(ensure(ctx, BUF_VALID, n, &valid));
   ST(ensure(ctx, BUF_KEYROWS, n * 64, &pk));
   k_wire_prepared_unpack<S><<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, key_index, (uint32_t)h->n_keys, h->rows, h->key_ok, sig,
                                                                               (uint8_t*)pk, output, c, s, (uint8_t*)valid, flags);
   LAUNCHED_AS(ctx, "wire_prepared_unpack");
-  ST(data_to_point_dev<S>(ctx, n, data, data_off, input, flags + n));
-  ST(ietf_verify_keyed_dev<S>(ctx, h, n, key_index, (const uint8_t*)pk, input, output, c, s, ad, ad_off, (uint8_t*)valid, out_ok, out_status));
+  if (pin) {
+    CU(cudaMemsetAsync(flags + n, 1, n, ctx->stream));
+    ST(gather_inputs(ctx, pin, n, input_index, input, flags + n));
+  } else {
+    ST(data_to_point_dev<S>(ctx, n, data, data_off, input, flags + n));
+  }
+  ST(ietf_verify_keyed_dev<S>(ctx, h, n, key_index, (const uint8_t*)pk, input, output, c, s, ad, ad_off, (uint8_t*)valid, out_ok, out_status, pin,
+                              input_index));
   if (out_hash) {
     k_point_to_hash<S><<<item_blocks(n), ITEM_THREADS, 0, ctx->stream>>>((uint32_t)n, output, out_hash);
     LAUNCHED_AS(ctx, "point_to_hash");
@@ -2363,6 +2461,13 @@ static vrfs_status ietf_verify_prepared_wire_dev(vrfs_ctx* ctx, const vrfs_publi
 }
 static vrfs_status check_keys(vrfs_ctx* ctx, const vrfs_public_keys* h) {
   if (!h || h->ctx != ctx) return fail(ctx, VRFS_BAD_ARG, "prepared keys of another (or a destroyed) context");
+  if (h->is_inputs) return fail(ctx, VRFS_BAD_ARG, "prepared inputs where prepared keys are expected");
+  return VRFS_OK;
+}
+static vrfs_status check_inputs(vrfs_ctx* ctx, const vrfs_public_keys* keys, const vrfs_inputs* in) {
+  ST(check_keys(ctx, keys));
+  if (!in || in->ctx != ctx || !in->is_inputs) return fail(ctx, VRFS_BAD_ARG, "prepared inputs of another (or a destroyed) context");
+  if (in->suite != keys->suite) return fail(ctx, VRFS_BAD_ARG, "prepared keys and inputs of different suites");
   return VRFS_OK;
 }
 extern "C" vrfs_status vrfs_ietf_verify_prepared_batch_dev(vrfs_ctx* ctx, const vrfs_public_keys* keys, size_t n, const uint32_t* key_index,
@@ -2446,6 +2551,94 @@ extern "C" vrfs_status vrfs_ietf_verify_prepared_wire_batch(vrfs_ctx* ctx, const
       return ietf_verify_prepared_wire_dev<S>(ctx, keys, m, (const uint32_t*)in[0].dev + o, d_data, d_doff + o, in[1].dev + o * sl, d_ad,
                                               d_off ? d_off + o : nullptr, d_in + o * 64, d_out + o * 64, d_c + o * 32, d_s + o * 32, d_flags + o * 2,
                                               d_ok + o, d_hash ? d_hash + o * hl : nullptr, d_st ? d_st + o : nullptr); }));
+    ST(pieces_copy_out(ctx, pc, k, out, nout));
+  }
+  return finish_call(ctx);
+}
+// proofs against prepared keys AND prepared inputs, both named by index: item i is vrfs_ietf_verify_prepared_batch with
+// input[i] = the point of input input_index[i].  Host form staged in pieces like that call, 136 B per item instead of 196.
+extern "C" vrfs_status vrfs_ietf_verify_prepared_io_batch_dev(vrfs_ctx* ctx, const vrfs_public_keys* keys, const vrfs_inputs* inputs, size_t n,
+                                                              const uint32_t* key_index, const uint32_t* input_index, const uint8_t* output,
+                                                              const uint8_t* c, const uint8_t* s, const uint8_t* ad, const uint64_t* ad_off,
+                                                              uint8_t* out_ok, uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  ST(check_inputs(ctx, keys, inputs));
+  if (n == 0) return VRFS_OK;
+  if (!key_index || !input_index || !output || !c || !s || !out_ok || (ad && !ad_off)) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  if (!aligned16(key_index) || !aligned16(input_index) || !aligned16(output) || !aligned16(c) || !aligned16(s))
+    return fail(ctx, VRFS_BAD_ARG, "device buffers must be 16-byte aligned");
+  ST(begin_call(ctx, keys->suite, n));
+  return with_suite(ctx, keys->suite, [&](auto S_) { typedef decltype(S_) S;
+    return ietf_verify_prepared_dev<S>(ctx, keys, n, key_index, nullptr, output, c, s, ad, ad_off, out_ok, out_status, inputs, input_index); });
+}
+extern "C" vrfs_status vrfs_ietf_verify_prepared_io_batch(vrfs_ctx* ctx, const vrfs_public_keys* keys, const vrfs_inputs* inputs, size_t n,
+                                                          const uint32_t* key_index, const uint32_t* input_index, const uint8_t* output,
+                                                          const uint8_t* c, const uint8_t* s, const uint8_t* ad, const uint64_t* ad_off,
+                                                          uint8_t* out_ok, uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  ST(check_inputs(ctx, keys, inputs));
+  if (n == 0) return VRFS_OK;
+  if (!key_index || !input_index || !output || !c || !s || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  ST(begin_call(ctx, keys->suite, n));
+  const uint8_t* d_ad; const uint64_t* d_off; uint8_t *d_ok, *d_st = nullptr;
+  ST(stage_ad(ctx, n, ad, ad_off, &d_ad, &d_off));
+  ST(stage_out(ctx, BUF_OUT0, n, &d_ok));
+  if (out_status) ST(stage_out(ctx, BUF_OUT1, n, &d_st));
+  HostIn in[5] = {{BUF_IN0, key_index, 4, false, nullptr}, {BUF_IN1, input_index, 4, false, nullptr}, {BUF_IN2, output, 64, false, nullptr},
+                  {BUF_IN3, c, 32, false, nullptr}, {BUF_IN4, s, 32, false, nullptr}};
+  Pieces pc;
+  ST(stage_in_pieces(ctx, n, in, 5, &pc, 2));
+  for (int k = 0; k < pc.count; k++) {
+    const size_t o = pc.cut[k], m = pc.cut[k + 1] - pc.cut[k];
+    ST(piece_ready(ctx, k));
+    ST(with_suite(ctx, keys->suite, [&](auto S_) { typedef decltype(S_) S;
+      return ietf_verify_prepared_dev<S>(ctx, keys, m, (const uint32_t*)in[0].dev + o, nullptr, in[2].dev + o * 64, in[3].dev + o * 32,
+                                         in[4].dev + o * 32, d_ad, d_off ? d_off + o : nullptr, d_ok + o, d_st ? d_st + o : nullptr, inputs,
+                                         (const uint32_t*)in[1].dev + o); }));
+  }
+  ST(copy_out(ctx, out_ok, d_ok, n));
+  if (out_status) ST(copy_out(ctx, out_status, d_st, n));
+  return finish_call(ctx);
+}
+// serialised signatures by key index and input index: vrfs_ietf_verify_prepared_wire_batch with data[i] = the data of input
+// input_index[i], without hash-to-curve.  Staged like that call, minus the data.
+extern "C" vrfs_status vrfs_ietf_verify_prepared_io_wire_batch(vrfs_ctx* ctx, const vrfs_public_keys* keys, const vrfs_inputs* inputs, size_t n,
+                                                               const uint32_t* key_index, const uint32_t* input_index, const uint8_t* sig,
+                                                               const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_hash,
+                                                               uint8_t* out_status) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  ST(check_inputs(ctx, keys, inputs));
+  if (!keys->from_encodings) return fail(ctx, VRFS_BAD_ARG, "prepared keys not made from encodings (vrfs_public_keys_prepare_encoded)");
+  if (n == 0) return VRFS_OK;
+  if (!key_index || !input_index || !sig || !out_ok) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  ST(begin_call(ctx, keys->suite, n));
+  const size_t sl = (size_t)vrfs_suite_ietf_signature_len(keys->suite), hl = (size_t)vrfs_suite_hash_len(keys->suite);
+  const uint8_t* d_ad; const uint64_t* d_off;
+  uint8_t *d_in, *d_out, *d_c, *d_s, *d_flags, *d_ok, *d_hash = nullptr, *d_st = nullptr;
+  HostIn in[3] = {{BUF_X0, key_index, 4, false, nullptr}, {BUF_X2, input_index, 4, false, nullptr}, {BUF_X1, sig, sl, false, nullptr}};
+  Pieces pc;
+  ST(stage_in_pieces(ctx, n, in, 3, &pc, 1));
+  ST(stage_ad(ctx, n, ad, ad_off, &d_ad, &d_off));
+  ST(stage_out(ctx, BUF_IN1, n * 64, &d_in)); ST(stage_out(ctx, BUF_IN2, n * 64, &d_out));
+  ST(stage_out(ctx, BUF_IN3, n * 32, &d_c)); ST(stage_out(ctx, BUF_IN4, n * 32, &d_s)); ST(stage_out(ctx, BUF_X4, 2 * n, &d_flags));
+  ST(stage_out(ctx, BUF_OUT0, n, &d_ok));
+  if (out_hash) ST(stage_out(ctx, BUF_OUT1, n * hl, &d_hash));
+  if (out_status) ST(stage_out(ctx, BUF_X5, n, &d_st));
+  HostOut out[3] = {{out_ok, d_ok, 1}, {nullptr, nullptr, 0}, {nullptr, nullptr, 0}};
+  int nout = 1;
+  if (out_hash) out[nout++] = {out_hash, d_hash, hl};
+  if (out_status) out[nout++] = {out_status, d_st, 1};
+  for (int k = 0; k < pc.count; k++) {
+    const size_t o = pc.cut[k], m = pc.cut[k + 1] - pc.cut[k];
+    ST(piece_ready(ctx, k));
+    ST(with_suite(ctx, keys->suite, [&](auto S_) { typedef decltype(S_) S;
+      return ietf_verify_prepared_wire_dev<S>(ctx, keys, m, (const uint32_t*)in[0].dev + o, nullptr, nullptr, in[2].dev + o * sl, d_ad,
+                                              d_off ? d_off + o : nullptr, d_in + o * 64, d_out + o * 64, d_c + o * 32, d_s + o * 32, d_flags + o * 2,
+                                              d_ok + o, d_hash ? d_hash + o * hl : nullptr, d_st ? d_st + o : nullptr, inputs,
+                                              (const uint32_t*)in[1].dev + o); }));
     ST(pieces_copy_out(ctx, pc, k, out, nout));
   }
   return finish_call(ctx);

@@ -153,9 +153,70 @@ class PreparedPublics:
         res = res + (st,) if status else res
         return res if len(res) > 1 else res[0]
 
+    def verify_io(self, inputs, key_index, input_index, outp, c, s, ad=None, status=False):
+        """verify with inp[i] = inputs.points[input_index[i]] (vrfs_ietf_verify_prepared_io_batch; `inputs` from
+        Engine.inputs_prepare) -> ok flags [, status]; an input index >= n_inputs or an input with input_ok = 0: ITEM_INVALID_DATA"""
+        key_index = np.ascontiguousarray(key_index, dtype=np.uint32).reshape(-1); n = len(key_index)
+        input_index = np.ascontiguousarray(input_index, dtype=np.uint32).reshape(n)
+        outp = _u8(outp, (n, 64)); c = _u8(c, (n, 32)); s = _u8(s, (n, 32))
+        adb, off = pack_var(ad, n)
+        ok = np.zeros(n, np.uint8); st = np.zeros(n, np.uint8) if status else None
+        self.engine._call("vrfs_ietf_verify_prepared_io_batch", self.handle, inputs.handle, C.c_size_t(n), _p(key_index), _p(input_index), _p(outp),
+                          _p(c), _p(s), _p(adb), _p(off), _p(ok), _p(st))
+        return (ok, st) if status else ok
+
+    def verify_io_dev(self, inputs, n, d_key_index, d_input_index, d_outp, d_c, d_s, d_ok, d_ad=None, d_off=None, d_status=None):
+        """verify_io on device buffers (ints or torch CUDA tensors; indices uint32, 16-byte aligned); enqueued on the context stream"""
+        self.engine._call("vrfs_ietf_verify_prepared_io_batch_dev", self.handle, inputs.handle, C.c_size_t(n), _dev_ptr(d_key_index),
+                          _dev_ptr(d_input_index), _dev_ptr(d_outp), _dev_ptr(d_c), _dev_ptr(d_s), _dev_ptr(d_ad), _dev_ptr(d_off), _dev_ptr(d_ok),
+                          _dev_ptr(d_status))
+
+    def verify_io_wire(self, inputs, key_index, input_index, sig, ad=None, want_hash=True, status=False):
+        """verify_wire with datas[i] = the data of input input_index[i] (vrfs_ietf_verify_prepared_io_wire_batch; keys from
+        Engine.public_keys_prepare_encoded) -> (ok, beta[, status]); an input index >= n_inputs or an input with input_ok = 0:
+        ITEM_INVALID_DATA with a zero hash"""
+        e = self.engine
+        key_index = np.ascontiguousarray(key_index, dtype=np.uint32).reshape(-1); n = len(key_index)
+        input_index = np.ascontiguousarray(input_index, dtype=np.uint32).reshape(n)
+        sig = _u8(sig, (n, e.ietf_signature_len(self.suite))); adb, off = pack_var(ad, n)
+        ok = np.zeros(n, np.uint8)
+        h = np.zeros((n, e.hash_len(self.suite)), np.uint8) if want_hash else None
+        st = np.zeros(n, np.uint8) if status else None
+        e._call("vrfs_ietf_verify_prepared_io_wire_batch", self.handle, inputs.handle, C.c_size_t(n), _p(key_index), _p(input_index), _p(sig),
+                _p(adb), _p(off), _p(ok), _p(h), _p(st))
+        res = (ok, h) if want_hash else (ok,)
+        res = res + (st,) if status else res
+        return res if len(res) > 1 else res[0]
+
     def release(self):
         if self.handle:
             self.engine._lib.vrfs_public_keys_release(self.handle)
+            self.handle = None
+            if self in self.engine._prepared:
+                self.engine._prepared.remove(self)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.release()
+
+
+class PreparedInputs:
+    """VRF inputs prepared once for many verifies (vrfs_inputs_prepare): Input::new of each data item, and one fixed-base table per
+    input point on the engine's GPU.  input_ok[j] / points[j] are what Engine.data_to_point gives for datas[j].  Usable as a
+    context manager; release() frees the tables."""
+
+    def __init__(self, engine, handle, suite, input_ok, points):
+        self.engine, self.handle, self.suite, self.input_ok, self.points = engine, handle, suite, input_ok, points
+
+    @property
+    def n_inputs(self):
+        return len(self.input_ok)
+
+    def release(self):
+        if self.handle:
+            self.engine._lib.vrfs_inputs_release(self.handle)
             self.handle = None
             if self in self.engine._prepared:
                 self.engine._prepared.remove(self)
@@ -294,6 +355,17 @@ class Engine:
         h = C.c_void_p()
         self._call("vrfs_public_keys_prepare_encoded", suite, C.c_size_t(len(pk_enc)), _p(pk_enc), _p(key_ok), C.byref(h))
         p = PreparedPublics(self, h, suite, key_ok, from_encodings=True)
+        self._prepared.append(p)
+        return p
+
+    def inputs_prepare(self, suite, datas):
+        """VRF input data of one suite -> PreparedInputs: hashed to the curve once, one fixed-base table per input point (~400 KB)
+        on this GPU, so that proofs over a few distinct inputs are verified by input index (vrfs_inputs_prepare)"""
+        data, off = pack_var(datas); n = len(off) - 1
+        input_ok = np.zeros(n, np.uint8); pts = np.zeros((n, 64), np.uint8)
+        h = C.c_void_p()
+        self._call("vrfs_inputs_prepare", suite, C.c_size_t(n), _p(data), _p(off), _p(input_ok), _p(pts), C.byref(h))
+        p = PreparedInputs(self, h, suite, input_ok, pts)
         self._prepared.append(p)
         return p
 

@@ -161,6 +161,39 @@ vrfs_status vrfs_ietf_verify_prepared_wire_batch(vrfs_ctx*, const vrfs_public_ke
                                                  const uint8_t* data, const uint64_t* data_off, const uint8_t* sig /*n*sig_len*/,
                                                  const uint8_t* ad, const uint64_t* ad_off,
                                                  uint8_t* out_ok, uint8_t* out_hash /*n*hash_len, may be NULL*/, uint8_t* out_status /* may be NULL */);
+/* The same against PREPARED VRF INPUTS: a lottery or beacon round has every participant evaluate the VRF on the round's input, so a
+ * batch holds few distinct inputs (JAM/Safrole seals: hundreds of signatures over one to three inputs per epoch).
+ * vrfs_inputs_prepare runs Input::new on n_inputs data items once: out_input_ok[j] is the flag of vrfs_data_to_point_batch
+ * (0 = no point found) and out_points its points byte for byte; then it builds one table per input point, of the layout and size
+ * of a prepared key, so that s*I costs 32-33 mixed additions and V = s*I - c*O keeps one variable base, c*O.
+ * 1 <= n_inputs <= 65536, else VRFS_BAD_ARG.
+ *   vrfs_ietf_verify_prepared_io_batch[_dev]: item i is vrfs_ietf_verify_prepared_batch with input[i] = points[input_index[i]]
+ *     (ok and status), 136 bytes per item instead of 196.  input_index[i] >= n_inputs, or an input with input_ok = 0, makes item
+ *     i VRFS_ITEM_INVALID_DATA (never an out-of-range read).  The _dev form takes 16-byte aligned device buffers and is
+ *     asynchronous on the context's stream.
+ *   vrfs_ietf_verify_prepared_io_wire_batch: item i is vrfs_ietf_verify_prepared_wire_batch with data[i] = the data of input
+ *     input_index[i] as given to vrfs_inputs_prepare - and so vrfs_ietf_verify_wire_batch on the gathered key encodings and data -
+ *     ok, hash and status byte for byte, without hash-to-curve per item.  An input index out of range, or an input with
+ *     input_ok = 0, is VRFS_ITEM_INVALID_DATA with ok 0 and a zero hash.  The keys must come from vrfs_public_keys_prepare_encoded.
+ * Input points come from hash-to-curve and lie in the prime-order subgroup, where the table's s*I equals the s*I of the other
+ * calls; O goes through the same variable-base path as there, so this adds no caveat to those above.  Handles follow the rules
+ * of prepared keys: one context; orphaned by vrfs_ctx_destroy; release of an orphan or NULL only frees the record.  A keys and an
+ * inputs handle of different suites or contexts are VRFS_BAD_ARG.  n = 0 returns VRFS_OK. */
+typedef struct vrfs_inputs vrfs_inputs;
+vrfs_status vrfs_inputs_prepare(vrfs_ctx*, vrfs_suite, size_t n_inputs, const uint8_t* data, const uint64_t* data_off /*n_inputs+1*/,
+                                uint8_t* out_input_ok /*n_inputs, may be NULL*/, uint8_t* out_points /*n_inputs*64, may be NULL*/,
+                                vrfs_inputs** out);
+void vrfs_inputs_release(vrfs_inputs*);
+vrfs_status vrfs_ietf_verify_prepared_io_batch(vrfs_ctx*, const vrfs_public_keys*, const vrfs_inputs*, size_t n, const uint32_t* key_index,
+                                               const uint32_t* input_index, const uint8_t* output, const uint8_t* c, const uint8_t* s,
+                                               const uint8_t* ad, const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_status /* may be NULL */);
+vrfs_status vrfs_ietf_verify_prepared_io_batch_dev(vrfs_ctx*, const vrfs_public_keys*, const vrfs_inputs*, size_t n, const uint32_t* d_key_index,
+                                                   const uint32_t* d_input_index, const uint8_t* d_output, const uint8_t* d_c, const uint8_t* d_s,
+                                                   const uint8_t* d_ad, const uint64_t* d_ad_off, uint8_t* d_out_ok, uint8_t* d_out_status /* may be NULL */);
+vrfs_status vrfs_ietf_verify_prepared_io_wire_batch(vrfs_ctx*, const vrfs_public_keys*, const vrfs_inputs*, size_t n, const uint32_t* key_index,
+                                                    const uint32_t* input_index, const uint8_t* sig /*n*sig_len*/, const uint8_t* ad,
+                                                    const uint64_t* ad_off, uint8_t* out_ok, uint8_t* out_hash /*n*hash_len, may be NULL*/,
+                                                    uint8_t* out_status /* may be NULL */);
 
 /* pedersen::Prover::prove / Verifier::verify (A.10).  proof = pk_com || r || ok (3 x 64-byte affine) || s || sb (2 x 32 bytes) = 256 bytes. */
 vrfs_status vrfs_pedersen_prove_batch(vrfs_ctx*, vrfs_suite, size_t n, const uint8_t* sk, const uint8_t* input, const uint8_t* output,

@@ -163,6 +163,29 @@ struct Public : Points {
   }
 };
 
+// Inputs that many proofs share (a lottery or beacon round): Input::new of each data item once, and one fixed-base table per input
+// point on the engine's GPU (vrfs_inputs_prepare); PreparedPublics verifies proofs by key index and input index against them.
+// The engine must outlive the calls; destroying it first leaves release safe (RAII).
+class PreparedInputs {
+ public:
+  PreparedInputs(const Suite& s, const std::vector<Bytes>& datas) : suite_(s), input_ok_(datas.size()), points_(64 * datas.size()) {
+    Packed d(datas);
+    suite_.engine->check(vrfs_inputs_prepare(suite_.engine->ctx(), suite_.id, d.size(), d.ptr(), d.off.data(), input_ok_.data(), points_.data(), &h_));
+  }
+  ~PreparedInputs() { vrfs_inputs_release(h_); }
+  PreparedInputs(const PreparedInputs&) = delete;
+  PreparedInputs& operator=(const PreparedInputs&) = delete;
+  size_t size() const { return input_ok_.size(); }
+  const Bytes& input_ok() const { return input_ok_; }        // Input::new's Option: 0 = no point found
+  Input input() const { return Input{{suite_, points_}}; }   // the points, as Input::new gives them
+  const vrfs_inputs* handle() const { return h_; }
+
+ private:
+  Suite suite_;
+  Bytes input_ok_, points_;
+  vrfs_inputs* h_ = nullptr;
+};
+
 // A Public that is reused ("prepare once, verify many"): one fixed-base table per key on the engine's GPU (vrfs_public_keys_prepare),
 // proofs verified by key index.  The engine must outlive the calls; destroying it first leaves release safe (RAII).
 class PreparedPublics {
@@ -192,6 +215,23 @@ class PreparedPublics {
     Packed d(datas), a(ad); size_t n = key_index.size(); Bytes ok(n), beta(n * suite_.hash_len());
     suite_.engine->check(vrfs_ietf_verify_prepared_wire_batch(suite_.engine->ctx(), h_, n, key_index.data(), d.ptr(), d.off.data(), sigs.data(), a.ptr(),
                                                               a.off.data(), ok.data(), beta.data(), status_ptr(errors, n)));
+    return {std::move(ok), std::move(beta)};
+  }
+  // verify with input[i] = the point of prepared input input_index[i]; an input index out of range is Error::InvalidData
+  Bytes verify(const std::vector<uint32_t>& key_index, const PreparedInputs& inputs, const std::vector<uint32_t>& input_index, const Output& output,
+               const std::vector<Bytes>& ad, const ietf::Proof& proof, Errors* errors = nullptr) const {
+    Packed a(ad); size_t n = key_index.size(); Bytes ok(n);
+    suite_.engine->check(vrfs_ietf_verify_prepared_io_batch(suite_.engine->ctx(), h_, inputs.handle(), n, key_index.data(), input_index.data(),
+                                                            output.xy.data(), proof.c.data(), proof.s.data(), a.ptr(), a.off.data(), ok.data(),
+                                                            status_ptr(errors, n)));
+    return ok;
+  }
+  // verify_signatures with datas[i] = the data of prepared input input_index[i] -> (ok, Output::hash); only for from_compressed sets
+  std::pair<Bytes, Bytes> verify_signatures(const std::vector<uint32_t>& key_index, const PreparedInputs& inputs, const std::vector<uint32_t>& input_index,
+                                            const Bytes& sigs, const std::vector<Bytes>& ad, Errors* errors = nullptr) const {
+    Packed a(ad); size_t n = key_index.size(); Bytes ok(n), beta(n * suite_.hash_len());
+    suite_.engine->check(vrfs_ietf_verify_prepared_io_wire_batch(suite_.engine->ctx(), h_, inputs.handle(), n, key_index.data(), input_index.data(),
+                                                                 sigs.data(), a.ptr(), a.off.data(), ok.data(), beta.data(), status_ptr(errors, n)));
     return {std::move(ok), std::move(beta)};
   }
 
