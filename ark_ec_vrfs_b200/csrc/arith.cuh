@@ -101,22 +101,31 @@ HD_INLINE Fp<P> cneg(const Fp<P>& a, bool c) { return select(c, neg(a), a); }
 
 // Reduction rows m*p of the Montgomery product/square.  For p = 1 - 2^32 (mod 2^64) (BLS12-381 Fr: p[0] = 1,
 // p[1] = 2^32-1, so NINV = -1 and m = -column0) the lowest limb pair of each chain needs no multiplier:
-// m*1 = (0 : m) and m*(2^32-1) = (m - [m != 0] : -m).  VRFS_LOW_SPECIAL=0 keeps the generic rows for comparison.
+// m*1 = (0 : m) and m*(2^32-1) = (m - [m != 0] : -m).  With NINV = -1 the row's column value c0 is -m itself, and m and
+// m - [m != 0] come out of one borrow chain (MontChains::neg_bm1): no compare, no predicated negation - ptxas issued those as
+// IMAD.MOV on the multiplier pipe, which the products keep busy.  VRFS_LOW_SPECIAL=0 keeps the generic rows for comparison.
 #ifndef VRFS_LOW_SPECIAL
 #define VRFS_LOW_SPECIAL 1
 #endif
 template <class P> struct RedRows {
   typedef MontChains<P::N> C;
   static constexpr bool SPECIAL = P::LOW_1_FF && VRFS_LOW_SPECIAL;
-  static HD_INLINE uint32_t bm1(uint32_t m) { return m - (m != 0u ? 1u : 0u); }
-  static HD_INLINE void even(uint32_t* acc, uint32_t& top, const uint32_t* mod, uint32_t m) {
-    if (SPECIAL) C::mad_row_lo1(acc, top, mod, m); else C::mad_row(acc, top, mod, m);
+  static_assert(!SPECIAL || P::NINV == 0xffffffffu, "p = 1 - 2^32 (mod 2^64) has NINV = -1");
+  struct M { uint32_t m, nb, bm1; };   // the row multiplier; special rows also -m and m - [m != 0]
+  static HD_INLINE M mult(uint32_t c0) {
+    M r;
+    if (SPECIAL) { r.nb = c0; C::neg_bm1(r.m, r.bm1, c0); }
+    else { r.m = c0 * P::NINV; r.nb = r.bm1 = 0u; }
+    return r;
   }
-  static HD_INLINE void odd_top(uint32_t* acc, const uint32_t* mod, uint32_t m) {
-    if (SPECIAL) C::mad_row_top_loff(acc, mod + 1, m, 0u - m, bm1(m)); else C::mad_row_top(acc, mod + 1, m);
+  static HD_INLINE void even(uint32_t* acc, uint32_t& top, const uint32_t* mod, const M& m) {
+    if (SPECIAL) C::mad_row_lo1(acc, top, mod, m.m); else C::mad_row(acc, top, mod, m.m);
   }
-  static HD_INLINE void odd_shift(uint32_t* u, uint32_t& v0, const uint32_t* mod, uint32_t m) {
-    if (SPECIAL) C::shift_mad_row_loff(u, v0, mod + 1, m, 0u - m, bm1(m)); else C::shift_mad_row(u, v0, mod + 1, m);
+  static HD_INLINE void odd_top(uint32_t* acc, const uint32_t* mod, const M& m) {
+    if (SPECIAL) C::mad_row_top_loff(acc, mod + 1, m.m, m.nb, m.bm1); else C::mad_row_top(acc, mod + 1, m.m);
+  }
+  static HD_INLINE void odd_shift(uint32_t* u, uint32_t& v0, const uint32_t* mod, const M& m) {
+    if (SPECIAL) C::shift_mad_row_loff(u, v0, mod + 1, m.m, m.nb, m.bm1); else C::shift_mad_row(u, v0, mod + 1, m.m);
   }
 };
 
@@ -217,7 +226,7 @@ HD_INLINE void mont_mul_limbs(uint32_t* out, const uint32_t* a, const uint32_t* 
     C::mul_row(v, a, b[0]);
     C::mul_row(u, a + 1, b[0]);
     {
-      uint32_t m = v[0] * P::NINV;
+      const typename RedRows<P>::M m = RedRows<P>::mult(v[0]);
       RedRows<P>::odd_top(u, mod, m);
       RedRows<P>::even(v, u[N - 1], mod, m);
     }
@@ -226,13 +235,13 @@ HD_INLINE void mont_mul_limbs(uint32_t* out, const uint32_t* a, const uint32_t* 
       if (i & 1) {  // roles: dead-even = v, odd = u
         C::shift_mad_row(v, u[0], a + 1, b[i]);
         C::mad_row(u, v[N - 1], a, b[i]);
-        uint32_t m = u[0] * P::NINV;
+        const typename RedRows<P>::M m = RedRows<P>::mult(u[0]);
         RedRows<P>::odd_top(v, mod, m);
         RedRows<P>::even(u, v[N - 1], mod, m);
       } else {
         C::shift_mad_row(u, v[0], a + 1, b[i]);
         C::mad_row(v, u[N - 1], a, b[i]);
-        uint32_t m = v[0] * P::NINV;
+        const typename RedRows<P>::M m = RedRows<P>::mult(v[0]);
         RedRows<P>::odd_top(u, mod, m);
         RedRows<P>::even(v, u[N - 1], mod, m);
       }
@@ -302,11 +311,11 @@ HD_INLINE void mont_reduce_wide(uint32_t* out, const uint32_t* t) {
 #pragma unroll
   for (int i = 0; i < N; i++) {
     if (i & 1) {   // live-even = u, dead-even (to be shifted) = v
-      uint32_t m = (u[0] + v[1]) * P::NINV;
+      const typename RedRows<P>::M m = RedRows<P>::mult(u[0] + v[1]);
       RedRows<P>::odd_shift(v, u[0], mod, m);
       RedRows<P>::even(u, v[N - 1], mod, m);
     } else {
-      uint32_t m = (v[0] + u[1]) * P::NINV;
+      const typename RedRows<P>::M m = RedRows<P>::mult(v[0] + u[1]);
       RedRows<P>::odd_shift(u, v[0], mod, m);
       RedRows<P>::even(v, u[N - 1], mod, m);
     }

@@ -151,6 +151,16 @@ def gen(N):
     L.append("    (void)nb; (void)bm1; shift_mad_row(u, v0, x, b);")
     L.append("#endif")
     L.append("  }")
+    # ---- the multiplier of such a row from its column value c0 (NINV = -1): m = -c0 and m - [m != 0] from one borrow chain
+    #      (two ALU additions instead of a compare and a predicated negation, which ptxas issues as IMAD.MOV)
+    L.append("  // m = -c0 (the reduction multiplier when NINV = -1) and bm1 = m - [m != 0]: the borrow of 0 - c0 is [c0 != 0]")
+    L.append("  static HD_INLINE void neg_bm1(uint32_t& m, uint32_t& bm1, uint32_t c0) {")
+    L.append("#ifdef __CUDA_ARCH__")
+    L.append('    asm("sub.cc.u32 %0, 0, %2; subc.u32 %1, 0, %2;" : "=r"(m), "=r"(bm1) : "r"(c0));')
+    L.append("#else")
+    L.append("    m = 0u - c0; bm1 = m - (c0 != 0u ? 1u : 0u);")
+    L.append("#endif")
+    L.append("  }")
 
     # ---- merge: u[0..N-2] += v[1..N-1] with carry, u[N-1] += carry
     L.append("  // u[0..N-2] += v[1..N-1], carry into u[N-1]")
