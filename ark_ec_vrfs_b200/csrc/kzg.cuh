@@ -5,7 +5,10 @@
 //       L = sum_i r_i C_i + sum_i (r_i z_i) W_i - [sum_i r_i v_i] G1,      R = sum_i r_i W_i,
 //       accept  <=>  e(L, G2) e(-R, [tau] G2) = 1
 //   = one 2-column MSM over the 2k + 1 bases [C | W | G1] (csrc/msm.cuh) + one product of two pairings (csrc/pairing.cuh).
+// The prover's side, vrfs_kzg_open_batch: v = p(z) and W = [q(tau)] G1 for q = (p - p(z)) / (X - z), the quotient as a blocked
+// suffix scan (csrc/kzg_open.cuh) and W as the prepared MSM of its coefficients over the monomial SRS.
 #pragma once
+#include "kzg_open.cuh"
 #ifndef VRFS_PAIRING_LANES_MAX_N
 #define VRFS_PAIRING_LANES_MAX_N 4096      // measured cross-over with the one-thread kernel (tools/pairing_bench.py): 4096 products 20 ms vs 27.5 ms
 #endif
@@ -156,5 +159,121 @@ extern "C" vrfs_status vrfs_kzg_batch_verify(vrfs_ctx* ctx, size_t k, const uint
   ST(msm_stateless_dev(ctx, n, 2, d_aff, (const uint8_t*)d_scal, d_lr, 0));
   ST(kzg_pairing_launch(ctx, d_lr, (const uint8_t*)d_g2s, (const uint32_t*)d_misc, (uint32_t*)d_misc + 8, d_ok));
   ST(copy_out(ctx, out_ok, d_ok, 1));
+  return finish_call(ctx);
+}
+
+// ---- KZG opening proofs.  One launch of each quotient kernel covers a group of at most 32 polynomials (the MSM's column limit),
+// polynomial p of the group is blockIdx.y; its coefficients are the p-th row of len 32-byte LE values, its point zs[p].
+// Scan state of a group: agg[p * chunks + c] = A_c, the chunk's value sum_{j in c} a_j z^(j - c CH); carry[..] = K_c, everything
+// above chunk c, sum_{j >= (c+1) CH} a_j z^(j - (c+1) CH); seg[(p * chunks + c) * THREADS + t] = the exclusive suffix of segment t
+// inside its chunk.
+__device__ __forceinline__ Fr255 kzg_load_mont(const uint8_t* p) { return to_mont<BlsFr>(fr_load_reduced(p).v); }
+__device__ __forceinline__ Fr255 kzg_coeff(const uint8_t* a, uint32_t len, uint32_t j) { return j < len ? kzg_load_mont(a + (size_t)32 * j) : Fr255::zero(); }
+__device__ __forceinline__ KzgSpan kzg_span_shfl_down(const KzgSpan& s, unsigned d) {
+  KzgSpan r;
+  for (int i = 0; i < 8; i++) { r.h.v[i] = __shfl_down_sync(0xffffffffu, s.h.v[i], d); r.p.v[i] = __shfl_down_sync(0xffffffffu, s.p.v[i], d); }
+  return r;
+}
+// phase 1, grid (chunks, polynomials): segment values, then a block suffix scan (warp shuffles, then the warps above through
+// shared memory) gives every segment its exclusive suffix and the chunk its value A_c
+__global__ void __launch_bounds__(KZG_OPEN_THREADS) k_kzg_quotient_chunks(uint32_t len, uint32_t chunks, const uint8_t* coeffs, const uint8_t* zs,
+                                                                          Fr255* agg, KzgSpan* seg) {
+  __shared__ KzgSpan warp_sum[KZG_OPEN_THREADS / 32];
+  const uint32_t c = blockIdx.x, p = blockIdx.y, t = threadIdx.x, lane = t & 31u, w = t >> 5;
+  const uint8_t* a = coeffs + (size_t)32 * len * p;
+  const Fr255 z = kzg_load_mont(zs + (size_t)32 * p);
+  const uint32_t base = c * KZG_OPEN_CH + KZG_OPEN_SEG * t;
+  KzgSpan s = {kzg_segment_value(z, [&](int m) { return kzg_coeff(a, len, base + m); }), kzg_pow2k(z, KZG_OPEN_LOG_SEG)};
+  for (unsigned d = 1; d < 32; d <<= 1) {                        // inclusive suffix over the lanes of the warp
+    const KzgSpan up = kzg_span_shfl_down(s, d);
+    if (lane + d < 32) s = kzg_span_combine(s, up);
+  }
+  KzgSpan ex = kzg_span_shfl_down(s, 1);
+  if (lane == 31) ex = kzg_span_identity();
+  if (lane == 0) warp_sum[w] = s;
+  __syncthreads();
+  KzgSpan above = kzg_span_identity();
+  for (int u = KZG_OPEN_THREADS / 32 - 1; u > (int)w; u--) above = kzg_span_combine(warp_sum[u], above);
+  seg[((size_t)p * chunks + c) * KZG_OPEN_THREADS + t] = kzg_span_combine(ex, above);
+  if (t == 0) agg[(size_t)p * chunks + c] = kzg_span_combine(s, above).h;
+}
+// phase 2, one thread per polynomial: K_last = 0, K_c = A_{c+1} + z^CH K_{c+1}
+__global__ void __launch_bounds__(32) k_kzg_quotient_carry(uint32_t cols, uint32_t chunks, const uint8_t* zs, const Fr255* agg, Fr255* carry) {
+  const uint32_t p = threadIdx.x;
+  if (p >= cols) return;
+  const KzgSpan step = {Fr255::zero(), kzg_pow2k(kzg_load_mont(zs + (size_t)32 * p), KZG_OPEN_LOG_CH)};
+  const Fr255* A = agg + (size_t)p * chunks;
+  Fr255* K = carry + (size_t)p * chunks;
+  Fr255 k = Fr255::zero();
+  K[chunks - 1] = k;
+  for (uint32_t c = chunks - 1; c-- > 0;) {
+    KzgSpan e = step;
+    e.h = A[c + 1];
+    K[c] = k = kzg_carry_in(e, k);
+  }
+}
+// phase 3, grid (ceil(n / CH), polynomials): q_i as canonical LE into row i of the polynomial's MSM column (n rows; zeros from
+// len - 1 on, chunks above the coefficients included); the thread of coefficient 0 writes v = p(z)
+__global__ void __launch_bounds__(KZG_OPEN_THREADS) k_kzg_quotient_finish(uint32_t n, uint32_t len, uint32_t chunks, const uint8_t* coeffs, const uint8_t* zs,
+                                                                          const KzgSpan* seg, const Fr255* carry, uint8_t* columns, uint8_t* values) {
+  const uint32_t c = blockIdx.x, p = blockIdx.y, t = threadIdx.x;
+  const uint32_t base = c * KZG_OPEN_CH + KZG_OPEN_SEG * t;
+  uint8_t* col = columns + (size_t)32 * n * p;
+  auto store = [&](int m, const Fr255& q) {
+    if (base + m >= n) return;
+    Fr255 out;
+    from_mont<BlsFr>(out.v, q);
+    fr_store16(col + (size_t)32 * (base + m), out);
+  };
+  if (c >= chunks) {                                             // above every coefficient of the polynomial
+    for (int m = 0; m < KZG_OPEN_SEG; m++) store(m, Fr255::zero());
+    return;
+  }
+  const uint8_t* a = coeffs + (size_t)32 * len * p;
+  const Fr255 z = kzg_load_mont(zs + (size_t)32 * p);
+  const Fr255 in = kzg_carry_in(seg[((size_t)p * chunks + c) * KZG_OPEN_THREADS + t], carry[(size_t)p * chunks + c]);
+  const Fr255 v = kzg_segment_finish(z, in, [&](int m) { return kzg_coeff(a, len, base + m); }, store);
+  if (base == 0) {
+    Fr255 out;
+    from_mont<BlsFr>(out.v, v);
+    fr_store16(values + (size_t)32 * p, out);
+  }
+}
+
+#define KZG_OPEN_MAX_COEFFS (1ull << 26)
+extern "C" vrfs_status vrfs_kzg_open_batch(vrfs_ctx* ctx, const vrfs_msm_bases* srs, size_t k, size_t len, const uint8_t* coeffs, const uint8_t* points_z,
+                                           uint8_t* out_values, uint8_t* out_proofs) {
+  if (!ctx || !srs || srs->ctx != ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  if (k == 0) return VRFS_OK;
+  if (!coeffs || !points_z || !out_values || !out_proofs) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  if (len > srs->n) return fail(ctx, VRFS_BAD_ARG, "polynomial longer than the SRS (len %zu > n %zu)", len, srs->n);
+  if (k > KZG_OPEN_MAX_COEFFS / (len ? len : 1)) return fail(ctx, VRFS_BAD_ARG, "more than 2^26 coefficients per call are not supported");
+  ST(begin_call(ctx, k));
+  const size_t n = srs->n, chunks = len ? (len + KZG_OPEN_CH - 1) / KZG_OPEN_CH : 1, group = k < 32 ? k : 32;
+  // every buffer sized for the largest group before the loop: ensure() may move a buffer, and earlier groups still read theirs
+  const uint8_t *d_a, *d_z; uint8_t *d_w, *d_v; void *d_cols = nullptr, *d_scan = nullptr;
+  ST(stage_in(ctx, BUF_IN0, coeffs, k * len * 32, &d_a)); ST(stage_in(ctx, BUF_IN1, points_z, k * 32, &d_z));
+  ST(ensure(ctx, BUF_X0, group * n * 32, &d_cols));
+  ST(ensure(ctx, BUF_X1, group * chunks * (2 * sizeof(Fr255) + KZG_OPEN_THREADS * sizeof(KzgSpan)), &d_scan));
+  ST(stage_out(ctx, BUF_OUT0, group * 96, &d_w)); ST(stage_out(ctx, BUF_OUT1, group * 32, &d_v));
+  Fr255* agg = (Fr255*)d_scan;
+  Fr255* carry = agg + group * chunks;
+  KzgSpan* seg = (KzgSpan*)(carry + group * chunks);
+  for (size_t i0 = 0; i0 < k; i0 += group) {
+    const size_t cols = k - i0 < group ? k - i0 : group;
+    const uint8_t *a = d_a + 32 * len * i0, *z = d_z + 32 * i0;
+    k_kzg_quotient_chunks<<<dim3((unsigned)chunks, (unsigned)cols), KZG_OPEN_THREADS, 0, ctx->stream>>>((uint32_t)len, (uint32_t)chunks, a, z, agg, seg);
+    LAUNCHED_AS(ctx, "kzg_quotient_chunks");
+    k_kzg_quotient_carry<<<1, 32, 0, ctx->stream>>>((uint32_t)cols, (uint32_t)chunks, z, agg, carry);
+    LAUNCHED_AS(ctx, "kzg_quotient_carry");
+    k_kzg_quotient_finish<<<dim3((unsigned)((n + KZG_OPEN_CH - 1) / KZG_OPEN_CH), (unsigned)cols), KZG_OPEN_THREADS, 0, ctx->stream>>>(
+        (uint32_t)n, (uint32_t)len, (uint32_t)chunks, a, z, seg, carry, (uint8_t*)d_cols, d_v);
+    LAUNCHED_AS(ctx, "kzg_quotient_finish");
+    if (len > 1) ST(msm_prepared_dev(ctx, srs, (int)cols, 0, (const uint8_t*)d_cols, d_w, 0));
+    else CU(cudaMemsetAsync(d_w, 0, cols * 96, ctx->stream));  // q = 0: every proof is the identity
+    ST(copy_out(ctx, out_values + 32 * i0, d_v, cols * 32));
+    ST(copy_out(ctx, out_proofs + 96 * i0, d_w, cols * 96));
+  }
   return finish_call(ctx);
 }

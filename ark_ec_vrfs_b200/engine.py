@@ -59,6 +59,18 @@ class PreparedBases:
         self.engine._call("vrfs_msm_g1_prepared_partial", self.handle, _p(scalars), int(n_columns), _p(out))
         return out
 
+    def kzg_open(self, coeffs, zs):
+        """KZG openings over this handle as a monomial SRS [tau^j] G1: coeffs (k, len, 32) low to high, zs (k, 32) ->
+        (values (k, 32) = p_i(z_i), proofs (k, 96) = [(p_i - v_i) / (X - z_i)](tau) G1) (vrfs_kzg_open_batch)"""
+        coeffs = np.asarray(coeffs, np.uint8)
+        if coeffs.ndim != 3 or coeffs.shape[2] != 32:
+            raise ValueError(f"coeffs must have shape (k, len, 32), not {coeffs.shape}")
+        k, n_coeffs = coeffs.shape[0], coeffs.shape[1]
+        coeffs = _u8(coeffs, (k, n_coeffs, 32)); zs = _u8(zs, (k, 32))
+        values = np.zeros((k, 32), np.uint8); proofs = np.zeros((k, 96), np.uint8)
+        self.engine._call("vrfs_kzg_open_batch", self.handle, C.c_size_t(k), C.c_size_t(n_coeffs), _p(coeffs), _p(zs), _p(values), _p(proofs))
+        return values, proofs
+
     def ring_commit(self, keys, keyset_part_size, padding, tail, lagrange=True):
         """(cx, cy, selector) commitments (3, 96) of the ring's fixed columns over this SRS (vrfs_ring_commit)"""
         keys = _u8(keys, (-1, 64)); tail = _u8(tail, (-1, 64)); padding = _u8(padding, (64,)); out = np.zeros((3, 96), np.uint8)

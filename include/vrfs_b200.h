@@ -411,6 +411,17 @@ vrfs_status vrfs_pairing_product_batch(vrfs_ctx*, size_t n, int n_pairs, const u
 vrfs_status vrfs_kzg_batch_verify(vrfs_ctx*, size_t k, const uint8_t* commitments /*k*96*/, const uint8_t* points_z /*k*32*/, const uint8_t* values_v /*k*32*/,
                                   const uint8_t* proofs /*k*96*/, const uint8_t* coeffs_r /*k*32*/, const uint8_t* g2 /*192*/, const uint8_t* tau_g2 /*192*/,
                                   int check_points, uint8_t* out_ok /*1*/);
+/* KZG opening proofs over a prepared MONOMIAL SRS (vrfs_msm_g1_prepare of [tau^j] G1, j < n):
+ *   for i < k:  p_i(X) = sum_{j < len} coeffs[(i*len + j)*32 ..] X^j,  z_i = points_z[i*32 ..]
+ *   (32-byte LE, reduced mod r on load as vrfs_fr_fft_batch does);
+ *   out_values[i] = p_i(z_i), canonical 32-byte LE;
+ *   out_proofs[i] = [q_i(tau)] G1, q_i = (p_i - p_i(z_i)) / (X - z_i), 96-byte affine (identity = zeros).
+ * len <= n (VRFS_BAD_ARG otherwise: a polynomial longer than the SRS has no commitment), k * max(len, 1) <= 2^26.  len = 0 is the
+ * zero polynomial (v = 0), len = 1 a constant (v = a_0); both have the identity as proof.  k = 0 writes nothing.  The commitment
+ * of p_i is vrfs_msm_g1_prepared over the same handle with the coefficients zero-padded to n; the proofs of k polynomials cost
+ * the prepared MSM of ceil(k / 32) column groups (at most 32 columns each) plus the quotient. */
+vrfs_status vrfs_kzg_open_batch(vrfs_ctx*, const vrfs_msm_bases* srs, size_t k, size_t len, const uint8_t* coeffs /*k*len*32*/,
+                                const uint8_t* points_z /*k*32*/, uint8_t* out_values /*k*32*/, uint8_t* out_proofs /*k*96*/);
 
 /* self-test / measurement helper: 1/a in BLS12-381 Fq (the inversion behind the MSM's affine output) for n canonical 48-byte LE
  * values, 0 -> 0; out_ok[i] = 1 when the word-approximation GCD finished without falling back to the binary Euclid. */
