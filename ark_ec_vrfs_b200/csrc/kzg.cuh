@@ -6,7 +6,8 @@
 //       accept  <=>  e(L, G2) e(-R, [tau] G2) = 1
 //   = one 2-column MSM over the 2k + 1 bases [C | W | G1] (csrc/msm.cuh) + one product of two pairings (csrc/pairing.cuh).
 // The prover's side, vrfs_kzg_open_batch: v = p(z) and W = [q(tau)] G1 for q = (p - p(z)) / (X - z), the quotient as a blocked
-// suffix scan (csrc/kzg_open.cuh) and W as the prepared MSM of its coefficients over the monomial SRS.
+// suffix scan (csrc/kzg_open.cuh) and W as the prepared MSM of its coefficients over the monomial SRS.  vrfs_kzg_open_aggregated_batch:
+// every p_i(z_g) by chunked evaluation, P_g = sum nu_i p_i per group, and the openings of the P_g through the same slice loop.
 #pragma once
 #include "kzg_open.cuh"
 #ifndef VRFS_PAIRING_LANES_MAX_N
@@ -240,6 +241,102 @@ __global__ void __launch_bounds__(KZG_OPEN_THREADS) k_kzg_quotient_finish(uint32
   }
 }
 
+// evaluation of vrfs_kzg_open_aggregated_batch, grid (every chunk of every polynomial): the polynomials are concatenated
+// (coeff_off: n_polys + 1 coefficient offsets), chunk b is chunk b - chunk_off[p] of polynomial p = chunk_poly[b], whose point is
+// zs[poly_group[p]].  Segment values, then an ordered reduction of their spans (shuffles in lane order, then the warps in order)
+// gives the chunk's value A_b = sum_{j in the chunk} a_j z^(j - its lowest index).
+__global__ void __launch_bounds__(KZG_OPEN_THREADS) k_kzg_eval_chunks(const uint8_t* coeffs, const uint64_t* coeff_off, const uint32_t* chunk_off,
+                                                                      const uint32_t* chunk_poly, const uint32_t* poly_group, const uint8_t* zs, Fr255* agg) {
+  __shared__ KzgSpan warp_sum[KZG_OPEN_THREADS / 32];
+  const uint32_t b = blockIdx.x, p = chunk_poly[b], t = threadIdx.x, lane = t & 31u, w = t >> 5;
+  const uint64_t off = coeff_off[p];
+  const uint32_t len = (uint32_t)(coeff_off[p + 1] - off);
+  const uint8_t* a = coeffs + 32 * off;
+  const Fr255 z = kzg_load_mont(zs + (size_t)32 * poly_group[p]);
+  const uint32_t base = (b - chunk_off[p]) * KZG_OPEN_CH + KZG_OPEN_SEG * t;
+  KzgSpan s = {kzg_segment_value(z, [&](int m) { return kzg_coeff(a, len, base + m); }), kzg_pow2k(z, KZG_OPEN_LOG_SEG)};
+  // after step d, a lane l with l % 2d = 0 holds the lanes l .. l + 2d - 1 in order (the other lanes' values are never read)
+  for (unsigned d = 1; d < 32; d <<= 1) s = kzg_span_combine(s, kzg_span_shfl_down(s, d));
+  if (lane == 0) warp_sum[w] = s;
+  __syncthreads();
+  if (t == 0) {
+    KzgSpan c = warp_sum[0];
+    for (int u = 1; u < KZG_OPEN_THREADS / 32; u++) c = kzg_span_combine(c, warp_sum[u]);
+    agg[b] = c.h;
+  }
+}
+// one thread per polynomial: v_i = sum_c A_c (z^CH)^c over its chunks, canonical LE (0 for a polynomial without coefficients)
+__global__ void __launch_bounds__(128) k_kzg_eval_finish(uint32_t n_polys, const uint32_t* chunk_off, const uint32_t* poly_group, const uint8_t* zs,
+                                                         const Fr255* agg, uint8_t* values) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_polys) return;
+  const Fr255 z_ch = kzg_pow2k(kzg_load_mont(zs + (size_t)32 * poly_group[i]), KZG_OPEN_LOG_CH);
+  const Fr255* A = agg + chunk_off[i];
+  const Fr255 v = kzg_chunk_horner(z_ch, chunk_off[i + 1] - chunk_off[i], [&](uint32_t c) { return A[c]; });
+  Fr255 out;
+  from_mont<BlsFr>(out.v, v);
+  fr_store16(values + (size_t)32 * i, out);
+}
+// aggregation, grid (ceil(len / CH), groups of a slice): row j of slice group y (group g0 + y, polynomials group_off[g] ..
+// group_off[g + 1] - 1) = sum_{i in the group, j < len_i} nu_i a_{i,j}, canonical LE, rows of len coefficients per group
+__global__ void __launch_bounds__(KZG_OPEN_THREADS) k_kzg_aggregate(uint32_t g0, uint32_t len, const uint8_t* coeffs, const uint64_t* coeff_off,
+                                                                    const uint32_t* group_off, const uint8_t* nus, uint8_t* out) {
+  const uint32_t g = g0 + blockIdx.y, base = blockIdx.x * KZG_OPEN_CH + KZG_OPEN_SEG * threadIdx.x;
+  if (base >= len) return;
+  Fr255 acc[KZG_OPEN_SEG];
+  for (int m = 0; m < KZG_OPEN_SEG; m++) acc[m] = Fr255::zero();
+  for (uint32_t i = group_off[g]; i < group_off[g + 1]; i++) {
+    const uint64_t off = coeff_off[i];
+    const uint32_t len_i = (uint32_t)(coeff_off[i + 1] - off);
+    if (base >= len_i) continue;
+    const Fr255 nu = kzg_load_mont(nus + (size_t)32 * i);
+    const uint8_t* a = coeffs + 32 * (off + base);
+    for (int m = 0; m < KZG_OPEN_SEG; m++)
+      if (base + m < len_i) acc[m] = acc[m] + kzg_agg_term(nu, fr_load_reduced(a + 32 * m));
+  }
+  uint8_t* row = out + (size_t)32 * len * blockIdx.y;
+  for (int m = 0; m < KZG_OPEN_SEG; m++)
+    if (base + m < len) fr_store16(row + (size_t)32 * (base + m), acc[m]);
+}
+
+// The opening loop of vrfs_kzg_open_batch and vrfs_kzg_open_aggregated_batch: k polynomials at the points d_z (k * 32 bytes), in
+// slices of at most 32 (the MSM's column limit) through the three quotient kernels and the prepared MSM, values and proofs copied
+// out slice by slice (values only when out_values is not null).  slice(i0, cols, &a, &len) enqueues whatever produces the
+// coefficients of polynomials i0 .. i0 + cols - 1 and names them: cols rows of len <= max_len coefficients on the device.
+// Every buffer here is sized for the largest slice before the first one (ensure() may move a buffer, and earlier slices still
+// read theirs); the caller sizes its own buffers before calling.
+template <class Slice>
+static vrfs_status kzg_open_slices(vrfs_ctx* ctx, const vrfs_msm_bases* srs, size_t k, size_t max_len, const uint8_t* d_z, uint8_t* out_values,
+                                   uint8_t* out_proofs, Slice slice) {
+  const size_t n = srs->n, group = k < 32 ? k : 32, max_chunks = max_len ? (max_len + KZG_OPEN_CH - 1) / KZG_OPEN_CH : 1;
+  uint8_t *d_w, *d_v; void *d_cols = nullptr, *d_scan = nullptr;
+  ST(ensure(ctx, BUF_X0, group * n * 32, &d_cols));
+  ST(ensure(ctx, BUF_X1, group * max_chunks * (2 * sizeof(Fr255) + KZG_OPEN_THREADS * sizeof(KzgSpan)), &d_scan));
+  ST(stage_out(ctx, BUF_OUT0, group * 96, &d_w)); ST(stage_out(ctx, BUF_OUT1, group * 32, &d_v));
+  for (size_t i0 = 0; i0 < k; i0 += group) {
+    const size_t cols = k - i0 < group ? k - i0 : group;
+    const uint8_t* a = nullptr; size_t len = 0;
+    ST(slice(i0, cols, &a, &len));
+    const size_t chunks = len ? (len + KZG_OPEN_CH - 1) / KZG_OPEN_CH : 1;
+    Fr255* agg = (Fr255*)d_scan;
+    Fr255* carry = agg + group * chunks;
+    KzgSpan* seg = (KzgSpan*)(carry + group * chunks);
+    const uint8_t* z = d_z + 32 * i0;
+    k_kzg_quotient_chunks<<<dim3((unsigned)chunks, (unsigned)cols), KZG_OPEN_THREADS, 0, ctx->stream>>>((uint32_t)len, (uint32_t)chunks, a, z, agg, seg);
+    LAUNCHED_AS(ctx, "kzg_quotient_chunks");
+    k_kzg_quotient_carry<<<1, 32, 0, ctx->stream>>>((uint32_t)cols, (uint32_t)chunks, z, agg, carry);
+    LAUNCHED_AS(ctx, "kzg_quotient_carry");
+    k_kzg_quotient_finish<<<dim3((unsigned)((n + KZG_OPEN_CH - 1) / KZG_OPEN_CH), (unsigned)cols), KZG_OPEN_THREADS, 0, ctx->stream>>>(
+        (uint32_t)n, (uint32_t)len, (uint32_t)chunks, a, z, seg, carry, (uint8_t*)d_cols, d_v);
+    LAUNCHED_AS(ctx, "kzg_quotient_finish");
+    if (len > 1) ST(msm_prepared_dev(ctx, srs, (int)cols, 0, (const uint8_t*)d_cols, d_w, 0));
+    else CU(cudaMemsetAsync(d_w, 0, cols * 96, ctx->stream));  // q = 0: every proof is the identity
+    if (out_values) ST(copy_out(ctx, out_values + 32 * i0, d_v, cols * 32));
+    ST(copy_out(ctx, out_proofs + 96 * i0, d_w, cols * 96));
+  }
+  return VRFS_OK;
+}
+
 #define KZG_OPEN_MAX_COEFFS (1ull << 26)
 extern "C" vrfs_status vrfs_kzg_open_batch(vrfs_ctx* ctx, const vrfs_msm_bases* srs, size_t k, size_t len, const uint8_t* coeffs, const uint8_t* points_z,
                                            uint8_t* out_values, uint8_t* out_proofs) {
@@ -250,30 +347,88 @@ extern "C" vrfs_status vrfs_kzg_open_batch(vrfs_ctx* ctx, const vrfs_msm_bases* 
   if (len > srs->n) return fail(ctx, VRFS_BAD_ARG, "polynomial longer than the SRS (len %zu > n %zu)", len, srs->n);
   if (k > KZG_OPEN_MAX_COEFFS / (len ? len : 1)) return fail(ctx, VRFS_BAD_ARG, "more than 2^26 coefficients per call are not supported");
   ST(begin_call(ctx, k));
-  const size_t n = srs->n, chunks = len ? (len + KZG_OPEN_CH - 1) / KZG_OPEN_CH : 1, group = k < 32 ? k : 32;
-  // every buffer sized for the largest group before the loop: ensure() may move a buffer, and earlier groups still read theirs
-  const uint8_t *d_a, *d_z; uint8_t *d_w, *d_v; void *d_cols = nullptr, *d_scan = nullptr;
+  const uint8_t *d_a, *d_z;
   ST(stage_in(ctx, BUF_IN0, coeffs, k * len * 32, &d_a)); ST(stage_in(ctx, BUF_IN1, points_z, k * 32, &d_z));
-  ST(ensure(ctx, BUF_X0, group * n * 32, &d_cols));
-  ST(ensure(ctx, BUF_X1, group * chunks * (2 * sizeof(Fr255) + KZG_OPEN_THREADS * sizeof(KzgSpan)), &d_scan));
-  ST(stage_out(ctx, BUF_OUT0, group * 96, &d_w)); ST(stage_out(ctx, BUF_OUT1, group * 32, &d_v));
-  Fr255* agg = (Fr255*)d_scan;
-  Fr255* carry = agg + group * chunks;
-  KzgSpan* seg = (KzgSpan*)(carry + group * chunks);
-  for (size_t i0 = 0; i0 < k; i0 += group) {
-    const size_t cols = k - i0 < group ? k - i0 : group;
-    const uint8_t *a = d_a + 32 * len * i0, *z = d_z + 32 * i0;
-    k_kzg_quotient_chunks<<<dim3((unsigned)chunks, (unsigned)cols), KZG_OPEN_THREADS, 0, ctx->stream>>>((uint32_t)len, (uint32_t)chunks, a, z, agg, seg);
-    LAUNCHED_AS(ctx, "kzg_quotient_chunks");
-    k_kzg_quotient_carry<<<1, 32, 0, ctx->stream>>>((uint32_t)cols, (uint32_t)chunks, z, agg, carry);
-    LAUNCHED_AS(ctx, "kzg_quotient_carry");
-    k_kzg_quotient_finish<<<dim3((unsigned)((n + KZG_OPEN_CH - 1) / KZG_OPEN_CH), (unsigned)cols), KZG_OPEN_THREADS, 0, ctx->stream>>>(
-        (uint32_t)n, (uint32_t)len, (uint32_t)chunks, a, z, seg, carry, (uint8_t*)d_cols, d_v);
-    LAUNCHED_AS(ctx, "kzg_quotient_finish");
-    if (len > 1) ST(msm_prepared_dev(ctx, srs, (int)cols, 0, (const uint8_t*)d_cols, d_w, 0));
-    else CU(cudaMemsetAsync(d_w, 0, cols * 96, ctx->stream));  // q = 0: every proof is the identity
-    ST(copy_out(ctx, out_values + 32 * i0, d_v, cols * 32));
-    ST(copy_out(ctx, out_proofs + 96 * i0, d_w, cols * 96));
+  ST(kzg_open_slices(ctx, srs, k, len, d_z, out_values, out_proofs, [&](size_t i0, size_t, const uint8_t** a, size_t* l) {
+    *a = d_a + 32 * len * i0; *l = len;
+    return VRFS_OK;
+  }));
+  return finish_call(ctx);
+}
+
+#define KZG_OPEN_MAX_POLYS (1u << 16)
+extern "C" vrfs_status vrfs_kzg_open_aggregated_batch(vrfs_ctx* ctx, const vrfs_msm_bases* srs, size_t n_groups, size_t n_polys, const uint64_t* group_off,
+                                                      const uint64_t* coeff_off, const uint8_t* coeffs, const uint8_t* points_z, const uint8_t* nus,
+                                                      uint8_t* out_values, uint8_t* out_agg_values, uint8_t* out_proofs) {
+  if (!ctx || !srs || srs->ctx != ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  if (n_groups > KZG_OPEN_MAX_POLYS || n_polys > KZG_OPEN_MAX_POLYS) return fail(ctx, VRFS_BAD_ARG, "more than 2^16 groups or polynomials per call are not supported");
+  if (n_groups == 0) return n_polys ? fail(ctx, VRFS_BAD_ARG, "polynomials without a group (n_groups = 0, n_polys = %zu)", n_polys) : VRFS_OK;
+  if (!group_off || !coeff_off || !points_z || !out_proofs || (n_polys && (!nus || !out_values))) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  if (group_off[0] != 0 || group_off[n_groups] != n_polys) return fail(ctx, VRFS_BAD_ARG, "group offsets must run from 0 to n_polys");
+  for (size_t g = 0; g < n_groups; g++) if (group_off[g + 1] < group_off[g]) return fail(ctx, VRFS_BAD_ARG, "group offsets must be non-decreasing");
+  if (coeff_off[0] != 0) return fail(ctx, VRFS_BAD_ARG, "coefficient offsets must start at 0");
+  size_t n_chunks = 0;
+  for (size_t i = 0; i < n_polys; i++) {
+    if (coeff_off[i + 1] < coeff_off[i]) return fail(ctx, VRFS_BAD_ARG, "coefficient offsets must be non-decreasing");
+    const size_t len = coeff_off[i + 1] - coeff_off[i];
+    if (len > srs->n) return fail(ctx, VRFS_BAD_ARG, "polynomial %zu longer than the SRS (len %zu > n %zu)", i, len, srs->n);
+    n_chunks += (len + KZG_OPEN_CH - 1) / KZG_OPEN_CH;
   }
+  const size_t total = coeff_off[n_polys];
+  if (total > KZG_OPEN_MAX_COEFFS) return fail(ctx, VRFS_BAD_ARG, "more than 2^26 coefficients per call are not supported");
+  if (total && !coeffs) return fail(ctx, VRFS_BAD_ARG, "null buffer");
+  ST(begin_call(ctx, n_groups));
+  // host-built index tables, one u32 array: chunk_off (n_polys + 1) | poly_group (n_polys) | group_off (n_groups + 1) | chunk_poly (n_chunks)
+  std::vector<uint32_t> tab(2 * n_polys + n_groups + 2 + n_chunks);
+  uint32_t *chunk_off = tab.data(), *poly_group = chunk_off + n_polys + 1, *goff = poly_group + n_polys, *chunk_poly = goff + n_groups + 1;
+  std::vector<size_t> group_len(n_groups, 0);      // the longest polynomial of each group
+  chunk_off[0] = 0;
+  for (size_t g = 0; g < n_groups; g++) {
+    goff[g] = (uint32_t)group_off[g];
+    for (uint64_t i = group_off[g]; i < group_off[g + 1]; i++) {
+      const size_t len = coeff_off[i + 1] - coeff_off[i];
+      poly_group[i] = (uint32_t)g;
+      chunk_off[i + 1] = chunk_off[i] + (uint32_t)((len + KZG_OPEN_CH - 1) / KZG_OPEN_CH);
+      for (uint32_t b = chunk_off[i]; b < chunk_off[i + 1]; b++) chunk_poly[b] = (uint32_t)i;
+      if (len > group_len[g]) group_len[g] = len;
+    }
+  }
+  goff[n_groups] = (uint32_t)n_polys;
+  size_t max_len = 0;
+  for (size_t g = 0; g < n_groups; g++) if (group_len[g] > max_len) max_len = group_len[g];
+  const size_t slice = n_groups < 32 ? n_groups : 32;
+  // every buffer of the call sized before the first launch (kzg_open_slices sizes its own before its loop)
+  const uint8_t *d_a, *d_z, *d_nu, *d_coff, *d_tab; uint8_t* d_vals; void *d_p = nullptr, *d_A = nullptr;
+  ST(stage_in(ctx, BUF_IN0, coeffs, total * 32, &d_a)); ST(stage_in(ctx, BUF_IN1, points_z, n_groups * 32, &d_z));
+  ST(stage_in(ctx, BUF_IN2, nus, n_polys * 32, &d_nu)); ST(stage_in(ctx, BUF_IN3, coeff_off, (n_polys + 1) * 8, &d_coff));
+  ST(stage_in(ctx, BUF_IN4, tab.data(), tab.size() * 4, &d_tab));
+  ST(ensure(ctx, BUF_X2, slice * max_len * 32, &d_p));
+  ST(ensure(ctx, BUF_X3, n_chunks * sizeof(Fr255), &d_A));
+  ST(stage_out(ctx, BUF_X4, n_polys * 32, &d_vals));
+  const uint64_t* dc_off = (const uint64_t*)d_coff;
+  const uint32_t *d_chunk_off = (const uint32_t*)d_tab, *d_poly_group = d_chunk_off + n_polys + 1, *d_goff = d_poly_group + n_polys,
+                 *d_chunk_poly = d_goff + n_groups + 1;
+  if (n_chunks) {
+    k_kzg_eval_chunks<<<(unsigned)n_chunks, KZG_OPEN_THREADS, 0, ctx->stream>>>(d_a, dc_off, d_chunk_off, d_chunk_poly, d_poly_group, d_z, (Fr255*)d_A);
+    LAUNCHED_AS(ctx, "kzg_eval_chunks");
+  }
+  if (n_polys) {
+    k_kzg_eval_finish<<<(unsigned)((n_polys + 127) / 128), 128, 0, ctx->stream>>>((uint32_t)n_polys, d_chunk_off, d_poly_group, d_z, (const Fr255*)d_A, d_vals);
+    LAUNCHED_AS(ctx, "kzg_eval_finish");
+    ST(copy_out(ctx, out_values, d_vals, n_polys * 32));
+  }
+  // P_g of a slice of groups into X2, rows of the slice's longest polynomial; then the openings of P_g as vrfs_kzg_open_batch's
+  ST(kzg_open_slices(ctx, srs, n_groups, max_len, d_z, out_agg_values, out_proofs, [&](size_t g0, size_t cols, const uint8_t** a, size_t* l) {
+    size_t len = 0;
+    for (size_t g = g0; g < g0 + cols; g++) if (group_len[g] > len) len = group_len[g];
+    if (len) {
+      k_kzg_aggregate<<<dim3((unsigned)((len + KZG_OPEN_CH - 1) / KZG_OPEN_CH), (unsigned)cols), KZG_OPEN_THREADS, 0, ctx->stream>>>(
+          (uint32_t)g0, (uint32_t)len, d_a, dc_off, d_goff, d_nu, (uint8_t*)d_p);
+      LAUNCHED_AS(ctx, "kzg_aggregate");
+    }
+    *a = (const uint8_t*)d_p; *l = len;
+    return VRFS_OK;
+  }));
   return finish_call(ctx);
 }

@@ -1,5 +1,6 @@
 // The per-thread pieces of the KZG opening quotient (vrfs_kzg_open_batch, kernels in csrc/kzg.cuh).  Host-compilable: the CPU
-// tests run them through the same three phases as the kernels (tests/host_emul/hostemu_kzg.cpp).
+// tests run them through the same three phases as the kernels (tests/host_emul/hostemu_kzg.cpp), and the evaluation and
+// aggregation of vrfs_kzg_open_aggregated_batch likewise (tests/host_emul/hostemu_kzg_agg.cpp).
 //   p = sum_{j < len} a_j X^j,  q = (p - p(z)) / (X - z):  q_i = sum_{j > i} a_j z^(j - i - 1),  p(z) = a_0 + z q_0,
 // i.e. the suffix recurrence q_{i-1} = a_i + z q_i.  The coefficients, zero-padded at the top, split into chunks of KZG_OPEN_CH
 // (one block each), a chunk into segments of KZG_OPEN_SEG (one thread each).  A run of coefficients is a KzgSpan: its value
@@ -38,5 +39,17 @@ template <class Load, class Store> HD_INLINE Fr255 kzg_segment_finish(const Fr25
 // suffix above + z^(its distance) * what lies beyond it: the carry into a segment from its chunk (e = the exclusive suffix of the
 // segment inside the chunk, k = the chunk's carry K_c), and the chunk carry recurrence K_c = A_{c+1} + z^CH K_{c+1}
 HD_INLINE Fr255 kzg_carry_in(const KzgSpan& e, const Fr255& k) { return e.h + e.p * k; }
+
+// vrfs_kzg_open_aggregated_batch.  Evaluation: a chunk's value A_c is the ordered combination of its segments' spans (lower
+// segments on the left: kzg_span_combine is not commutative), and p(z) = sum_c A_c (z^CH)^c, by Horner from the top chunk
+// (A(c) = A_c, z_ch = z^CH).
+template <class Load> HD_INLINE Fr255 kzg_chunk_horner(const Fr255& z_ch, uint32_t chunks, Load A) {
+  Fr255 v = Fr255::zero();
+  for (uint32_t c = chunks; c-- > 0;) v = v * z_ch + A(c);
+  return v;
+}
+// Aggregation: nu in Montgomery form times a coefficient taken as a plain residue (not converted) is the Montgomery product
+// nu a R R^-1 = nu a, again a plain residue; the sums of such terms are the aggregated coefficients, with no conversion either way
+HD_INLINE Fr255 kzg_agg_term(const Fr255& nu_mont, const Fr255& a_plain) { return nu_mont * a_plain; }
 
 }  // namespace vrfs

@@ -71,6 +71,25 @@ class PreparedBases:
         self.engine._call("vrfs_kzg_open_batch", self.handle, C.c_size_t(k), C.c_size_t(n_coeffs), _p(coeffs), _p(zs), _p(values), _p(proofs))
         return values, proofs
 
+    def kzg_open_aggregated(self, polys, group_sizes, zs, nus):
+        """Aggregated KZG openings over this handle as a monomial SRS: polys a list of (len_i, 32) coefficient arrays, low to high,
+        in group order; group g is the next group_sizes[g] of them, opened at zs[g]; nus (n_polys, 32) one coefficient per
+        polynomial -> (values (n_polys, 32) = p_i(z_g), agg_values (n_groups, 32) = P_g(z_g), proofs (n_groups, 96) =
+        [(P_g - P_g(z_g)) / (X - z_g)](tau) G1) with P_g = sum_{i in g} nu_i p_i (vrfs_kzg_open_aggregated_batch)"""
+        polys = [_u8(p, (-1, 32)) for p in polys]
+        sizes = np.asarray(group_sizes, np.int64).reshape(-1)
+        if (sizes < 0).any() or int(sizes.sum()) != len(polys):
+            raise ValueError(f"group sizes {sizes.tolist()} do not partition {len(polys)} polynomials")
+        n_groups, n_polys = len(sizes), len(polys)
+        group_off = np.zeros(n_groups + 1, np.uint64); group_off[1:] = np.cumsum(sizes)
+        coeff_off = np.zeros(n_polys + 1, np.uint64); coeff_off[1:] = np.cumsum([p.shape[0] for p in polys])
+        coeffs = np.ascontiguousarray(np.concatenate(polys) if int(coeff_off[-1]) else np.zeros((1, 32), np.uint8))
+        zs = _u8(zs, (n_groups, 32)); nus = _u8(nus, (n_polys, 32))
+        values = np.zeros((n_polys, 32), np.uint8); agg = np.zeros((n_groups, 32), np.uint8); proofs = np.zeros((n_groups, 96), np.uint8)
+        self.engine._call("vrfs_kzg_open_aggregated_batch", self.handle, C.c_size_t(n_groups), C.c_size_t(n_polys), _p(group_off), _p(coeff_off),
+                          _p(coeffs), _p(zs), _p(nus), _p(values), _p(agg), _p(proofs))
+        return values, agg, proofs
+
     def ring_commit(self, keys, keyset_part_size, padding, tail, lagrange=True):
         """(cx, cy, selector) commitments (3, 96) of the ring's fixed columns over this SRS (vrfs_ring_commit)"""
         keys = _u8(keys, (-1, 64)); tail = _u8(tail, (-1, 64)); padding = _u8(padding, (64,)); out = np.zeros((3, 96), np.uint8)

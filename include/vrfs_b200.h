@@ -422,6 +422,29 @@ vrfs_status vrfs_kzg_batch_verify(vrfs_ctx*, size_t k, const uint8_t* commitment
  * the prepared MSM of ceil(k / 32) column groups (at most 32 columns each) plus the quotient. */
 vrfs_status vrfs_kzg_open_batch(vrfs_ctx*, const vrfs_msm_bases* srs, size_t k, size_t len, const uint8_t* coeffs /*k*len*32*/,
                                 const uint8_t* points_z /*k*32*/, uint8_t* out_values /*k*32*/, uint8_t* out_proofs /*k*96*/);
+/* Aggregated KZG openings over the same kind of handle (a PLONK prover's opening round in one call): n_polys polynomials of their
+ * own lengths in n_groups groups, one point per group, one coefficient nu_i per polynomial:
+ *   p_i(X) = sum_{j < len_i} coeffs[(coeff_off[i] + j)*32 ..] X^j,  len_i = coeff_off[i+1] - coeff_off[i]  (offsets in coefficients);
+ *   group g = the polynomials group_off[g] .. group_off[g+1] - 1, opened at z_g = points_z[g*32 ..];  nu_i = nus[i*32 ..]
+ *   (32-byte LE, coefficients, points and nu reduced mod r on load);
+ *   out_values[i] = p_i(z_g(i));  with P_g = sum_{i in g} nu_i p_i:
+ *   out_agg_values[g] = P_g(z_g) = sum_{i in g} nu_i out_values[i] (not written when out_agg_values is NULL);
+ *   out_proofs[g] = [(P_g - P_g(z_g)) / (X - z_g)](tau) G1, 96-byte affine (identity = zeros).
+ * out_proofs[g] and out_agg_values[g] equal, byte for byte, what vrfs_kzg_open_batch returns over the same handle for P_g
+ * (coefficients reduced mod r, len = the longest polynomial of the group) at z_g, and out_values[i] what it returns for p_i alone;
+ * with one polynomial per group and nu = 1 the call returns exactly what vrfs_kzg_open_batch does.  An empty group, or one whose
+ * polynomials all have len <= 1, has the identity as proof (an empty group the value 0); len_i = 0 gives the value 0.
+ * n_groups = 0 (with n_polys = 0) writes nothing.  VRFS_BAD_ARG, before anything is staged or written: a handle of another
+ * context; a null buffer that the counts need (group_off, coeff_off, points_z, out_proofs always; nus, out_values when n_polys > 0;
+ * coeffs when there are coefficients); group_off not running non-decreasing from 0 to n_polys; coeff_off not starting at 0 or
+ * decreasing; len_i > n; more than 2^26 coefficients in all; n_polys or n_groups above 2^16.  Cost: the prepared MSM of ceil(g / 32)
+ * column groups, as vrfs_kzg_open_batch of g polynomials, plus about one product per coefficient for the aggregation and two
+ * for the evaluations. */
+vrfs_status vrfs_kzg_open_aggregated_batch(vrfs_ctx*, const vrfs_msm_bases* srs, size_t n_groups, size_t n_polys,
+                                           const uint64_t* group_off /*n_groups+1, polynomial indices*/,
+                                           const uint64_t* coeff_off /*n_polys+1, coefficient indices*/, const uint8_t* coeffs /*coeff_off[n_polys]*32*/,
+                                           const uint8_t* points_z /*n_groups*32*/, const uint8_t* nus /*n_polys*32*/, uint8_t* out_values /*n_polys*32*/,
+                                           uint8_t* out_agg_values /*n_groups*32, may be NULL*/, uint8_t* out_proofs /*n_groups*96*/);
 
 /* self-test / measurement helper: 1/a in BLS12-381 Fq (the inversion behind the MSM's affine output) for n canonical 48-byte LE
  * values, 0 -> 0; out_ok[i] = 1 when the word-approximation GCD finished without falling back to the binary Euclid. */
