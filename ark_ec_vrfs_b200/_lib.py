@@ -30,7 +30,7 @@ SYMBOLS = [
     "vrfs_multi_ietf_verify_batch", "vrfs_multi_msm_g1_prepare", "vrfs_multi_msm_g1_prepared", "vrfs_multi_ring_commit", "vrfs_multi_msm_g1_release",
     "vrfs_pairing_product_batch", "vrfs_kzg_batch_verify", "vrfs_kzg_open_batch", "vrfs_kzg_open_aggregated_batch", "vrfs_pedersen_batch_verify", "vrfs_pedersen_batch_verify_wire",
     "vrfs_host_alloc", "vrfs_host_free", "vrfs_host_register", "vrfs_host_unregister",
-    "vrfs_ring_fixed_columns", "vrfs_ring_commit", "vrfs_ring_commit_delta", "vrfs_ring_commit_rows_partial", "vrfs_fr_fft_batch", "vrfs_fq381_inv_batch", "vrfs_g1_compress_batch", "vrfs_g1_decompress_batch",
+    "vrfs_ring_fixed_columns", "vrfs_ring_commit", "vrfs_ring_commit_delta", "vrfs_ring_commit_rows_partial", "vrfs_fr_fft_batch", "vrfs_g1_fft_batch", "vrfs_fq381_inv_batch", "vrfs_g1_compress_batch", "vrfs_g1_decompress_batch",
 ]
 
 _lib = None

@@ -369,6 +369,20 @@ class RingContext:
             raise ValueError("SRS point %d is not a valid compressed G1 point" % int(np.argmin(ok)))
         return cls(suite, pts, lagrange, padding, blinding_base_powers, keyset_part_size)
 
+    @classmethod
+    def from_powers(cls, suite, powers_g1, domain_size, padding, blinding_base_powers, keyset_part_size=None):
+        """ring-proof's `RingBuilderKey::from_srs`: the published monomial powers [tau^j]G1 ((m, 96) affine points in G1, m >= domain_size;
+        an SRS is longer, only the first domain_size are used) -> their Lagrange basis over the radix-2 domain (one inverse G1 FFT on the
+        GPU) -> a Lagrange-basis context, whose verifier_key_commitment takes the incremental path"""
+        powers = np.asarray(powers_g1, np.uint8).reshape(-1, 96)
+        n = int(domain_size)
+        if n < 1 or n & (n - 1):
+            raise ValueError(f"domain_size must be a power of two, not {n}")
+        if len(powers) < n:
+            raise ValueError(f"{len(powers)} powers of tau for a domain of {n}")
+        lagrange = suite.engine.g1_fft(powers[:n], inverse=True)
+        return cls(suite, lagrange, True, padding, blinding_base_powers, keyset_part_size)
+
     def max_ring_size(self):
         return self.keyset_part_size
 

@@ -19,6 +19,7 @@
 #include "msm.cuh"
 #include "te_msm.cuh"
 #include "ring.cuh"
+#include "g1_fft.cuh"
 #include "pairing_coop.cuh"
 
 using namespace vrfs;
@@ -2680,6 +2681,33 @@ extern "C" vrfs_status vrfs_fr_fft_batch(vrfs_ctx* ctx, int log_n, int n_columns
   ST(stage_out(ctx, BUF_OUT1, bytes, &d_o));
   ST(ntt_dev(ctx, log_n, (uint32_t)n_columns, inverse != 0, d_i, d_o));
   ST(copy_out(ctx, out, d_o, bytes));
+  return finish_call(ctx);
+}
+// the same transform over BLS12-381 G1 (csrc/g1_fft.cuh): one vector of 2^log_n affine points, in and out 96-byte LE (may alias)
+extern "C" vrfs_status vrfs_g1_fft_batch(vrfs_ctx* ctx, int log_n, int inverse, const uint8_t* in, uint8_t* out) {
+  if (!ctx) return VRFS_BAD_ARG;
+  CallGuard guard_(ctx, __func__);
+  if (log_n < 0 || log_n > 24 || !in || !out) return fail(ctx, VRFS_BAD_ARG, "bad argument (0 <= log_n <= 24, non-null buffers)");
+  const size_t n = (size_t)1 << log_n;
+  ST(begin_call(ctx, n));
+  const uint8_t* d_i; uint8_t* d_o; void *work = nullptr, *tw = nullptr;
+  ST(stage_in(ctx, BUF_IN0, in, n * 96, &d_i));
+  ST(stage_out(ctx, BUF_OUT0, n * 96, &d_o));
+  ST(ensure(ctx, BUF_X0, n * sizeof(G1Pt), &work));
+  ST(ensure(ctx, BUF_X1, (n / 2 + 1) * sizeof(Fr255), &tw));
+  k_ntt_twiddles<<<(unsigned)((n / 2 + 1 + 127) / 128), 128, 0, ctx->stream>>>(log_n, inverse != 0, (Fr255*)tw);   // n/2 twiddles + 1/n
+  LAUNCHED_AS(ctx, "ntt_twiddles");
+  k_g1_fft_load<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(log_n, d_i, (G1Pt*)work);
+  LAUNCHED_AS(ctx, "g1_fft_load");
+  for (int s = 1; s <= log_n; s++) {
+    k_g1_fft_stage<<<(unsigned)((n / 2 + G1_FFT_STAGE_THREADS - 1) / G1_FFT_STAGE_THREADS), G1_FFT_STAGE_THREADS, 0, ctx->stream>>>(
+        log_n, s, (const Fr255*)tw, (G1Pt*)work);
+    LAUNCHED_AS(ctx, "g1_fft_stage");
+  }
+  k_g1_fft_store<<<(unsigned)((n + G1_FFT_STORE_THREADS - 1) / G1_FFT_STORE_THREADS), G1_FFT_STORE_THREADS, 0, ctx->stream>>>(
+      log_n, inverse != 0, (const G1Pt*)work, (const Fr255*)tw, d_o);
+  LAUNCHED_AS(ctx, "g1_fft_store");
+  ST(copy_out(ctx, out, d_o, n * 96));
   return finish_call(ctx);
 }
 // rows [row_lo, row_lo + n) of the columns; `keys` holds the keys of those rows only (rows row_lo .. min(n_keys, row_lo + n) - 1)

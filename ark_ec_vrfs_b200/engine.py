@@ -628,6 +628,16 @@ class Engine:
         self._call("vrfs_fr_fft_batch", int(n.bit_length() - 1), int(n_columns), int(bool(inverse)), _p(values), _p(out))
         return out
 
+    def g1_fft(self, points, inverse=False):
+        """the same transform over BLS12-381 G1 (vrfs_g1_fft_batch): (n, 96) affine LE points in G1, n a power of two, -> (n, 96)
+        out_i = sum_j [w^ij] P_j, or [1/n] sum_j [w^-ij] P_j for the inverse; the inverse of [tau^j] G1 is the Lagrange basis [L_i(tau)] G1"""
+        points = _u8(points, (-1, 96)); n = len(points)
+        if n == 0 or n & (n - 1):
+            raise ValueError(f"the vector length must be a power of two, not {n}")
+        out = np.zeros_like(points)
+        self._call("vrfs_g1_fft_batch", int(n.bit_length() - 1), int(bool(inverse)), _p(points), _p(out))
+        return out
+
     def g1_compress(self, points):
         """(n, 96) affine LE G1 points (zeros = identity) -> (n, 48) ark-bls12-381 / zcash compressed encodings"""
         points = _u8(points, (-1, 96)); out = np.zeros((len(points), 48), np.uint8)

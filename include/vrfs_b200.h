@@ -380,6 +380,20 @@ vrfs_status vrfs_ring_commit_rows_partial(vrfs_ctx*, const vrfs_msm_bases* srs_r
  * n_columns vectors of 2^log_n canonical 32-byte LE values (values >= r are reduced); group_gen = TWO_ADIC_ROOT_OF_UNITY^(2^(32-log_n)).
  * in and out may be the same buffer. */
 vrfs_status vrfs_fr_fft_batch(vrfs_ctx*, int log_n, int n_columns, int inverse, const uint8_t* in /*n_columns*2^log_n*32*/, uint8_t* out);
+/* The same transform over BLS12-381 G1, on one vector of n = 2^log_n points: the domain of vrfs_fr_fft_batch,
+ * w = TWO_ADIC_ROOT_OF_UNITY^(2^(32 - log_n)), natural order on both sides.
+ *   forward (inverse = 0):  out_i = sum_j [w^(ij)] P_j
+ *   inverse (inverse != 0): out_i = [n^-1] sum_j [w^(-ij)] P_j
+ * The inverse transform of the monomial powers [tau^j] G1, j < n, is [L_i(tau)] G1 with L_i(X) = (w^i / n)(X^n - 1)/(X - w^i):
+ * exactly the basis vrfs_ring_commit(srs_is_lagrange = 1) expects (row i <-> w^i).  The forward transform maps it back to the powers.
+ * Points are 96-byte affine LE as vrfs_msm_g1_prepare takes them; the identity is 96 zero bytes, in and out.  The output is
+ * canonical: equal points give equal bytes.
+ * Precondition (as for the stateless MSM): every input point lies in the prime-order subgroup G1; the twiddle multiplication uses
+ * G1's endomorphism.  vrfs_g1_decompress_batch(check_subgroup = 1) is the validating loader.  Points outside G1 give an unspecified
+ * result, never a fault.
+ * VRFS_BAD_ARG, with out untouched, for null buffers, log_n < 0 and log_n > 24 (the size limit of vrfs_msm_g1_prepare, which the
+ * output is meant to feed).  in == out is allowed.  log_n = 0 returns the input. */
+vrfs_status vrfs_g1_fft_batch(vrfs_ctx*, int log_n, int inverse, const uint8_t* in /*2^log_n*96*/, uint8_t* out /*2^log_n*96*/);
 
 /* BLS12-381 G1 on the wire (the points of a `RingCommitment`, an SRS file): ark-bls12-381's compressed CanonicalSerialize /
  * validated CanonicalDeserialize, i.e. the zcash encoding - 48 bytes, big-endian x; bit 7 of byte 0 = compressed, bit 6 = infinity,
